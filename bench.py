@@ -3,10 +3,15 @@
 configs[1]: D=784 NonUSFlow, K=8 coupling blocks, conditioner MLP 784-256-256-1568, LU + Householder
 affine conjugation, Normal base), synthetic data, batch-sharded over N GPUs (weak scaling).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
 
-One JSON line on stdout (rank 0).  See DESIGN.md "Measurement" for every field.
+One JSON line on stdout (rank 0).  See DESIGN.md "Measurement" for every field.  `--dump-outputs DIR` also writes the
+log_prob vector the last timed step returned as DIR/log_prob.npy (float32; one file per rank under torchrun); inputs and
+weights are seeded, so two builds run with the same arguments can be compared output for output.  Compare within the
+tier's tolerance: packing the weights is not bit-reproducible in fp32, and in the bf16 tier that moves a few bf16
+roundings, so one build's log_prob varies from run to run by up to about 3e-3 relative (bf16x2: 5e-6, fp32: 1e-6;
+measured on a B200 at its 1000 W power limit).
 """
 import argparse
 import ctypes
@@ -276,13 +281,31 @@ def timed_steps_with_flush(step, steps, dev, busy=None):
     return sum(a.elapsed_time(b) for a, b in evs), out
 
 
+DUMP_LIMIT_BYTES = 64 << 20        # --dump-outputs: bytes written in all, over every rank
+
+
+def dump_outputs(path, arrays, world=1):
+    """Writes each `{name: tensor}` as `path/<name>.npy`, float32 (float64 stays float64).  Past this rank's share of
+    DUMP_LIMIT_BYTES, every array keeps the same seeded sample of its rows, in order, so that runs stay comparable."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    arrays = {k: (v if v.dtype == torch.float64 else v.float()).detach().cpu().numpy() for k, v in arrays.items()}
+    limit = DUMP_LIMIT_BYTES // world
+    total = sum(a.nbytes for a in arrays.values())
+    for name, a in arrays.items():
+        if total > limit:
+            keep = max(1, a.shape[0] * limit // total)
+            a = a[np.sort(np.random.default_rng(0).choice(a.shape[0], keep, replace=False))]
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 def cpu_reference_run(steps, warmup, rows, config=DEFAULT_CONFIG):
     """The reference's CPU PyTorch path for the same workload, fp32, eval() + no_grad() exactly as
     `adbench_wrapper.py:422-424`, all host threads: the reference's OWN unmodified `nf4ad.flows.NonUSFlow` +
     `nf4ad.transforms.MaskedAffineCoupling` (snapshot `oracle/_ref`, kind "reference") -- or, if the snapshot is missing,
     the oracle's restatement of them (kind "port") -- on the oracle's `src.usflows` / `pyro` shim (the genuine USFlows /
     pyro packages are not installable: no network, un-vendored, un-pinned).  3 warm-ups, median of >= 10 repeats with
-    perf_counter (BASELINE.md section 3).  -> (samples/s from the median, cores, median ms, kind)"""
+    perf_counter (BASELINE.md section 3).  -> (samples/s from the median, cores, median ms, kind, last step's log_prob)"""
     import oracle
     kind = "reference" if oracle.ref_available() else "port"
     ns = oracle.load_ref() if kind == "reference" else oracle.load()
@@ -297,11 +320,11 @@ def cpu_reference_run(steps, warmup, rows, config=DEFAULT_CONFIG):
         ts = []
         for _ in range(steps):
             t0 = time.perf_counter()
-            flow.log_prob(x)
+            lp = flow.log_prob(x)
             ts.append(time.perf_counter() - t0)
     ts.sort()
     med = ts[len(ts) // 2] if len(ts) % 2 else 0.5 * (ts[len(ts) // 2 - 1] + ts[len(ts) // 2])
-    return rows / med, cores, med * 1e3, kind
+    return rows / med, cores, med * 1e3, kind, lp
 
 
 def reference_train_run(device, rows, steps, warmup, config=DEFAULT_CONFIG):
@@ -397,7 +420,11 @@ def main():
     ap.add_argument("--config", default=DEFAULT_CONFIG, choices=sorted(CONFIGS), help="BASELINE.json config shape to bench")
     ap.add_argument("--no-configs", dest="configs", action="store_false", help="skip the short per-config lines")
     ap.add_argument("--no-sweep", dest="sweep", action="store_false", help="skip the batch-size sweep")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the log_prob the last timed step returned to DIR/log_prob.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
     # a run that stops making progress (a collective waiting for a rank that died, a hung teardown) must not sit on the
     # GPUs: after USF_BENCH_TIMEOUT_S seconds every thread's stack goes to stderr and the process exits non-zero
@@ -427,8 +454,10 @@ def main():
         budget_s = 240.0
         if (args.steps + args.warmup) * t_probe > budget_s:
             rows = max(1024, int(rows * budget_s / ((args.steps + args.warmup) * t_probe)) // 1024 * 1024)
-        v, cores, ms, kind = cpu_reference_run(args.steps, args.warmup, rows, args.config)
-        v32, _, ms32, _ = cpu_reference_run(max(args.steps, 10), 3, CPU_SMALL_ROWS, args.config)
+        v, cores, ms, kind, lp = cpu_reference_run(args.steps, args.warmup, rows, args.config)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, {"log_prob": lp})
+        v32, _, ms32, _, _ = cpu_reference_run(max(args.steps, 10), 3, CPU_SMALL_ROWS, args.config)
         line = {"impl": "reference", "metric": "log_prob samples/sec", "value": v, "unit": "samples/s",
                 "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup, "ms_per_step": ms,
                 "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f32",
@@ -538,6 +567,8 @@ def main():
         fpr_main = flow._stack(True, dev, eff_main).flops_per_row()
         assert launches_per_step > 0, "fused CUDA path did not run"
         assert bool(torch.isfinite(lp).all())
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, {"log_prob" if world == 1 else f"log_prob_rank{rank}": lp}, world)
 
         # ---- end to end through the public API: pinned host rows -> H2D -> log_prob -> scores D2H, every step
         # (the call sequence of ADBenchFlow.predict_score, adbench_wrapper.py:419-433) + score gather to rank 0
@@ -879,8 +910,8 @@ def main():
                     "note": "the reference's own batch size (adbench_wrapper.py:310), bf16 tier, one CUDA-graph replay per step"}
         if world == 1 and not args.no_cpu_baseline:
             # BASELINE.md section 3: B = 65536 (and 32), 3 warm-ups, median of 10 -- about 30 s of host work
-            v, cores, cms, kind = cpu_reference_run(10, 3, CPU_ROWS, args.config)
-            v32, _, cms32, _ = cpu_reference_run(10, 3, CPU_SMALL_ROWS, args.config)
+            v, cores, cms, kind, _ = cpu_reference_run(10, 3, CPU_ROWS, args.config)
+            v32, _, cms32, _, _ = cpu_reference_run(10, 3, CPU_SMALL_ROWS, args.config)
             line["cpu_baseline"] = {"value": v, "unit": "samples/s", "cores": cores, "kind": kind,
                                     "sample": f"{CPU_ROWS} rows per step, 3 warm-ups, median of 10 steps ({cms:.0f} ms), fp32, "
                                               f"{cores} threads; the reference's own NonUSFlow + MaskedAffineCoupling "

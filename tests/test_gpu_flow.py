@@ -654,6 +654,40 @@ def test_full_size_properties_c2(O, P):
         assert float(lp_err(lp32, ref).max()) < FP32_TOL
 
 
+def test_bench_dump_outputs_are_the_timed_log_prob(O, P, tmp_path):
+    """`bench.py --dump-outputs DIR`: DIR/log_prob.npy is the float32 log_prob the timed steps return for the seeded
+    benchmark rows -- the same in two runs with the same arguments, the same as this process computes with the bench's
+    flow, and within the tier's tolerance of the fp64 oracle.  Run at the fp32-grade bf16x2 tier: each packing of the
+    weights may move a few bf16 roundings, which in the bf16 tier changes log_prob by up to ~3e-3 from run to run."""
+    import json
+    import subprocess
+    import sys
+    import bench
+    rows = 4096
+    cmd = [sys.executable, bench.__file__, "--steps", "3", "--warmup", "3", "--rows", str(rows), "--precision", "bf16x2",
+           "--prewarm-s", "0", "--train-steps", "0", "--no-cpu-baseline", "--no-configs", "--no-sweep"]
+    dumps = []
+    for run in range(2):
+        out = tmp_path / f"run{run}"
+        r = subprocess.run(cmd + ["--dump-outputs", str(out)], capture_output=True, text=True, timeout=600, cwd=tmp_path)
+        assert r.returncode == 0, r.stderr[-2000:]
+        j = json.loads([l for l in r.stdout.splitlines() if l.startswith("{")][-1])
+        assert j["steps"] == 3 and j["config"]["rows_per_gpu"] == rows
+        assert sorted(p.name for p in out.iterdir()) == ["log_prob.npy"]
+        lp = np.load(out / "log_prob.npy")
+        assert lp.dtype == np.float32 and lp.shape == (rows,) and np.isfinite(lp).all()
+        dumps.append(torch.from_numpy(lp))
+    assert rel(dumps[1], dumps[0]) < FP32_TOL
+    fp = bench.build_flow(P, "cuda")
+    fp.precision = "bf16x2"
+    x = torch.randn(rows, 784, generator=torch.Generator().manual_seed(42))
+    with torch.no_grad():
+        assert rel(dumps[0], fp.log_prob(x.cuda())) < FP32_TOL and fp.effective_precision == "bf16x2"
+        fo = bench.build_flow(O, "cpu").double()
+        fo.load_state_dict({k: v.double().cpu() for k, v in fp.state_dict().items()})
+        assert float(lp_err(dumps[0][:256], fo.log_prob(x[:256].double())).max()) < FP32_TOL
+
+
 @pytest.mark.parametrize("tier,tol", [("tf32x3", 2e-4), ("bf16x2", 1e-4)])
 def test_split_operand_tiers(O, P, tier, tol):
     """The fp32-grade tensor-core tiers: `"tf32x3"` (fp32 operands as tf32 hi + lo, three kind::tf32 MMAs per K step) and

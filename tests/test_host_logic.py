@@ -185,13 +185,36 @@ def test_affine_run_plan_groups_the_layers_between_couplings():
     assert conditioner_weights(torch.nn.Sequential(torch.nn.Tanh()), cpl.mask) is None      # opaque conditioner
 
 
-def test_bench_reference_arm_contract():
-    """`bench.py --impl reference` (the driver's reference arm): rank 0 prints ONE JSON line with the contract's keys --
+def test_bench_dump_outputs_sample_past_the_limit(tmp_path, monkeypatch):
+    """`bench.py --dump-outputs`: float32 files (float64 stays float64); past the byte limit every array keeps the same
+    seeded sample of its rows, in order, so that two runs -- and the arrays of one run -- stay aligned entry for entry."""
+    import numpy as np
+    import bench
+    monkeypatch.setattr(bench, "DUMP_LIMIT_BYTES", 4000)
+    a = torch.arange(1000, dtype=torch.float64)
+    b = torch.arange(2000, dtype=torch.float32).reshape(1000, 2)
+    for run in ("r0", "r1"):
+        bench.dump_outputs(str(tmp_path / run), {"a": a, "b": b})
+    ra, rb = np.load(tmp_path / "r0" / "a.npy"), np.load(tmp_path / "r0" / "b.npy")
+    assert ra.dtype == np.float64 and rb.dtype == np.float32 and 0 < ra.nbytes + rb.nbytes <= 4000
+    assert np.all(np.diff(ra) > 0) and np.array_equal(rb[:, 0], 2 * ra)
+    assert np.array_equal(ra, np.load(tmp_path / "r1" / "a.npy")) and np.array_equal(rb, np.load(tmp_path / "r1" / "b.npy"))
+    bench.dump_outputs(str(tmp_path / "small"), {"c": torch.arange(10, dtype=torch.bfloat16)})
+    c = np.load(tmp_path / "small" / "c.npy")
+    assert c.dtype == np.float32 and np.array_equal(c, np.arange(10))
+
+
+def test_bench_reference_arm_contract(tmp_path):
+    """`bench.py --impl reference` (the CPU reference arm): rank 0 prints ONE JSON line with the contract's keys --
     `impl`, BASELINE.json's metric / unit, a `cpu_baseline` describing this very run (`kind` "reference" when the
-    `oracle/_ref` snapshot exists, else "port"), an `e2e` that moves no bytes -- and every other rank exits 0 silently."""
+    `oracle/_ref` snapshot exists, else "port"), an `e2e` that moves no bytes, and with `--dump-outputs` the log_prob of
+    its last timed step on the seeded rows -- and every other rank exits 0 silently."""
     import json
+    import numpy as np
+    import bench
+    import oracle
     cmd = [sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--gpus", "2", "--steps", "2", "--warmup", "3",
-           "--rows", "1024", "--config", "C4-adbench-D64"]
+           "--rows", "1024", "--config", "C4-adbench-D64", "--dump-outputs", str(tmp_path)]
     env = dict(os.environ, RANK="0", WORLD_SIZE="2", LOCAL_RANK="0", OMP_NUM_THREADS="4")
     r = subprocess.run(cmd, capture_output=True, text=True, timeout=600, env=env, cwd=ROOT)
     assert r.returncode == 0, r.stderr[-2000:]
@@ -205,6 +228,13 @@ def test_bench_reference_arm_contract():
     assert cb["kind"] in ("reference", "port") and cb["cores"] >= 1 and cb["value"] == j["value"] and "1024 rows" in cb["sample"]
     assert j["e2e"] == {"value": j["value"], "unit": "samples/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
     assert "C4-adbench-D64" in j["config"]["workload"] and "model" not in j["config"]
+    lp = np.load(tmp_path / "log_prob.npy")
+    assert lp.dtype == np.float32 and lp.shape == (1024,)
+    ns = oracle.load_ref() if cb["kind"] == "reference" else oracle.load()
+    with torch.no_grad():
+        want = bench.build_config_flow(ns, "C4-adbench-D64", "cpu").log_prob(
+            torch.randn(1024, 64, generator=torch.Generator().manual_seed(42)))
+    np.testing.assert_allclose(lp, want.numpy(), rtol=1e-5, atol=1e-5)
     # the other ranks of a torchrun launch: no work, no output, exit 0
     r1 = subprocess.run(cmd, capture_output=True, text=True, timeout=600, env=dict(env, RANK="1", LOCAL_RANK="1"), cwd=ROOT)
     assert r1.returncode == 0 and r1.stdout.strip() == ""
