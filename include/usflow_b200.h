@@ -295,6 +295,36 @@ int usf_stack_run_bf16in(const usf_stack_desc* st, const uint16_t* x_bf16, int64
                          float* out_y, int64_t ldy, float* out_ladj, void* workspace, size_t workspace_bytes,
                          int* gpu_launches, usf_stream_t stream);
 
+/* ---- input gradient of log p: log p(x) and d log p(x) / dx per row in one call ---------------------------------------
+ * The reverse (vector-Jacobian) chain of an inverse-direction stack, with the weights treated as constants.  It needs
+ * every matrix of the chain transposed: for a forward layer W (N x K) a `usf_linear_desc` T with T.N = round_up(K, 16)
+ * rows holding W^T (zero in the padded rows), T.K = N, T.ldw = N, bias unused (NULL).  T.W (fp32) is read by
+ * USF_PREC_FP32, T.Wb (2 T.N bf16 rows: hi, then lo = bf16(W^T - hi) computed from fp32) by USF_PREC_BF16X2. */
+typedef struct {
+  usf_linear_desc G;                  /* G_j^T */
+  usf_linear_desc mlp[USF_MAX_MLP];   /* conditioner layer l transposed */
+} usf_block_grad_desc;
+
+typedef struct {
+  int32_t n_blocks;                     /* == usf_stack_desc.n_blocks */
+  const usf_block_grad_desc* blocks;    /* HOST pointer to n_blocks descriptors, in the stack's execution order */
+  usf_linear_desc G_final;              /* G_final^T */
+} usf_stack_grad_desc;
+
+/* Workspace bytes usf_stack_log_prob_grad needs for up to B rows (0 on a bad descriptor).  Rows are processed in chunks
+ * of at most 16384, so the size stops growing there. */
+size_t usf_stack_grad_workspace_bytes(const usf_stack_desc* st, const usf_stack_grad_desc* gd, int64_t B, int precision);
+
+/* log p(x) (out_logprob, (B)) and g = d log p(x) / dx (out_grad, (B, D) with leading dimension ldg) of an inverse-direction
+ * stack with a base density, x:(B, D + ctx_dim).  precision: USF_PREC_FP32 (SIMT chain) or USF_PREC_BF16X2.  A forward
+ * chain that keeps every block's output row and hidden activations is followed by the reverse chain on the same GEMM
+ * kernels.  No atomics touch the gradient (bit-identical run to run); out_logprob follows usf_set_deterministic as in
+ * usf_stack_run and equals its result bit for bit in deterministic mode at the same precision on the launch chain.  The
+ * context gradient is not formed.  gpu_launches (optional) receives the number of kernels enqueued. */
+int usf_stack_log_prob_grad(const usf_stack_desc* st, const usf_stack_grad_desc* gd, const float* x, int64_t ldx, int64_t B,
+                            float* out_logprob, float* out_grad, int64_t ldg, void* workspace, size_t workspace_bytes,
+                            int precision, int* gpu_launches, usf_stream_t stream);
+
 /* HOST function (no CUDA call): dst[r, c] = bf16(src[r, c]), round-to-nearest-even, NaN -> 0x7FFF -- the bit pattern the
  * device conversion produces.  src/dst are host pointers (pinned or not), leading dimensions in elements; `threads`
  * host threads of a persistent pool (<= 0: all hardware threads).  Calls are serialised. */

@@ -36,6 +36,14 @@ class StackDesc(C.Structure):
                 ("ctx_dim", _i32)]
 
 
+class BlockGradDesc(C.Structure):
+    _fields_ = [("G", LinearDesc), ("mlp", LinearDesc * USF_MAX_MLP)]
+
+
+class StackGradDesc(C.Structure):
+    _fields_ = [("n_blocks", _i32), ("blocks", C.POINTER(BlockGradDesc)), ("G_final", LinearDesc)]
+
+
 # name -> (restype, argtypes); mirrors include/usflow_b200.h one to one
 _PROTOS = {
     "usf_version": (_int, []),
@@ -83,6 +91,9 @@ _PROTOS = {
     "usf_set_deterministic": (_int, [_int]),
     "usf_stack_run": (_int, [C.POINTER(StackDesc), _vp, _i64, _i64, _vp, _vp, _i64, _vp, _vp, _sz, _int,
                              C.POINTER(_int), _vp]),
+    "usf_stack_grad_workspace_bytes": (_sz, [C.POINTER(StackDesc), C.POINTER(StackGradDesc), _i64, _int]),
+    "usf_stack_log_prob_grad": (_int, [C.POINTER(StackDesc), C.POINTER(StackGradDesc), _vp, _i64, _i64, _vp, _vp, _i64,
+                                       _vp, _sz, _int, C.POINTER(_int), _vp]),
     "usf_profile_begin": (_int, [_int]),
     "usf_profile_end": (_int, [C.POINTER(_f32), C.POINTER(_int), C.POINTER(_int)]),
     "usf_debug_graph_stats": (_int, [C.POINTER(C.c_longlong), C.c_char_p, _int]),

@@ -94,6 +94,18 @@ class ADBenchFlow:
         # the PCIe copy and the compute -- no whole-array pin_memory() copy
         return scorer.predict_score_host(X).numpy()
 
+    def score_gradients(self, X_test: np.ndarray, chunk_rows: int = 65536) -> np.ndarray:
+        """Gradient of the anomaly score with respect to the input, -d log p(x) / dx, shape of X_test: which features make
+        a sample anomalous.  Rows go to the device `chunk_rows` at a time (`Flow.log_prob_and_grad`)."""
+        with torch.cuda.device(self.device):
+            X = torch.as_tensor(np.asarray(X_test), dtype=torch.float32)
+            self.flow_model.eval()
+            out = np.empty(tuple(X.shape), dtype=np.float32)
+            for i in range(0, X.shape[0], chunk_rows):
+                _, g = self.flow_model.log_prob_and_grad(X[i:i + chunk_rows].to(self.device))
+                out[i:i + chunk_rows] = (-g).cpu().numpy()
+            return out
+
     def predict(self, X_test: np.ndarray, threshold: Optional[float] = None) -> np.ndarray:
         """1 = anomaly.  Default threshold: median score (adbench_wrapper.py:435-449)."""
         scores = self.predict_score(X_test)

@@ -9,7 +9,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIBDIR = os.path.join(HERE, "lib")
 LIB = os.path.join(LIBDIR, "libusflow_b200.so")
-SOURCES = ["usf_api.cu", "usf_simt.cu", "usf_tc.cu", "usf_trsm.cu", "usf_small.cu", "usf_host.cpp"]
+SOURCES = ["usf_api.cu", "usf_simt.cu", "usf_tc.cu", "usf_trsm.cu", "usf_small.cu", "usf_grad.cu", "usf_host.cpp"]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
          "-Xcompiler", "-fPIC", "-Xptxas", "-v"]

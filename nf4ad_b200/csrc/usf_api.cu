@@ -85,6 +85,12 @@ inline int det_slots_of(int precision, int64_t N, int bn, bool fused) {
 // a scratch area and one last kernel adds the slots in order, instead of fp32 atomics whose order varies run to run.
 thread_local int g_deterministic = 0;
 
+}  // namespace
+
+int deterministic_mode() { return g_deterministic; }
+
+namespace {
+
 constexpr int64_t kChunkRows = 131072;  // rows pushed through the stack per pass (bounds the workspace)
 constexpr int64_t kSmallRows = 2048;    // fp32 path: batches up to this size may use the split-K + epilogue-kernel GEMM form
 

@@ -39,6 +39,7 @@ __host__ __device__ static inline int64_t ceil_div(int64_t a, int64_t b) { retur
 __host__ __device__ static inline int64_t round_up(int64_t a, int64_t b) { return ceil_div(a, b) * b; }
 
 int num_sms();
+int deterministic_mode();   // usf_set_deterministic of the calling thread
 
 // ---- epilogue description shared by the SIMT and the tcgen05 GEMM kernels --------------------
 // The GEMM computes acc[m, n] = sum_k A[m,k] * W[n,k]; the epilogue turns one accumulator tile into

@@ -119,6 +119,7 @@ class Flow(torch.nn.Module):
         # tensor-core training: compose the affine runs between couplings in weight space (`_compose_affine_runs`)
         self.compose_affine = os.environ.get("USF_COMPOSE_AFFINE", "1") != "0"
         self.last_launches = 0                  # kernels enqueued by the last fused call
+        self.last_grad_precision = None         # tier of the last log_prob_and_grad: "bf16x2", "fp32" or "autograd"
         self._compiled = {}
         self._key_slots = None
         # the reference builds its flows with `device=...` and then scores device tensors without an explicit `.to()`
@@ -333,13 +334,14 @@ class Flow(torch.nn.Module):
             xin = None
         return self._tier(x2, xin)
 
-    def _stack(self, inverse, device, precision=None):
-        """Compiled (packed) stack for this direction / precision / weight version, or None."""
+    def _stack(self, inverse, device, precision=None, grad=False):
+        """Compiled (packed) stack for this direction / precision / weight version, or None.  `grad`: the inverse stack
+        with the transposed matrices of the reverse chain as well (`log_prob_and_grad`)."""
         precision = precision or self.precision
         if precision == "auto":
             precision = self.FP32_GRADE_TC if self.event_dim >= self.BF16_MIN_DIM else "fp32"
         prec = _PRECISIONS[precision]
-        slot = (bool(inverse), prec)
+        slot = ("grad", prec) if grad else (bool(inverse), prec)
         key = (self._weights_key(), str(device))
         hit = self._compiled.get(slot)
         if hit is not None and hit[0] == key:
@@ -347,7 +349,7 @@ class Flow(torch.nn.Module):
         try:
             if len(self.event_shape) != 1:
                 raise stack.Unsupported("image-shaped event: the layer-wise kernels are used")
-            cs = stack.CompiledStack(self.layers, self.base_distribution, self.event_dim, device, inverse, prec)
+            cs = stack.CompiledStack(self.layers, self.base_distribution, self.event_dim, device, inverse, prec, grad=grad)
         except stack.Unsupported as e:
             cs = None
             self._unsupported_reason = str(e)
@@ -415,6 +417,54 @@ class Flow(torch.nn.Module):
             z, neg_ladj = self._inverse_layers(self._unflat(x2), context)
             lp = self._base_log_prob(z.reshape(z.shape[0], -1)) + neg_ladj
         return lp.reshape(lead)
+
+    @_on_device
+    def log_prob_and_grad(self, x, context=None):
+        """(log p(x), d log p(x) / dx) per row, the weights taken as constants: `lp` has the leading batch shape, `g` the
+        shape of `x` (fp32).  Equal to `torch.autograd.grad(self.log_prob(x).sum(), x)` in exact arithmetic (relu'(0) = 0,
+        sign(0) = 0 for a Laplace base); builds no autograd graph, touches no `p.grad`, works under `torch.no_grad()`.
+        The gradient is the per-feature attribution of the anomaly score -log p (the context gradient is not formed).
+
+        Flat-event stacks run the reverse launch chain of the fused path in one library call: at bf16x2 when the request
+        is "auto" with D >= BF16_MIN_DIM, or "bf16x2" / "bf16" / "tf32x3" (a gradient at bf16 operand precision would be
+        of little use), else on the fp32 SIMT kernels.  Other flows (image-shaped events, opaque conditioners, softplus
+        scales, a context handed to an unconditional flow) differentiate the layer-wise pass with autograd.
+        `last_grad_precision` reports which: "bf16x2", "fp32" or "autograd"."""
+        x2, lead = self._prep(x)
+        ctx = self._soft_context(x2, context)
+        cs, xin = self._grad_stack(x2, ctx)
+        if cs is None:
+            self.last_grad_precision = "autograd"
+            with torch.enable_grad():
+                xr = x.detach().to(torch.float32).requires_grad_(True)
+                lp = self.log_prob(xr, context)
+                g, = torch.autograd.grad(lp.sum(), xr)
+            return lp.detach(), g
+        lp, g, n = cs.run_grad(xin, deterministic=self.deterministic)
+        self.last_grad_precision = "bf16x2" if cs.precision == _lib.USF_PREC_BF16X2 else "fp32"
+        self.last_launches = n
+        return lp.reshape(lead), g.reshape(x.shape)
+
+    def _grad_stack(self, x2, context):
+        """-> (compiled stack with its transposed matrices | None, input rows incl. context columns) for
+        `log_prob_and_grad`, by the tier rule there."""
+        cd = self.context_dim()
+        if len(self.event_shape) != 1 or (cd == 0 and context is not None):
+            return None, x2
+        if cd > 0 and context is None:
+            raise ValueError("this flow's conditioners take a context (ConditionalDenseNN): pass `context=` or build the "
+                             "flow with soft_training=True")
+        xin = x2.to(torch.float32)
+        if cd > 0:
+            ctx = context if context.dim() == 2 else context.reshape(-1, cd)
+            xin = torch.cat([xin, ctx.to(torch.float32).expand(x2.shape[0], cd)], dim=1)
+        want = self.precision
+        tc = (want == "auto" and self.event_dim >= self.BF16_MIN_DIM) or want in ("bf16x2", "bf16", "tf32x3")
+        for tier in (("bf16x2", "fp32") if tc else ("fp32",)):
+            cs = self._stack(True, x2.device, tier, grad=True)
+            if cs is not None and cs.ctx_dim == cd and cs.desc.base_kind >= 0:
+                return cs, xin
+        return None, x2
 
     def _prefetch_lu_inverses(self, y):
         """Mixed-precision training: the dense inverses of all LU layers this pass will apply are independent of the
