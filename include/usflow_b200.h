@@ -136,7 +136,8 @@ int usf_base_logprob(int kind, const float* z, int64_t ldz, const float* loc, co
 /* ------------------------------------------------------------------------- */
 
 /* Backward of y = x W^T + b (optionally through relu, given y):
- *   dx = dy W (dx may be NULL), dW (+)= dy^T x, db (+)= colsum(dy).  accumulate != 0 adds. */
+ *   dx = dy W (dx may be NULL), dW (+)= dy^T x, db (+)= colsum(dy).  accumulate != 0 adds.
+ * B == 0 (dy, x, y_relu may then be NULL) still writes dW = 0 and db = 0 when accumulate == 0. */
 int usf_linear_bwd(const float* dy, int64_t lddy, const float* x, int64_t ldx, const float* W,
                    int64_t ldw, const float* y_relu, int64_t ldyr, float* dx, int64_t lddx, float* dW,
                    int64_t lddw, float* db, int accumulate, float* scratch, int64_t B, int64_t N,

@@ -1327,7 +1327,7 @@ extern "C" int usf_to_tf32x3(const float* x, int64_t ldx, const float* relu_mask
 
 extern "C" int usf_linear(const float* x, int64_t ldx, const float* W, int64_t ldw, const float* bias, int relu,
                           float* y, int64_t ldy, int64_t B, int64_t N, int64_t K, usf_stream_t stream) {
-  USF_CHECK_ARG(x && W && y, "usf_linear: null pointer");
+  USF_CHECK_ARG(W && ((x && y) || B == 0), "usf_linear: null pointer");   // (an empty batch may come with NULL rows)
   USF_CHECK_ARG(B >= 0 && N > 0 && K > 0 && ldx >= K && ldw >= K && ldy >= N, "usf_linear: bad sizes");
   if (B > 0 && K >= 64 && ceil_div(B, BM) * ceil_div(N, BN) * 2 <= num_sms()) {
     // small problem: split-K GEMM (atomic partial sums) + a bias/activation pass, instead of a few serial tiles
@@ -1440,10 +1440,12 @@ extern "C" int usf_linear_bwd(const float* dy, int64_t lddy, const float* x, int
                               int64_t ldw, const float* y_relu, int64_t ldyr, float* dx, int64_t lddx, float* dW,
                               int64_t lddw, float* db, int accumulate, float* scratch, int64_t B, int64_t N,
                               int64_t K, usf_stream_t stream) {
-  USF_CHECK_ARG(dy && B >= 0 && N > 0 && K > 0, "usf_linear_bwd: bad arguments");
-  USF_CHECK_ARG(!(dx && !W) && !(dW && !x), "usf_linear_bwd: dx needs W, dW needs x");
+  // an empty batch may come with NULL rows (dy, x); it still defines dW = 0 and db = 0 when accumulate == 0, so it runs
+  // through the same steps: the dgrad GEMM returns at M = 0, the wgrad GEMM stores (or adds) a K = 0 product, the
+  // column sum clears its output before it looks at B
+  USF_CHECK_ARG((dy || B == 0) && B >= 0 && N > 0 && K > 0, "usf_linear_bwd: bad arguments");
+  USF_CHECK_ARG(!(dx && !W) && !(dW && !x && B > 0), "usf_linear_bwd: dx needs W, dW needs x");
   USF_CHECK_ARG(!(y_relu && !scratch), "usf_linear_bwd: relu backward needs scratch");
-  if (B == 0) return USF_OK;
   cudaStream_t st = as_stream(stream);
   const float* g = dy;
   int64_t ldg = lddy;

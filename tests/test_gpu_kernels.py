@@ -82,7 +82,8 @@ def test_householder_scale(ops, O, D, nvs):
     assert relerr(ops.scale(x.float().cuda(), s.float().cuda(), True), x / s) < 1e-6
 
 
-@pytest.mark.parametrize("D,affine", [(7, True), (64, True), (785, True), (20, False)])
+# D = 2600: more columns than the base density kernel stages in shared memory (2048)
+@pytest.mark.parametrize("D,affine", [(7, True), (64, True), (785, True), (20, False), (2600, True)])
 def test_coupling_and_base(ops, D, affine):
     torch.manual_seed(D)
     B = 37
@@ -91,13 +92,20 @@ def test_coupling_and_base(ops, D, affine):
     t = torch.randn(B, D, dtype=torch.float64)
     m = (torch.arange(D) % 2).double()
     ls = 5.0 * torch.tanh(s) if affine else torch.zeros_like(s)
-    for inverse in (False, True):
-        ref = x * m + (1 - m) * ((x - t) * torch.exp(-ls) if inverse else x * torch.exp(ls) + t)
-        ladj_ref = ((1 - m) * ls).sum(1)
-        y, ladj = ops.coupling(x.float().cuda(), s.float().cuda() if affine else None, t.float().cuda(),
-                               m.float().cuda(), 5.0, inverse)
-        assert relerr(y, ref) < 1e-5
-        assert float((ladj.double().cpu() - ladj_ref).abs().max()) < 1e-4 * max(1.0, float(ladj_ref.abs().max()))
+    for act in (0, 1):
+        if act == 0 or not affine:       # the additive form has no scale: the activation does not apply
+            sc, inv_sc, lsc = torch.exp(ls), torch.exp(-ls), ls
+        else:                            # softplus, with the reference's literal 1e-6 / 1e-12
+            sp = torch.nn.functional.softplus(ls)
+            sc, lsc = sp + 1e-6, torch.log(sp + 1e-12)
+            inv_sc = 1.0 / (sc + 1e-12)
+        for inverse in (False, True):
+            ref = x * m + (1 - m) * ((x - t) * inv_sc if inverse else x * sc + t)
+            ladj_ref = ((1 - m) * lsc).sum(1)
+            y, ladj = ops.coupling(x.float().cuda(), s.float().cuda() if affine else None, t.float().cuda(),
+                                   m.float().cuda(), 5.0, inverse, act)
+            assert relerr(y, ref) < 1e-5, (act, inverse)
+            assert float((ladj.double().cpu() - ladj_ref).abs().max()) < 1e-4 * max(1.0, float(ladj_ref.abs().max()))
     loc = torch.randn(D, dtype=torch.float64)
     for kind, dist in ((0, torch.distributions.Normal), (1, torch.distributions.Laplace)):
         for scale in (torch.rand(D, dtype=torch.float64) + 0.5, torch.tensor([1.7], dtype=torch.float64)):
@@ -273,22 +281,22 @@ def test_vae_latent_tail_kernels():
         mu = torch.randn(B, L, generator=g).cuda().requires_grad_()
         lv = (0.5 * torch.randn(B, L, generator=g)).cuda().requires_grad_()
         eps = torch.randn(B, L, generator=g).cuda()
-        x = torch.randn(B, *img, generator=g).cuda()
+        x = torch.randn(B, *img, generator=g).cuda().requires_grad_()
         xr = torch.randn(B, *img, generator=g).cuda().requires_grad_()
         wz = torch.randn(B, L, generator=g).cuda()
         wq, wn = torch.randn(B, generator=g).cuda(), torch.randn(B, generator=g).cuda()
         z, log_q = vae.reparameterize(mu, lv, eps)
         nll = vae.recon_nll(x, xr, 0.1)
         ((z * wz).sum() + (log_q * wq).sum() + (nll * wn).sum()).backward()
-        mud, lvd, xrd = (t.detach().double().requires_grad_() for t in (mu, lv, xr))
+        mud, lvd, xd, xrd = (t.detach().double().requires_grad_() for t in (mu, lv, x, xr))
         std = torch.exp(0.5 * lvd)
         zd = mud + eps.double() * std
         lqd = torch.distributions.Normal(mud, std).log_prob(zd).view(B, -1).sum(1)
         D = x[0].numel()
-        nlld = 0.5 * ((x.double() - xrd) ** 2).view(B, -1).sum(1) / 0.01 + 0.5 * D * math.log(2 * math.pi * 0.01)
+        nlld = 0.5 * ((xd - xrd) ** 2).view(B, -1).sum(1) / 0.01 + 0.5 * D * math.log(2 * math.pi * 0.01)
         ((zd * wz.double()).sum() + (lqd * wq.double()).sum() + (nlld * wn.double()).sum()).backward()
         for got, ref, name in ((z, zd, "z"), (log_q, lqd, "log_q"), (nll, nlld, "nll"), (mu.grad, mud.grad, "dmu"),
-                               (lv.grad, lvd.grad, "dlogvar"), (xr.grad, xrd.grad, "dx_recon")):
+                               (lv.grad, lvd.grad, "dlogvar"), (xr.grad, xrd.grad, "dx_recon"), (x.grad, xd.grad, "dx")):
             assert relerr(got, ref) < 2e-5, (B, L, name, relerr(got, ref))
     # log q evaluated through the reparameterised z has no gradient path to mu (z - mu = eps std): dmu == dz exactly
     mu = torch.randn(4, 8).cuda().requires_grad_()
