@@ -1,5 +1,6 @@
 // Host side of the C ABI: error plumbing, device probe, and the fused-stack runner that turns a packed
-// layer-descriptor array into one launch chain (Flow.log_prob / Flow.backward / Flow.forward).
+// layer-descriptor array into one launch chain (Flow.log_prob / Flow.backward / Flow.forward, and the forward half of
+// usf_stack_log_prob_grad).
 #include <stdarg.h>
 #include <stdlib.h>
 
@@ -74,13 +75,6 @@ struct StackPlan {
   size_t total;
 };
 
-// partial-sum slots one accumulating launch uses (the `sub` range of row_accumulate in its kernel)
-inline int det_slots_of(int precision, int64_t N, int bn, bool fused) {
-  if (fused) return 4;                                                       // MLP_EPI_PARTS warps per row
-  if (precision == USF_PREC_FP32) return (int)ceil_div(N, 128);              // SIMT tile: 128 columns per blockIdx.y
-  return 2 * (int)ceil_div(N, bn);                                           // tcgen05 kernels: 2 epilogue warps per N tile
-}
-
 // Deterministic mode (usf_set_deterministic, per thread): every per-row partial sum of the chain goes to its own slot of
 // a scratch area and one last kernel adds the slots in order, instead of fp32 atomics whose order varies run to run.
 thread_local int g_deterministic = 0;
@@ -89,12 +83,24 @@ thread_local int g_deterministic = 0;
 
 int deterministic_mode() { return g_deterministic; }
 
+int det_slots(const usf_stack_desc* st, int b, int precision) {
+  // the SIMT kernel: one slot per 128 output columns (blockIdx.y); the tcgen05 kernels: 2 epilogue warps per N tile
+  const bool tc = precision != USF_PREC_FP32;
+  if (b == st->n_blocks)   // (the SIMT kernel stores exactly D columns)
+    return tc ? 2 * (int)ceil_div(st->G_final.N, tc_pick_bn(st->G_final.N)) : (int)ceil_div(st->D, 128);
+  const usf_block_desc& blk = st->blocks[b];
+  if (!blk.affine) return 0;
+  const int64_t N = blk.mlp[blk.n_mlp - 1].N;
+  if (!tc) return (int)ceil_div(N, 128);
+  // the fused bf16 conditioner kernel takes 4 (MLP_EPI_PARTS warps per row): either form of a block takes max(n, 4)
+  const int n = 2 * (int)ceil_div(N, 2 * blk.C);
+  return n > 4 ? n : 4;
+}
+
 namespace {
 
 constexpr int64_t kChunkRows = 131072;  // rows pushed through the stack per pass (bounds the workspace)
 constexpr int64_t kSmallRows = 2048;    // fp32 path: batches up to this size may use the split-K + epilogue-kernel GEMM form
-
-inline size_t align256(size_t v) { return (v + 255) & ~size_t(255); }
 
 int plan_stack(const usf_stack_desc* st, int64_t rows, int precision, StackPlan* p) {
   USF_CHECK_ARG(st != nullptr && st->D > 0 && st->n_blocks >= 0 && st->ctx_dim >= 0, "stack: bad descriptor");
@@ -123,18 +129,8 @@ int plan_stack(const usf_stack_desc* st, int64_t rows, int precision, StackPlan*
   p->small_bytes = (precision == USF_PREC_FP32 && rows <= kSmallRows && !g_deterministic)
                        ? align256((size_t)rows * (size_t)nmax * sizeof(float)) : 0;   // (split-K sums atomically: not in deterministic mode)
   p->det_slots = 0;
-  if (g_deterministic) {
-    const bool tc = precision != USF_PREC_FP32;
-    for (int b = 0; b < st->n_blocks; ++b) {
-      const usf_block_desc& blk = st->blocks[b];
-      if (!blk.affine) continue;                                  // additive couplings add nothing to the row sums
-      const usf_linear_desc& L = blk.mlp[blk.n_mlp - 1];
-      p->det_slots += tc ? (2 * (int)ceil_div(L.N, 2 * blk.C) > 4 ? 2 * (int)ceil_div(L.N, 2 * blk.C) : 4)
-                         : det_slots_of(precision, L.N, 0, false);
-    }
-    p->det_slots += tc ? det_slots_of(precision, st->G_final.N, tc_pick_bn(st->G_final.N), false)
-                       : det_slots_of(precision, st->D, 0, false);
-  }
+  if (g_deterministic)
+    for (int b = 0; b <= st->n_blocks; ++b) p->det_slots += det_slots(st, b, precision);
   p->det_bytes = align256((size_t)p->det_slots * (size_t)rows * sizeof(float));
   // 3xTF32 / bf16x2: every activation buffer has a low-part twin
   const size_t twins = (precision == USF_PREC_TF32X3 || precision == USF_PREC_BF16X2) ? 2 : 1;
@@ -143,6 +139,191 @@ int plan_stack(const usf_stack_desc* st, int64_t rows, int precision, StackPlan*
 }
 
 }  // namespace
+
+int chain_gemm(int precision, const Buf& A, const usf_linear_desc& L, int64_t rows, int64_t N, int bn,
+               const EpiParams& ep, void* out_lo, void* ub_lo, float* scratch, size_t scratch_floats, cudaStream_t s) {
+  const bool f32w = precision == USF_PREC_FP32 || precision == USF_PREC_TF32X3;
+  USF_CHECK_ARG(f32w ? L.W != nullptr : L.Wb != nullptr, "stack: %s weights missing in descriptor", f32w ? "fp32" : "bf16");
+  if (precision == USF_PREC_FP32)
+    return simt_gemm(static_cast<const float*>(A.hi), A.ld, 0, L.W, L.ldw, 0, rows, N, L.K, ep, s, scratch, scratch_floats);
+  if (bn == 0) bn = tc_pick_bn(N);
+  const size_t lo = (size_t)L.N * (size_t)L.ldw;   // the low-part rows follow the N high-part rows
+  if (precision == USF_PREC_BF16)
+    return tc_gemm(static_cast<const uint16_t*>(A.hi), A.ld, L.Wb, L.ldw, rows, N, L.K, bn, ep, s);
+  if (precision == USF_PREC_TF32X3)
+    return tc3_gemm(static_cast<const float*>(A.hi), static_cast<const float*>(A.lo), A.ld, L.W, L.W + lo, L.ldw, rows, N,
+                    L.K, bn, ep, static_cast<float*>(out_lo), static_cast<float*>(ub_lo), s);
+  return tcb2_gemm(static_cast<const uint16_t*>(A.hi), static_cast<const uint16_t*>(A.lo), A.ld, L.Wb, L.Wb + lo, L.ldw,
+                   rows, N, L.K, bn, ep, static_cast<uint16_t*>(out_lo), static_cast<uint16_t*>(ub_lo), s);
+}
+
+int run_chain(const usf_stack_desc* st, const void* x, int64_t ldx, bool x_bf16, int64_t rows, int precision,
+              const ChainIO& io, int* launches, cudaStream_t s) {
+  const bool bf16 = precision == USF_PREC_BF16;
+  const bool b2 = precision == USF_PREC_BF16X2;      // bf16 (hi, lo) operand pairs
+  const bool t3 = precision == USF_PREC_TF32X3;
+  const size_t esz = (bf16 || b2) ? 2 : 4;
+  const int64_t d_in = (int64_t)st->D + st->ctx_dim;   // input row = D coordinates + the context columns
+  // deterministic mode: the accumulating launches store into consecutive slots instead of adding atomically
+  float* det = io.row_acc != nullptr ? io.det : nullptr;
+  int det_cursor = 0;
+  auto det_assign = [&](EpiParams& ep, int n) {
+    if (det == nullptr || n == 0) return;
+    ep.row_part = det;
+    ep.part_ld = rows;
+    ep.part_slot = det_cursor;
+    det_cursor += n;
+  };
+  // Serpentine tile order (bf16 tier): every tensor-core kernel of the chain walks the row tiles in the opposite
+  // direction of its predecessor, so that it starts on the rows that kernel wrote last and that are still in L2
+  // (usf_tc.cu: tc_set_tile_order).  The input pack walks first -> last, so the first GEMM starts reversed.
+  static const bool serpentine = []() { const char* e = getenv("USF_TC_SERPENTINE"); return !(e != nullptr && e[0] == '0'); }();
+  int flip = 1;
+  auto next_order = [&]() { tc_set_tile_order(serpentine ? flip : 0); flip ^= 1; };
+  struct OrderReset { ~OrderReset() { tc_set_tile_order(0); } } order_reset;   // stand-alone GEMM calls stay first -> last
+  auto gemm = [&](const Buf& A, const usf_linear_desc& L, int64_t N, int bn, const EpiParams& ep, void* out_lo,
+                  void* ub_lo) {
+    if (bf16) next_order();
+    return chain_gemm(precision, A, L, rows, N, bn, ep, out_lo, ub_lo, io.scratch, io.scratch_floats, s);
+  };
+  int rc;
+
+  // stage 0: bring x into the activation layout (bf16, or padded fp32) and seed the per-row accumulator
+  if (det != nullptr) USF_CUDA(cudaMemsetAsync(det, 0, (size_t)io.det_n * (size_t)rows * sizeof(float), s));
+  const Buf& a0 = io.act[0];
+  {
+    ProfScope ps(s, 0);
+    if (b2)
+      rc = launch_split_rows_bf16x2(static_cast<const float*>(x), ldx, static_cast<uint16_t*>(a0.hi),
+                                    static_cast<uint16_t*>(a0.lo), a0.ld, rows, d_in, io.row_acc, io.acc_init, s);
+    else if (x_bf16)
+      rc = launch_copy_rows_bf16(static_cast<const uint16_t*>(x), ldx, static_cast<uint16_t*>(a0.hi), a0.ld, rows, d_in,
+                                 io.row_acc, io.acc_init, s);
+    else
+      rc = launch_convert_rows(static_cast<const float*>(x), ldx, bf16 ? static_cast<uint16_t*>(a0.hi) : nullptr,
+                               bf16 ? nullptr : static_cast<float*>(a0.hi), a0.ld, rows, d_in, io.row_acc, io.acc_init, s);
+  }
+  if (rc) return rc;
+  ++*launches;
+  if (t3) {
+    rc = launch_split_lo(static_cast<const float*>(a0.hi), a0.ld, static_cast<float*>(a0.hi), static_cast<float*>(a0.lo),
+                         a0.ld, rows, a0.ld, s);
+    if (rc) return rc;
+    ++*launches;
+  }
+
+  int k = 0;   // hidden activations of the earlier blocks
+  for (int b = 0; b < st->n_blocks; ++b) {
+    const usf_block_desc& blk = st->blocks[b];
+    const Buf& u = io.act[(b + 1) % io.n_act];
+    // (1) dense affine map u = G x + g, written in [a | pad | b] column order
+    {
+      EpiParams ep{};
+      ep.mode = EPI_BIAS;
+      ep.bias = blk.G.bias;
+      ep.out = u.hi;
+      ep.ldo = u.ld;
+      ep.out_bf16 = bf16 || b2;
+      ProfScope ps(s, 1);
+      rc = gemm(io.act[b % io.n_act], blk.G, blk.G.N, 0, ep, u.lo, nullptr);
+    }
+    if (rc) return rc;
+    ++*launches;
+    // (2) conditioner MLP on the a-part, last layer fused with the coupling update of the b-part
+    EpiParams cp{};
+    if (blk.affine) cp.mode = st->inverse ? EPI_COUPLING_INV : EPI_COUPLING_FWD;
+    else cp.mode = st->inverse ? EPI_ADD_INV : EPI_ADD_FWD;
+    cp.ub = static_cast<uint8_t*>(u.hi) + (size_t)blk.b_off * esz;
+    cp.ldub = u.ld;
+    cp.ub_bf16 = bf16 || b2;
+    cp.Db = blk.Db;
+    cp.C = blk.C;
+    cp.clamp = blk.clamp;
+    cp.row_acc = io.row_acc;
+    det_assign(cp, det_slots(st, b, precision));
+    void* ub_lo = u.lo != nullptr ? static_cast<uint8_t*>(u.lo) + (size_t)blk.b_off * esz : nullptr;
+    const int k0 = k;
+    k += blk.n_mlp - 1;
+    if (bf16 && blk.n_mlp >= 2) {
+      int Ns[USF_MAX_MLP], Ks[USF_MAX_MLP], ldws[USF_MAX_MLP];
+      const uint16_t* Wbs[USF_MAX_MLP];
+      const float* biases[USF_MAX_MLP];
+      bool have = true;
+      for (int l = 0; l < blk.n_mlp; ++l) {
+        Ns[l] = blk.mlp[l].N; Ks[l] = blk.mlp[l].K; ldws[l] = blk.mlp[l].ldw;
+        Wbs[l] = blk.mlp[l].Wb; biases[l] = blk.mlp[l].bias;
+        have = have && Wbs[l] != nullptr && biases[l] != nullptr;
+      }
+      if (have && blk.n_mlp <= 4 && tc_mlp_supported(blk.n_mlp, Ns, Ks, blk.Da)) {
+        // ONE kernel: the whole conditioner chain with hidden activations resident in shared memory + coupling
+        next_order();
+        {
+          ProfScope ps(s, 5);
+          rc = tc_mlp_coupling(static_cast<const uint16_t*>(u.hi), u.ld, rows, blk.n_mlp, Wbs, ldws, biases, Ns, Ks,
+                               blk.affine ? 2 * blk.C : blk.C, cp, s);
+        }
+        if (rc) return rc;
+        ++*launches;
+        continue;
+      }
+    }
+    Buf in = u;
+    for (int l = 0; l < blk.n_mlp; ++l) {
+      const usf_linear_desc& L = blk.mlp[l];
+      if (l + 1 < blk.n_mlp) {
+        const Buf& h = io.hid[(k0 + l) % io.n_hid];
+        EpiParams ep{};
+        ep.mode = EPI_BIAS_RELU;
+        ep.bias = L.bias;
+        ep.out = h.hi;
+        ep.ldo = h.ld;
+        ep.out_bf16 = bf16 || b2;
+        ProfScope ps(s, 2);
+        rc = gemm(in, L, L.N, 0, ep, h.lo, nullptr);
+        in = h;
+      } else {
+        cp.bias = L.bias;
+        ProfScope ps(s, 3);
+        rc = gemm(in, L, L.N, blk.affine ? 2 * blk.C : blk.C, cp, nullptr, ub_lo);
+      }
+      if (rc) return rc;
+      ++*launches;
+    }
+  }
+  // (3) last affine map, fused with the base log-density when a density is requested
+  {
+    EpiParams ep{};
+    ep.bias = st->G_final.bias;
+    ep.n_valid = st->D;
+    ep.out = io.out;
+    ep.ldo = io.ldo;
+    ep.out_bf16 = 0;
+    if (io.density) {
+      ep.mode = st->base_kind == 0 ? EPI_BASE_NORMAL : EPI_BASE_LAPLACE;
+      ep.loc = st->loc;
+      ep.inv_scale = st->inv_scale;
+      ep.row_acc = io.row_acc;
+      det_assign(ep, det_slots(st, st->n_blocks, precision));
+    } else {
+      USF_CHECK_ARG(io.out != nullptr, "usf_stack_run: nothing to compute (no output requested)");
+      ep.mode = EPI_BIAS;
+    }
+    // fp32 path: the SIMT kernel stores exactly N = D columns
+    ProfScope ps(s, 4);
+    rc = gemm(io.act[st->n_blocks % io.n_act], st->G_final, precision == USF_PREC_FP32 ? st->D : st->G_final.N, 0, ep,
+              nullptr, nullptr);
+  }
+  if (rc) return rc;
+  ++*launches;
+  // deterministic mode: the slots, added in slot order, on top of the seeded accumulator
+  if (det != nullptr && det_cursor > 0) {
+    rc = launch_sum_row_parts(io.row_acc, det, rows, det_cursor, rows, s);
+    if (rc) return rc;
+    ++*launches;
+  }
+  return USF_OK;
+}
+
 }  // namespace usf
 
 using namespace usf;
@@ -292,239 +473,38 @@ static int stack_run_eager(const usf_stack_desc* st, const float* x, int64_t ldx
     set_error("usf_stack_run: workspace too small (%zu < %zu bytes)", workspace_bytes, p.total);
     return USF_E_WORKSPACE;
   }
-  cudaStream_t s = as_stream(stream);
-  const bool bf16 = precision == USF_PREC_BF16;
-  const bool b2 = precision == USF_PREC_BF16X2;      // bf16 (hi, lo) operand pairs
-  const size_t esz = (bf16 || b2) ? 2 : 4;
-  uint8_t* base = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(workspace) + 255) & ~uintptr_t(255));
-  uint8_t* act[2] = {base, base + p.act_bytes};
-  uint8_t* hid[2] = {base + 2 * p.act_bytes, base + 2 * p.act_bytes + p.hid_bytes};
-  float* small = p.small_bytes ? reinterpret_cast<float*>(base + 2 * p.act_bytes + 2 * p.hid_bytes + p.acc_bytes) : nullptr;
-  const bool t3 = precision == USF_PREC_TF32X3;
-  // low-part twins of the activation / hidden buffers (3xTF32 / bf16x2), placed after the accumulator region
-  uint8_t* lo_base = base + 2 * p.act_bytes + 2 * p.hid_bytes + p.acc_bytes + p.small_bytes;
-  uint8_t* act_lo[2] = {lo_base, lo_base + p.act_bytes};
-  uint8_t* hid_lo[2] = {lo_base + 2 * p.act_bytes, lo_base + 2 * p.act_bytes + p.hid_bytes};
-  auto lo_of = [&](const void* hi) -> float* {   // the twin of one of the four hi buffers (or of a pointer into it)
-    if (!t3 && !b2) return nullptr;
-    const uint8_t* h = reinterpret_cast<const uint8_t*>(hi);
-    return reinterpret_cast<float*>(lo_base + (h - base));
-  };
-  (void)act_lo; (void)hid_lo;
-  // deterministic mode: slot area for the per-row partial sums, after everything else
-  const size_t twins_n = (t3 || b2) ? 2 : 1;
-  float* det = p.det_slots > 0 ? reinterpret_cast<float*>(lo_base + (twins_n - 1) * (2 * p.act_bytes + 2 * p.hid_bytes)) : nullptr;
-  int det_cursor = 0;
-  // points an accumulating launch at its slots (n of them) instead of the atomics
-  auto det_assign = [&](EpiParams& ep, int n, int64_t rows) {
-    if (det == nullptr || ep.row_acc == nullptr) return;
-    ep.row_part = det;
-    ep.part_ld = rows;
-    ep.part_slot = det_cursor;
-    det_cursor += n;
-  };
-
+  // two ping-pong activation and hidden buffers, the (unused) accumulator region, the split-K scratch, the low-part
+  // twins of the four buffers (3xTF32 / bf16x2), the deterministic slot area
+  Arena ws(workspace);
+  Buf act[2], hid[2];
+  for (Buf& a : act) a = {ws.take(p.act_bytes), nullptr, p.ld_act};
+  for (Buf& h : hid) h = {ws.take(p.hid_bytes), nullptr, p.ld_hid};
+  ws.take(p.acc_bytes);
+  ChainIO io{};
+  io.scratch = p.small_bytes ? static_cast<float*>(ws.take(p.small_bytes)) : nullptr;
+  io.scratch_floats = p.small_bytes / sizeof(float);
+  if (precision == USF_PREC_TF32X3 || precision == USF_PREC_BF16X2) {
+    for (Buf& a : act) a.lo = ws.take(p.act_bytes);
+    for (Buf& h : hid) h.lo = ws.take(p.hid_bytes);
+  }
+  io.det = p.det_slots > 0 ? static_cast<float*>(ws.take(p.det_bytes)) : nullptr;
+  io.det_n = p.det_slots;
+  io.act = act;
+  io.n_act = 2;
+  io.hid = hid;
+  io.n_hid = 2;
+  io.density = out_logprob != nullptr;
+  io.ldo = ldy;
+  io.acc_init = out_logprob ? st->const_term : 0.f;
+  float* acc = out_logprob ? out_logprob : out_ladj;
   int launches = 0;
-  // Serpentine tile order (bf16 tier): every tensor-core kernel of the chain walks the row tiles in the opposite
-  // direction of its predecessor, so that it starts on the rows that kernel wrote last and that are still in L2
-  // (usf_tc.cu: tc_set_tile_order).  The input pack walks first -> last, so the first GEMM starts reversed.
-  static const bool serpentine = []() { const char* e = getenv("USF_TC_SERPENTINE"); return !(e != nullptr && e[0] == '0'); }();
-  int flip = 1;
-  auto next_order = [&]() { tc_set_tile_order(serpentine ? flip : 0); flip ^= 1; };
-  struct OrderReset { ~OrderReset() { tc_set_tile_order(0); } } order_reset;   // stand-alone GEMM calls stay first -> last
-
-  // One GEMM of the chain at the chosen precision.
-  auto gemm = [&](const void* A, int64_t lda, const usf_linear_desc& L, int bn, EpiParams& ep, int64_t rows) -> int {
-    if (bf16) {
-      USF_CHECK_ARG(L.Wb != nullptr, "usf_stack_run: bf16 weights missing in descriptor");
-      next_order();
-      return tc_gemm(reinterpret_cast<const uint16_t*>(A), lda, L.Wb, L.ldw, rows, L.N, L.K, bn, ep, s);
-    }
-    if (b2) {
-      USF_CHECK_ARG(L.Wb != nullptr, "usf_stack_run: bf16 (hi, lo) weights missing in descriptor");
-      const uint16_t* Ab = reinterpret_cast<const uint16_t*>(A);
-      uint16_t* ub_lo = ep.ub != nullptr ? reinterpret_cast<uint16_t*>(lo_of(ep.ub)) : nullptr;
-      uint16_t* out_lo = (ep.out != nullptr && (ep.mode == EPI_BIAS || ep.mode == EPI_BIAS_RELU) &&
-                          reinterpret_cast<uint8_t*>(ep.out) >= base && reinterpret_cast<uint8_t*>(ep.out) < lo_base)
-                             ? reinterpret_cast<uint16_t*>(lo_of(ep.out)) : nullptr;
-      return tcb2_gemm(Ab, reinterpret_cast<const uint16_t*>(lo_of(Ab)), lda, L.Wb, L.Wb + (size_t)L.N * (size_t)L.ldw, L.ldw,
-                       rows, L.N, L.K, bn, ep, out_lo, ub_lo, s);
-    }
-    USF_CHECK_ARG(L.W != nullptr, "usf_stack_run: fp32 weights missing in descriptor");
-    if (t3) {
-      const float* Af = reinterpret_cast<const float*>(A);
-      float* ub_lo = ep.ub != nullptr ? lo_of(ep.ub) : nullptr;
-      float* out_lo = (ep.out != nullptr && (ep.mode == EPI_BIAS || ep.mode == EPI_BIAS_RELU) &&
-                       reinterpret_cast<uint8_t*>(ep.out) >= base && reinterpret_cast<uint8_t*>(ep.out) < lo_base)
-                          ? lo_of(ep.out) : nullptr;
-      return tc3_gemm(Af, lo_of(Af), lda, L.W, L.W + (size_t)L.N * (size_t)L.ldw, L.ldw, rows, L.N, L.K, bn, ep, out_lo,
-                      ub_lo, s);
-    }
-    return simt_gemm(reinterpret_cast<const float*>(A), lda, 0, L.W, L.ldw, 0, rows, L.N, L.K, ep, s, small,
-                     p.small_bytes / sizeof(float));
-  };
-
   for (int64_t r0 = 0; r0 < B; r0 += kChunkRows) {
     const int64_t rows = (B - r0) < kChunkRows ? (B - r0) : kChunkRows;
-    float* row_acc = out_logprob ? out_logprob + r0 : (out_ladj ? out_ladj + r0 : nullptr);
-    const float acc_init = out_logprob ? st->const_term : 0.f;
-
-
-    // stage 0: bring x into the activation layout (bf16, or padded fp32) and seed the per-row accumulator
-    int cur = 0;
-    flip = 1;
-    det_cursor = 0;
-    if (det != nullptr && row_acc != nullptr)
-      USF_CUDA(cudaMemsetAsync(det, 0, (size_t)p.det_slots * (size_t)rows * sizeof(float), s));
-    {
-      ProfScope ps(s, 0);
-      if (b2)
-        rc = launch_split_rows_bf16x2(x + r0 * ldx, ldx, reinterpret_cast<uint16_t*>(act[0]),
-                                      reinterpret_cast<uint16_t*>(lo_of(act[0])), p.ld_act, rows, d_in, row_acc, acc_init, s);
-      else if (x_bf16)
-        rc = launch_copy_rows_bf16(reinterpret_cast<const uint16_t*>(x) + r0 * ldx, ldx, reinterpret_cast<uint16_t*>(act[0]),
-                                   p.ld_act, rows, d_in, row_acc, acc_init, s);
-      else
-        rc = launch_convert_rows(x + r0 * ldx, ldx, bf16 ? reinterpret_cast<uint16_t*>(act[0]) : nullptr,
-                                 bf16 ? nullptr : reinterpret_cast<float*>(act[0]), p.ld_act, rows, d_in, row_acc,
-                                 acc_init, s);
-    }
+    io.out = out_y ? out_y + r0 * ldy : nullptr;
+    io.row_acc = acc ? acc + r0 : nullptr;
+    const void* xr = x_bf16 ? static_cast<const void*>(reinterpret_cast<const uint16_t*>(x) + r0 * ldx) : x + r0 * ldx;
+    rc = run_chain(st, xr, ldx, x_bf16, rows, precision, io, &launches, as_stream(stream));
     if (rc) return rc;
-    ++launches;
-    if (t3) {
-      rc = launch_split_lo(reinterpret_cast<const float*>(act[0]), p.ld_act, reinterpret_cast<float*>(act[0]), lo_of(act[0]),
-                           p.ld_act, rows, p.ld_act, s);
-      if (rc) return rc;
-      ++launches;
-    }
-
-    for (int b = 0; b < st->n_blocks; ++b) {
-      const usf_block_desc& blk = st->blocks[b];
-      // (1) dense affine map u = G x + g, written in [a | pad | b] column order
-      {
-        EpiParams ep{};
-        ep.mode = EPI_BIAS;
-        ep.bias = blk.G.bias;
-        ep.out = act[cur ^ 1];
-        ep.ldo = p.ld_act;
-        ep.out_bf16 = bf16 || b2;
-        {
-          ProfScope ps(s, 1);
-          rc = gemm(act[cur], p.ld_act, blk.G, (bf16 || t3 || b2) ? tc_pick_bn(blk.G.N) : 0, ep, rows);
-        }
-        if (rc) return rc;
-        ++launches;
-        cur ^= 1;
-      }
-      // (2) conditioner MLP on the a-part, last layer fused with the coupling update of the b-part
-      bool fused = false;
-      if (bf16 && blk.n_mlp >= 2) {
-        int Ns[USF_MAX_MLP], Ks[USF_MAX_MLP], ldws[USF_MAX_MLP];
-        const uint16_t* Wbs[USF_MAX_MLP];
-        const float* biases[USF_MAX_MLP];
-        bool have = true;
-        for (int l = 0; l < blk.n_mlp; ++l) {
-          Ns[l] = blk.mlp[l].N; Ks[l] = blk.mlp[l].K; ldws[l] = blk.mlp[l].ldw;
-          Wbs[l] = blk.mlp[l].Wb; biases[l] = blk.mlp[l].bias;
-          have = have && Wbs[l] != nullptr && biases[l] != nullptr;
-        }
-        if (have && blk.n_mlp <= 4 && tc_mlp_supported(blk.n_mlp, Ns, Ks, blk.Da)) {
-          // ONE kernel: the whole conditioner chain with hidden activations resident in shared memory + coupling
-          EpiParams ep{};
-          if (blk.affine) ep.mode = st->inverse ? EPI_COUPLING_INV : EPI_COUPLING_FWD;
-          else ep.mode = st->inverse ? EPI_ADD_INV : EPI_ADD_FWD;
-          ep.ub = act[cur] + (size_t)blk.b_off * esz;
-          ep.ldub = p.ld_act;
-          ep.ub_bf16 = 1;
-          ep.Db = blk.Db;
-          ep.C = blk.C;
-          ep.clamp = blk.clamp;
-          ep.row_acc = row_acc;
-          if (blk.affine) det_assign(ep, 2 * (int)ceil_div(blk.mlp[blk.n_mlp - 1].N, 2 * blk.C) > 4 ? 2 * (int)ceil_div(blk.mlp[blk.n_mlp - 1].N, 2 * blk.C) : 4, rows);
-          next_order();
-          {
-            ProfScope ps(s, 5);
-            rc = tc_mlp_coupling(reinterpret_cast<const uint16_t*>(act[cur]), p.ld_act, rows, blk.n_mlp, Wbs, ldws, biases,
-                                 Ns, Ks, blk.affine ? 2 * blk.C : blk.C, ep, s);
-          }
-          if (rc) return rc;
-          ++launches;
-          fused = true;
-        }
-      }
-      const void* in = act[cur];
-      int64_t ld_in = p.ld_act;
-      for (int l = 0; l < blk.n_mlp && !fused; ++l) {
-        const usf_linear_desc& L = blk.mlp[l];
-        EpiParams ep{};
-        ep.bias = L.bias;
-        int bn = 0;
-        if (l + 1 < blk.n_mlp) {
-          ep.mode = EPI_BIAS_RELU;
-          ep.out = hid[l & 1];
-          ep.ldo = p.ld_hid;
-          ep.out_bf16 = bf16 || b2;
-          if (bf16 || t3 || b2) bn = tc_pick_bn(L.N);
-        } else {
-          if (blk.affine) ep.mode = st->inverse ? EPI_COUPLING_INV : EPI_COUPLING_FWD;
-          else ep.mode = st->inverse ? EPI_ADD_INV : EPI_ADD_FWD;
-          ep.ub = act[cur] + (size_t)blk.b_off * esz;
-          ep.ldub = p.ld_act;
-          ep.ub_bf16 = bf16 || b2;
-          ep.Db = blk.Db;
-          ep.C = blk.C;
-          ep.clamp = blk.clamp;
-          ep.row_acc = row_acc;
-          if (bf16 || t3 || b2) bn = blk.affine ? 2 * blk.C : blk.C;
-          if (blk.affine)      // (the same slot count as the fused form of this block would take: see plan_stack)
-            det_assign(ep, (bf16 || t3 || b2) ? (2 * (int)ceil_div(L.N, 2 * blk.C) > 4 ? 2 * (int)ceil_div(L.N, 2 * blk.C) : 4)
-                                             : det_slots_of(precision, L.N, 0, false), rows);
-        }
-        {
-          ProfScope ps(s, l + 1 < blk.n_mlp ? 2 : 3);
-          rc = gemm(in, ld_in, L, bn, ep, rows);
-        }
-        if (rc) return rc;
-        ++launches;
-        in = hid[l & 1];
-        ld_in = p.ld_hid;
-      }
-    }
-    // (3) last affine map, fused with the base log-density when a density is requested
-    {
-      EpiParams ep{};
-      ep.bias = st->G_final.bias;
-      ep.n_valid = st->D;
-      ep.out = out_y ? out_y + r0 * ldy : nullptr;
-      ep.ldo = ldy;
-      ep.out_bf16 = 0;
-      if (out_logprob) {
-        ep.mode = st->base_kind == 0 ? EPI_BASE_NORMAL : EPI_BASE_LAPLACE;
-        ep.loc = st->loc;
-        ep.inv_scale = st->inv_scale;
-        ep.row_acc = row_acc;
-        det_assign(ep, (bf16 || t3 || b2) ? det_slots_of(precision, st->G_final.N, tc_pick_bn(st->G_final.N), false)
-                                          : det_slots_of(precision, st->D, 0, false), rows);
-      } else {
-        USF_CHECK_ARG(out_y != nullptr, "usf_stack_run: nothing to compute (no output requested)");
-        ep.mode = EPI_BIAS;
-      }
-      // fp32 path: the SIMT kernel stores exactly N = D columns
-      usf_linear_desc Lf = st->G_final;
-      if (!bf16 && !t3 && !b2) Lf.N = st->D;
-      {
-        ProfScope ps(s, 4);
-        rc = gemm(act[cur], p.ld_act, Lf, (bf16 || t3 || b2) ? tc_pick_bn(Lf.N) : 0, ep, rows);
-      }
-      if (rc) return rc;
-      ++launches;
-    }
-    // deterministic mode: the slots, added in slot order, on top of the seeded accumulator
-    if (det != nullptr && row_acc != nullptr && det_cursor > 0) {
-      rc = launch_sum_row_parts(row_acc, det, rows, det_cursor, rows, s);
-      if (rc) return rc;
-      ++launches;
-    }
   }
   if (gpu_launches) *gpu_launches = launches;
   return USF_OK;

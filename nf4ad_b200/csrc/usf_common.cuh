@@ -37,6 +37,18 @@ int cuda_fail(cudaError_t e, const char* what);
 static inline cudaStream_t as_stream(usf_stream_t s) { return reinterpret_cast<cudaStream_t>(s); }
 __host__ __device__ static inline int64_t ceil_div(int64_t a, int64_t b) { return (a + b - 1) / b; }
 __host__ __device__ static inline int64_t round_up(int64_t a, int64_t b) { return ceil_div(a, b) * b; }
+inline size_t align256(size_t v) { return (v + 255) & ~size_t(255); }
+
+// Bump allocation from a caller's workspace: the start rounded up to 256 bytes, every buffer 256-byte aligned.
+struct Arena {
+  uint8_t* cur;
+  explicit Arena(void* ws) : cur(reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(ws) + 255) & ~uintptr_t(255))) {}
+  void* take(size_t bytes) {
+    void* q = cur;
+    cur += align256(bytes);
+    return q;
+  }
+};
 
 int num_sms();
 int deterministic_mode();   // usf_set_deterministic of the calling thread
@@ -146,5 +158,48 @@ int launch_copy_rows_bf16(const uint16_t* x, int64_t ldx, uint16_t* y, int64_t l
 int launch_sum_row_parts(float* out, const float* part, int64_t ld, int slots, int64_t rows, cudaStream_t stream);
 int launch_bf16_to_f32(const uint16_t* x, int64_t ldx, float* y, int64_t ldy, int64_t B, int64_t D,
                        cudaStream_t stream);
+
+// ---- the forward launch chain of a packed stack (usf_api.cu): usf_stack_run and usf_stack_log_prob_grad ------------
+// One row buffer of a chain: hi with leading dimension ld (elements), and lo its low-part twin when the operands travel
+// as (hi, lo) pairs (3xTF32, bf16x2); lo is nullptr at fp32 / bf16 and for fp32 GEMM outputs.
+struct Buf {
+  void* hi;
+  void* lo;
+  int64_t ld;
+};
+
+// Deterministic mode: partial-sum slots (the `sub` range of row_accumulate) of the accumulating launch of block b's
+// coupling (0 for an additive one), or of the final GEMM's base density at b == st->n_blocks.  Every chain sizes and
+// assigns its slots with it, so that all of them add the same slots in the same order.
+int det_slots(const usf_stack_desc* st, int b, int precision);
+
+// One GEMM of a chain at `precision`: A (rows, L.K) times L^T, N output columns, N tile bn (0: tc_pick_bn(N); the SIMT
+// kernel takes none), epilogue ep.  out_lo / ub_lo: the low-part twins of ep.out / ep.ub (3xTF32, bf16x2), or nullptr.
+// scratch: the fp32 split-K accumulator of simt_gemm, or nullptr.
+int chain_gemm(int precision, const Buf& A, const usf_linear_desc& L, int64_t rows, int64_t N, int bn,
+               const EpiParams& ep, void* out_lo, void* ub_lo, float* scratch, size_t scratch_floats, cudaStream_t stream);
+
+// Where one pass of run_chain puts its rows.
+struct ChainIO {
+  const Buf* act;            // act[0] receives the packed input, act[(j + 1) % n_act] block j's output row
+  int n_act;
+  const Buf* hid;            // the k-th hidden activation of the pass (counted over all blocks) goes to hid[k % n_hid]
+  int n_hid;
+  bool density;              // the final GEMM adds the base log-density to row_acc (else: the plain affine map into out)
+  float* out;                // the final GEMM's rows (z or y, D columns), or nullptr
+  int64_t ldo;
+  float* row_acc;            // per-row log p / log-det, seeded with acc_init by the input pack; or nullptr
+  float acc_init;
+  float* det;                // deterministic mode: slot area of det_n slots of `rows` floats (nullptr: fp32 atomics)
+  int det_n;
+  float* scratch;            // fp32 split-K accumulator (chain_gemm), or nullptr
+  size_t scratch_floats;
+};
+
+// The forward chain over `rows` rows of x (fp32 rows, or bf16 rows when x_bf16) at `precision`: input pack, per block
+// the G GEMM, the conditioner GEMMs (or the fused bf16 conditioner kernel) ending in the coupling, the final GEMM, and
+// in deterministic mode the slot sum.  Adds the launches it enqueues to *launches.
+int run_chain(const usf_stack_desc* st, const void* x, int64_t ldx, bool x_bf16, int64_t rows, int precision,
+              const ChainIO& io, int* launches, cudaStream_t stream);
 
 }  // namespace usf

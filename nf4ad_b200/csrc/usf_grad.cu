@@ -14,16 +14,6 @@ namespace {
 // while every GEMM of the chain still has >= 64 row tiles of 256 to spread over the 74 SM pairs
 constexpr int64_t kGradChunkRows = 16384;
 
-inline size_t align256(size_t v) { return (v + 255) & ~size_t(255); }
-
-// One row buffer of the chain: fp32 (lo == nullptr: the fp32 tier, or any fp32 GEMM output) or a (hi, lo) bf16 pair
-// (the bf16x2 tier's GEMM operands).
-struct Buf {
-  void* hi;
-  void* lo;
-  int64_t ld;
-};
-
 __device__ __forceinline__ float ld_op(const void* hi, const void* lo, int64_t i) {
   if (lo == nullptr) return reinterpret_cast<const float*>(hi)[i];
   return __uint_as_float((uint32_t)reinterpret_cast<const uint16_t*>(hi)[i] << 16) +
@@ -120,17 +110,6 @@ __global__ void usf_grad_residual_kernel(const float* g, int64_t ldg, const floa
   }
 }
 
-// partial-sum slots of the accumulating launches -- the same counts usf_stack_run's chain takes (plan_stack), so that
-// the deterministic log p adds the same slots in the same order
-int coupling_slots(bool tc, const usf_linear_desc& L, int C) {
-  if (!tc) return (int)ceil_div(L.N, 128);
-  const int n = 2 * (int)ceil_div(L.N, 2 * C);
-  return n > 4 ? n : 4;
-}
-int base_slots(bool tc, const usf_stack_desc* st) {
-  return tc ? 2 * (int)ceil_div(st->G_final.N, tc_pick_bn(st->G_final.N)) : (int)ceil_div(st->D, 128);
-}
-
 struct GradPlan {
   int64_t ld_act, ld_hid, ld_st, ld_gh, ld_z;
   int n_hidden;   // saved hidden activations over all blocks
@@ -170,7 +149,6 @@ int plan_grad(const usf_stack_desc* st, const usf_stack_grad_desc* gd, int64_t r
       if (T.N > hmax) hmax = T.N;
     }
     USF_CHECK_ARG(b2 ? gb.G.Wb != nullptr : gb.G.W != nullptr, "stack grad: block %d: G^T weights missing", b);
-    if (blk.affine) p->det_slots += coupling_slots(b2, blk.mlp[blk.n_mlp - 1], blk.C);
   }
   USF_CHECK_ARG(gd->G_final.K == st->G_final.N && gd->G_final.N >= st->G_final.K &&
                     (b2 ? gd->G_final.Wb != nullptr : gd->G_final.W != nullptr), "stack grad: G_final^T does not match");
@@ -178,8 +156,8 @@ int plan_grad(const usf_stack_desc* st, const usf_stack_grad_desc* gd, int64_t r
   if (gd->G_final.N > wmax) wmax = gd->G_final.N;
   if (st->G_final.N > wmax) wmax = st->G_final.N;
   if (st->G_final.N > smax) smax = st->G_final.N;      // the [ds | dt] operand buffer carries dL/dz first
-  p->det_slots += base_slots(b2, st);
-  if (!deterministic_mode()) p->det_slots = 0;
+  if (deterministic_mode())   // the slots of usf_stack_run's chain: the same log p, bit for bit
+    for (int b = 0; b <= st->n_blocks; ++b) p->det_slots += det_slots(st, b, precision);
   p->ld_act = round_up(wmax, 16);
   p->ld_hid = round_up(hmax, 16);
   p->ld_st = round_up(smax, 16);
@@ -233,17 +211,15 @@ extern "C" int usf_stack_log_prob_grad(const usf_stack_desc* st, const usf_stack
   const int nb = st->n_blocks;
   const int64_t R = rows_max;
 
-  // bump allocation of the workspace (every buffer 256-byte aligned)
-  uint8_t* cur = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(workspace) + 255) & ~uintptr_t(255));
-  auto take = [&](size_t bytes) { void* q = cur; cur += align256(bytes); return q; };
+  Arena ws(workspace);
   auto op_buf = [&](int64_t ld) {   // a GEMM operand: fp32, or a (hi, lo) bf16 pair
     Buf o;
     o.ld = ld;
-    o.hi = take((size_t)R * ld * esz);
-    o.lo = b2 ? take((size_t)R * ld * esz) : nullptr;
+    o.hi = ws.take((size_t)R * ld * esz);
+    o.lo = b2 ? ws.take((size_t)R * ld * esz) : nullptr;
     return o;
   };
-  auto f32_buf = [&](int64_t ld) { return reinterpret_cast<float*>(take((size_t)R * ld * 4)); };
+  auto f32_buf = [&](int64_t ld) { return reinterpret_cast<float*>(ws.take((size_t)R * ld * 4)); };
   std::vector<Buf> act(nb + 1);             // act[0]: the input row; act[j + 1]: block j's output row (u, b-part coupled)
   for (int j = 0; j <= nb; ++j) act[j] = op_buf(p.ld_act);
   std::vector<Buf> hid(p.n_hidden);         // hidden activations, block-major
@@ -255,18 +231,24 @@ extern "C" int usf_stack_log_prob_grad(const usf_stack_desc* st, const usf_stack
   float* gh = f32_buf(p.ld_gh);
   Buf gho = op_buf(p.ld_gh);
   Buf guo = b2 ? op_buf(p.ld_act) : Buf{nullptr, nullptr, p.ld_act};
-  float* det = p.det_slots > 0 ? reinterpret_cast<float*>(take((size_t)p.det_slots * (size_t)R * 4)) : nullptr;
+  // the forward pass: usf_stack_run's chain, with every block's output row and hidden activation kept in its own slot
+  ChainIO io{};
+  io.act = act.data();
+  io.n_act = nb + 1;
+  io.hid = hid.data();
+  io.n_hid = p.n_hidden;
+  io.density = true;
+  io.out = z;
+  io.ldo = p.ld_z;
+  io.acc_init = st->const_term;
+  io.det = p.det_slots > 0 ? reinterpret_cast<float*>(ws.take((size_t)p.det_slots * (size_t)R * 4)) : nullptr;
+  io.det_n = p.det_slots;
 
   int launches = 0;
-  int det_cursor = 0;
-  // A (rows, L.K) x L^T with the epilogue `ep`; bf16x2 operand low parts from `A.lo`, output / b-part low parts as given
-  auto gemm = [&](const Buf& A, const usf_linear_desc& L, int64_t N, int bn, const EpiParams& ep, uint16_t* out_lo,
-                  uint16_t* ub_lo, int64_t rows) -> int {
+  // A (rows, L.K) x L^T, N columns, into the fp32 product `ep`
+  auto gemm = [&](const Buf& A, const usf_linear_desc& L, int64_t N, const EpiParams& ep, int64_t rows) -> int {
     ++launches;
-    if (b2)
-      return tcb2_gemm(reinterpret_cast<const uint16_t*>(A.hi), reinterpret_cast<const uint16_t*>(A.lo), A.ld, L.Wb,
-                       L.Wb + (size_t)L.N * (size_t)L.ldw, L.ldw, rows, N, L.K, bn ? bn : tc_pick_bn(N), ep, out_lo, ub_lo, s);
-    return simt_gemm(reinterpret_cast<const float*>(A.hi), A.ld, 0, L.W, L.ldw, 0, rows, N, L.K, ep, s);
+    return chain_gemm(precision, A, L, rows, N, 0, ep, nullptr, nullptr, nullptr, 0, s);
   };
   auto plain = [&](float* out, int64_t ldo, int n_valid) {   // fp32 product, no bias
     EpiParams ep{};
@@ -276,95 +258,11 @@ extern "C" int usf_stack_log_prob_grad(const usf_stack_desc* st, const usf_stack
     ep.n_valid = n_valid;
     return ep;
   };
-  auto off = [&](const Buf& b, int64_t cols) {   // the same buffer from column `cols` on
-    Buf o = b;
-    o.hi = reinterpret_cast<uint8_t*>(b.hi) + cols * esz;
-    if (b.lo) o.lo = reinterpret_cast<uint8_t*>(b.lo) + cols * esz;
-    return o;
-  };
 
   for (int64_t r0 = 0; r0 < B; r0 += kGradChunkRows) {
     const int64_t rows = (B - r0) < kGradChunkRows ? (B - r0) : kGradChunkRows;
-    float* lp = out_logprob + r0;
-    det_cursor = 0;
-    auto det_assign = [&](EpiParams& ep, int n) {
-      if (det == nullptr) return;
-      ep.row_part = det;
-      ep.part_ld = rows;
-      ep.part_slot = det_cursor;
-      det_cursor += n;
-    };
-    if (det != nullptr) USF_CUDA(cudaMemsetAsync(det, 0, (size_t)p.det_slots * (size_t)rows * sizeof(float), s));
-
-    // ---- forward: usf_stack_run's chain, every block's output row and hidden activation kept in its own slot
-    if (b2)
-      rc = launch_split_rows_bf16x2(x + r0 * ldx, ldx, reinterpret_cast<uint16_t*>(act[0].hi),
-                                    reinterpret_cast<uint16_t*>(act[0].lo), p.ld_act, rows, d_in, lp, st->const_term, s);
-    else
-      rc = launch_convert_rows(x + r0 * ldx, ldx, nullptr, reinterpret_cast<float*>(act[0].hi), p.ld_act, rows, d_in, lp,
-                               st->const_term, s);
-    if (rc) return rc;
-    ++launches;
-    int hi_idx = 0;
-    for (int j = 0; j < nb; ++j) {
-      const usf_block_desc& blk = st->blocks[j];
-      {
-        EpiParams ep{};
-        ep.mode = EPI_BIAS;
-        ep.bias = blk.G.bias;
-        ep.out = act[j + 1].hi;
-        ep.ldo = p.ld_act;
-        ep.out_bf16 = b2;
-        if ((rc = gemm(act[j], blk.G, blk.G.N, 0, ep, reinterpret_cast<uint16_t*>(act[j + 1].lo), nullptr, rows))) return rc;
-      }
-      Buf in = act[j + 1];
-      for (int l = 0; l < blk.n_mlp; ++l) {
-        const usf_linear_desc& L = blk.mlp[l];
-        EpiParams ep{};
-        ep.bias = L.bias;
-        if (l + 1 < blk.n_mlp) {
-          const Buf& h = hid[hi_idx + l];
-          ep.mode = EPI_BIAS_RELU;
-          ep.out = h.hi;
-          ep.ldo = p.ld_hid;
-          ep.out_bf16 = b2;
-          if ((rc = gemm(in, L, L.N, 0, ep, reinterpret_cast<uint16_t*>(h.lo), nullptr, rows))) return rc;
-          in = h;
-        } else {
-          const Buf ub = off(act[j + 1], blk.b_off);
-          ep.mode = blk.affine ? EPI_COUPLING_INV : EPI_ADD_INV;
-          ep.ub = ub.hi;
-          ep.ldub = p.ld_act;
-          ep.ub_bf16 = b2;
-          ep.Db = blk.Db;
-          ep.C = blk.C;
-          ep.clamp = blk.clamp;
-          ep.row_acc = lp;
-          if (blk.affine) det_assign(ep, coupling_slots(b2, L, blk.C));
-          if ((rc = gemm(in, L, L.N, blk.affine ? 2 * blk.C : blk.C, ep, nullptr, reinterpret_cast<uint16_t*>(ub.lo), rows)))
-            return rc;
-        }
-      }
-      hi_idx += blk.n_mlp - 1;
-    }
-    {
-      EpiParams ep{};
-      ep.mode = st->base_kind == 0 ? EPI_BASE_NORMAL : EPI_BASE_LAPLACE;
-      ep.bias = st->G_final.bias;
-      ep.n_valid = st->D;
-      ep.out = z;
-      ep.ldo = p.ld_z;
-      ep.loc = st->loc;
-      ep.inv_scale = st->inv_scale;
-      ep.row_acc = lp;
-      det_assign(ep, base_slots(b2, st));
-      // fp32 tier: the SIMT kernel stores exactly N = D columns (as in usf_stack_run)
-      if ((rc = gemm(act[nb], st->G_final, b2 ? st->G_final.N : st->D, 0, ep, nullptr, nullptr, rows))) return rc;
-    }
-    if (det != nullptr && det_cursor > 0) {
-      if ((rc = launch_sum_row_parts(lp, det, rows, det_cursor, rows, s))) return rc;
-      ++launches;
-    }
+    io.row_acc = out_logprob + r0;
+    if ((rc = run_chain(st, x + r0 * ldx, ldx, false, rows, precision, io, &launches, s))) return rc;
 
     // ---- reverse: dL/dz, then back through G_final^T and every block
     float* go = out_grad + r0 * ldg;
@@ -375,11 +273,11 @@ extern "C" int usf_stack_log_prob_grad(const usf_stack_desc* st, const usf_stack
       USF_LAUNCH_CHECK("usf_grad_base_kernel");
       ++launches;
       const usf_linear_desc& T = gd->G_final;
-      if (nb == 0) rc = gemm(gz, T, b2 ? T.N : st->D, 0, plain(go, ldg, st->D), nullptr, nullptr, rows);
-      else rc = gemm(gz, T, T.N, 0, plain(gy[0], p.ld_act, 0), nullptr, nullptr, rows);
+      if (nb == 0) rc = gemm(gz, T, b2 ? T.N : st->D, plain(go, ldg, st->D), rows);
+      else rc = gemm(gz, T, T.N, plain(gy[0], p.ld_act, 0), rows);
       if (rc) return rc;
     }
-    int g = 0;
+    int g = 0, hi_idx = p.n_hidden;
     for (int j = nb - 1; j >= 0; --j) {
       const usf_block_desc& blk = st->blocks[j];
       const usf_block_grad_desc& gb = gd->blocks[j];
@@ -390,7 +288,7 @@ extern "C" int usf_stack_log_prob_grad(const usf_stack_desc* st, const usf_stack
       const Buf in_last = nl >= 2 ? hid[hi_idx + nl - 2] : act[j + 1];
       EpiParams ep = plain(stb, p.ld_st, 0);
       ep.bias = Ll.bias;
-      if ((rc = gemm(in_last, Ll, Ll.N, 0, ep, nullptr, nullptr, rows))) return rc;
+      if ((rc = gemm(in_last, Ll, Ll.N, ep, rows))) return rc;
       const int W = blk.affine ? 2 * blk.C : blk.C;
       usf_grad_coupling_kernel<<<grid_of(rows * (Ll.N / W) * blk.C), 256, 0, s>>>(
           stb, p.ld_st, act[j + 1], blk.b_off, gy[g], p.ld_act, gst, blk.Db, blk.C, Ll.N / W, blk.affine, blk.clamp, rows);
@@ -400,7 +298,7 @@ extern "C" int usf_stack_log_prob_grad(const usf_stack_desc* st, const usf_stack
       Buf a = gst;
       for (int l = nl - 1; l >= 0; --l) {
         const usf_linear_desc& T = gb.mlp[l];
-        if ((rc = gemm(a, T, T.N, 0, plain(gh, p.ld_gh, 0), nullptr, nullptr, rows))) return rc;
+        if ((rc = gemm(a, T, T.N, plain(gh, p.ld_gh, 0), rows))) return rc;
         if (l > 0) {
           const int64_t n = blk.mlp[l - 1].N;
           usf_grad_relu_kernel<<<grid_of(rows * n), 256, 0, s>>>(gh, p.ld_gh, hid[hi_idx + l - 1], n, gho, rows);
@@ -417,8 +315,8 @@ extern "C" int usf_stack_log_prob_grad(const usf_stack_desc* st, const usf_stack
       ++launches;
       // dL/dx_j = dL/du G_j: into the other gradient row, or (block 0) the caller's output, context columns dropped
       const usf_linear_desc& T = gb.G;
-      if (j == 0) rc = gemm(gu, T, b2 ? T.N : st->D, 0, plain(go, ldg, st->D), nullptr, nullptr, rows);
-      else rc = gemm(gu, T, T.N, 0, plain(gy[g ^ 1], p.ld_act, 0), nullptr, nullptr, rows);
+      if (j == 0) rc = gemm(gu, T, b2 ? T.N : st->D, plain(go, ldg, st->D), rows);
+      else rc = gemm(gu, T, T.N, plain(gy[g ^ 1], p.ld_act, 0), rows);
       if (rc) return rc;
       g ^= 1;
     }

@@ -335,25 +335,30 @@ class Flow(torch.nn.Module):
         return self._tier(x2, xin)
 
     def _stack(self, inverse, device, precision=None, grad=False):
-        """Compiled (packed) stack for this direction / precision / weight version, or None.  `grad`: the inverse stack
-        with the transposed matrices of the reverse chain as well (`log_prob_and_grad`)."""
+        """Compiled (packed) stack for this direction / precision / weight version, or None.  `grad`: the same stack with
+        the transposed matrices of the reverse chain built (`log_prob_and_grad`), or None where they cannot be."""
         precision = precision or self.precision
         if precision == "auto":
             precision = self.FP32_GRADE_TC if self.event_dim >= self.BF16_MIN_DIM else "fp32"
         prec = _PRECISIONS[precision]
-        slot = ("grad", prec) if grad else (bool(inverse), prec)
+        slot = (bool(inverse), prec)
         key = (self._weights_key(), str(device))
         hit = self._compiled.get(slot)
-        if hit is not None and hit[0] == key:
-            return hit[1]
-        try:
-            if len(self.event_shape) != 1:
-                raise stack.Unsupported("image-shaped event: the layer-wise kernels are used")
-            cs = stack.CompiledStack(self.layers, self.base_distribution, self.event_dim, device, inverse, prec, grad=grad)
-        except stack.Unsupported as e:
-            cs = None
-            self._unsupported_reason = str(e)
-        self._compiled[slot] = (key, cs)
+        if hit is None or hit[0] != key:
+            try:
+                if len(self.event_shape) != 1:
+                    raise stack.Unsupported("image-shaped event: the layer-wise kernels are used")
+                cs = stack.CompiledStack(self.layers, self.base_distribution, self.event_dim, device, inverse, prec)
+            except stack.Unsupported as e:
+                cs = None
+                self._unsupported_reason = str(e)
+            hit = self._compiled[slot] = (key, cs)
+        cs = hit[1]
+        if grad and cs is not None:
+            try:
+                cs.grad_desc            # built on first use, kept with the stack
+            except stack.Unsupported as e:
+                cs, self._unsupported_reason = None, str(e)
         return cs
 
     def _needs_grad(self, x):

@@ -82,16 +82,15 @@ def base_params(base, D, device):
 
 
 class CompiledStack:
-    """Device-resident packed weights + the ctypes descriptor tree for one (direction, precision).  `grad`: also pack
-    every matrix of the inverse chain transposed (`grad_desc`, the reverse chain of `run_grad`)."""
+    """Device-resident packed weights + the ctypes descriptor tree for one (direction, precision); `grad_desc`: the
+    transposed matrices of the reverse chain (`run_grad`), built from the same packs on first use."""
 
-    def __init__(self, layers, base, D, device, inverse, precision, grad=False):
+    def __init__(self, layers, base, D, device, inverse, precision):
         self.D, self.inverse, self.precision = D, bool(inverse), precision
-        if grad and (not self.inverse or precision not in (_lib.USF_PREC_FP32, _lib.USF_PREC_BF16X2)):
-            raise Unsupported("the input-gradient chain runs the inverse direction at fp32 or bf16x2")
-        self.grad = bool(grad)
         self.device = device
         self._keep = []          # every tensor the descriptors point to
+        self._packs = {}         # descriptor address -> the packed weight tensor behind it (W, or bf16x2 [hi ; lo])
+        self._grad_desc = None
         self._mlp_widths = {}    # block -> unpadded widths of its conditioner layers
         bf16 = precision == _lib.USF_PREC_BF16
         self._t3 = precision == _lib.USF_PREC_TF32X3      # fp32 weights travel as [W ; W - tf32(W)] (2N rows)
@@ -168,24 +167,21 @@ class CompiledStack:
             natural = torch.arange(Dx, dtype=torch.int32, device=device)
             in_cols = natural                        # column layout of the current activation
             self.blocks = (BlockDesc * max(n, 1))()
-            self.grad_blocks = (BlockGradDesc * max(n, 1))() if self.grad else None
             logdet = 0.0
             for j, (run, cpl, L) in enumerate(order):
                 blk = self.blocks[j]
                 Mt = run_matrix(run)
-                gblk = self.grad_blocks[j] if self.grad else None
-                self._fill_affine(blk.G, Mt, in_cols, L["cols"], bf16, gblk.G if gblk is not None else None)
+                self._fill_affine(blk.G, Mt, in_cols, L["cols"], bf16)
                 blk.b_off, blk.Da, blk.Db = L["b_off"], L["Da"], L["Db"]
                 blk.clamp = float(getattr(cpl, "clamp", 5.0))
-                self._fill_conditioner(blk, cpl, L, D, bf16, gblk)
+                self._fill_conditioner(blk, cpl, L, D, bf16)
                 in_cols = L["cols"]
             Mt = run_matrix(last_run)
             out_w = _round_up(D, 16)
             out_cols = torch.full((out_w,), -1, dtype=torch.int32, device=device)
             out_cols[:D] = natural[:D]
             self.G_final = LinearDesc()
-            self.G_final_t = LinearDesc() if self.grad else None
-            self._fill_affine(self.G_final, Mt, in_cols, out_cols, bf16, self.G_final_t)
+            self._fill_affine(self.G_final, Mt, in_cols, out_cols, bf16)
 
             # ---- data-independent terms ------------------------------------------------------------
             probe = torch.zeros(1, D, device=device, dtype=torch.float32)
@@ -213,12 +209,6 @@ class CompiledStack:
                     base_const = -float((2.0 * scale).log().sum())
                 st.const_term = base_const - logdet
             self.desc = st
-            if self.grad:
-                gd = StackGradDesc()
-                gd.n_blocks = n
-                gd.blocks = C.cast(self.grad_blocks, C.POINTER(BlockGradDesc))
-                gd.G_final = self.G_final_t
-                self.grad_desc = gd
 
     # -------------------------------------------------------------------------------------------
     def _fill_linear(self, desc, W32, Wb, bias, N, K, ldw):
@@ -233,29 +223,14 @@ class CompiledStack:
             hi = ((W32.view(torch.int32) + 0x1000) & -8192).view(torch.float32)   # rounded to tf32 (exact under the
             W32 = torch.cat([hi, W32 - hi], dim=0).contiguous()                   # tensor core's truncating read)
         self._keep += [t for t in (W32, Wb, bias) if t is not None]
+        self._packs[C.addressof(desc)] = W32 if W32 is not None else Wb
         desc.W = W32.data_ptr() if W32 is not None else None
         desc.Wb = Wb.data_ptr() if Wb is not None else None
         desc.bias = bias.data_ptr()
         desc.N, desc.K, desc.ldw = N, K, ldw
 
-    def _fill_linear_t(self, desc, Wt, N, K):
-        """Transposed matrix of the reverse chain: Wt (N, K) fp32 holds W^T of a forward (K, N) layer; bf16x2 takes
-        [bf16(Wt) ; bf16(Wt - bf16(Wt))], the low part derived from fp32 as in `_fill_linear`."""
-        if self._b2:
-            if N > 1024:
-                raise Unsupported("bf16x2 path keeps the per-column vectors resident: N <= 1024")
-            hi = Wt.to(torch.bfloat16)
-            Wb, Wt = torch.cat([hi, (Wt - hi.float()).to(torch.bfloat16)], dim=0).contiguous(), None
-        else:
-            Wb = None
-        self._keep += [t for t in (Wt, Wb) if t is not None]
-        desc.W = Wt.data_ptr() if Wt is not None else None
-        desc.Wb = Wb.data_ptr() if Wb is not None else None
-        desc.bias = None
-        desc.N, desc.K, desc.ldw = N, K, K
-
-    def _fill_affine(self, desc, Mt, in_cols, out_cols, bf16, tdesc=None):
-        """W[j, i] = A[out_cols[j], in_cols[i]], bias[j] = c[out_cols[j]]  (index -1 -> 0); tdesc: W^T as well."""
+    def _fill_affine(self, desc, Mt, in_cols, out_cols, bf16):
+        """W[j, i] = A[out_cols[j], in_cols[i]], bias[j] = c[out_cols[j]]  (index -1 -> 0)."""
         N, K = out_cols.numel(), in_cols.numel()
         ldw = _round_up(K, 8)
         src_rows = torch.where(in_cols >= 0, in_cols + 1, in_cols).contiguous()
@@ -263,14 +238,8 @@ class CompiledStack:
                                   want_f32=not bf16, want_bf16=bf16 or self._b2)
         bias, _ = ops.pack_matrix(Mt[:1], None, out_cols, 1, N, N)
         self._fill_linear(desc, W32, Wb, bias.reshape(-1), N, K, ldw)
-        if tdesc is not None:
-            Kp = _round_up(K, 16)
-            rows_t = torch.full((Kp,), -1, dtype=torch.int32, device=self.device)
-            rows_t[:K] = src_rows
-            Wt, _ = ops.pack_matrix(Mt, rows_t, out_cols, Kp, N, N, sub_row0=True)
-            self._fill_linear_t(tdesc, Wt, Kp, N)
 
-    def _fill_conditioner(self, blk, cpl, L, D, bf16, gblk=None):
+    def _fill_conditioner(self, blk, cpl, L, D, bf16):
         linears = mlp_layers(cpl.conditioner)
         cd = self.ctx_dim
         out_f = linears[-1].out_features
@@ -337,14 +306,6 @@ class CompiledStack:
             W32, Wb = ops.pack_matrix(Wsrc, row_idx, col_idx, N, K, ldw, want_f32=not bf16, want_bf16=bf16 or self._b2)
             bias, _ = ops.pack_matrix(bsrc.reshape(-1, 1), row_idx, None, N, 1, 1)
             self._fill_linear(blk.mlp[li], W32, Wb, bias.reshape(-1), N, K, ldw)
-            if gblk is not None:
-                Kp = _round_up(K, 16)
-                cols_t = torch.full((Kp,), -1, dtype=torch.int32, device=dev)
-                cols_t[:K] = col_idx if col_idx is not None else torch.arange(K, dtype=torch.int32, device=dev)
-                if row_idx is None:
-                    row_idx = torch.arange(N, dtype=torch.int32, device=dev)
-                Wt, _ = ops.pack_matrix(Wsrc, cols_t, row_idx, Kp, N, N, transpose_src=True)
-                self._fill_linear_t(gblk.mlp[li], Wt, Kp, N)
 
     @staticmethod
     def _verify_mlp(cond, linears, D, cd=0):
@@ -422,9 +383,42 @@ class CompiledStack:
         finally:
             lib().usf_set_deterministic(prev)
 
+    @property
+    def grad_desc(self):
+        """The `usf_stack_grad_desc` of `run_grad`, built on first use from this stack's own forward packs: for a matrix
+        W (N, K valid columns), W^T[:K] = W[:, :K]^T (bf16x2: the hi and the lo half each), rows K .. round_up(K, 16)
+        zero, no bias.  Raises Unsupported where the gradient chain does not run."""
+        if self._grad_desc is not None:
+            return self._grad_desc
+        if not self.inverse or self.precision not in (_lib.USF_PREC_FP32, _lib.USF_PREC_BF16X2):
+            raise Unsupported("the input-gradient chain runs the inverse direction at fp32 or bf16x2")
+        n = self.desc.n_blocks
+        self.grad_blocks = (BlockGradDesc * max(n, 1))()
+        gd = StackGradDesc()
+        gd.n_blocks = n
+        gd.blocks = C.cast(self.grad_blocks, C.POINTER(BlockGradDesc))
+        pairs = [(gd.G_final, self.G_final)]          # (transposed, forward) descriptors
+        for j in range(n):
+            blk, gb = self.blocks[j], self.grad_blocks[j]
+            pairs += [(gb.G, blk.G)] + [(gb.mlp[l], blk.mlp[l]) for l in range(blk.n_mlp)]
+        if self._b2 and any(_round_up(F.K, 16) > 1024 for _, F in pairs):
+            raise Unsupported("bf16x2 path keeps the per-column vectors resident: N <= 1024")
+        for T, F in pairs:
+            Kp = _round_up(F.K, 16)
+            halves = self._packs[C.addressof(F)].view(-1, F.N, F.ldw)[:, :, :F.K]     # fp32 W, or bf16x2 hi and lo
+            Wt = halves.new_zeros(halves.shape[0], Kp, F.N)
+            Wt[:, :F.K] = halves.transpose(1, 2)
+            Wt = Wt.reshape(-1, F.N)
+            self._keep.append(Wt)
+            T.W, T.Wb = (None, Wt.data_ptr()) if self._b2 else (Wt.data_ptr(), None)
+            T.bias = None
+            T.N, T.K, T.ldw = Kp, F.N, F.N
+        self._grad_desc = gd
+        return gd
+
     def run_grad(self, x, deterministic=False):
-        """log p(x) and d log p(x) / dx of rows x:(B, D + ctx_dim) on the reverse launch chain (a stack built with
-        grad=True).  Returns (logprob (B,), grad (B, D) fp32, n_launches)."""
+        """log p(x) and d log p(x) / dx of rows x:(B, D + ctx_dim) on the reverse launch chain (`grad_desc`).
+        Returns (logprob (B,), grad (B, D) fp32, n_launches)."""
         _lib.require_cuda(x)
         if x.dim() != 2 or x.shape[1] != self.D + self.ctx_dim:
             raise ValueError(f"expected rows of {self.D} coordinates (+ {self.ctx_dim} context columns), got shape {tuple(x.shape)}")

@@ -146,13 +146,12 @@ def test_invariants(O, P, precision, D, hidden):
     x = torch.randn(1000, D, generator=torch.Generator().manual_seed(7)).cuda()
     lp, g = fp.log_prob_and_grad(x)
     assert fp.last_grad_precision == precision
-    # deterministic mode: log p bit-identical to the launch chain of log_prob at the fp32 tier; at bf16x2 the two agree
-    # to the tier's accuracy (measured 3e-6) but not bit for bit: log_prob runs its own packing of the weights, which can
-    # differ in the last bits (on one descriptor the two chains agree bit for bit: test_gpu_stack_grad_kernels.py)
+    # deterministic mode: log p bit-identical to log_prob's, which runs the same packed stack
     with torch.no_grad():
         lq = fp.log_prob(x)
     assert fp.effective_precision == precision
-    assert torch.equal(lp, lq) if precision == "fp32" else rel(lp, lq) < FP32_TOL
+    assert torch.equal(lp, lq), rel(lp, lq)
+    assert len(fp._compiled) == 1, list(fp._compiled)
     # run to run: bit-identical
     lp2, g2 = fp.log_prob_and_grad(x)
     assert torch.equal(g, g2) and torch.equal(lp, lp2)
