@@ -391,15 +391,6 @@ int usf_debug_graph_stats(long long* stats4, char* last_failure, int failure_byt
  * GEMM expired (a pipeline protocol bug); synchronises the device. */
 int usf_debug_tc_timeout(int* flag, int reset);
 
-/* Debug: in-kernel pipeline trace of the tcgen05 GEMM.  Bits 0-7 of `on`: 1 = record the plain GEMM, 2 = the
- * fused conditioner kernel, for subsequent launches (CTAs 0 and 1; roles 0 TMA producer, 1 MMA issuer, 2 first
- * epilogue warp; 2048 records of {tile<<8 | event, SM clock} per (CTA, role)); out != NULL copies the last
- * launch's 12288 records.  Bits 8-15 of `on` (with out == NULL): ablation switches of the plain GEMM's
- * instrumented variant (1 no global stores, 2 no epilogue, 4 no A loads, 8 no W loads, 16 no MMAs, 32 back-off
- * waits, 64 single-lane polling, 128 nothing: just select the instrumented variant) -- results are then wrong by
- * construction, only times matter (scripts/tc_ablate.py).  Production launches run an uninstrumented variant. */
-int usf_debug_tc_trace(int on, unsigned long long* out, int max_records);
-
 /* 3xTF32: fp32-grade accuracy on the tensor cores.  Every fp32 operand travels as hi + lo, where hi is what the tensor
  * core sees when it reads fp32 as tf32 (low 13 mantissa bits dropped) and lo = value - hi; usf_split_lo computes lo
  * for a (rows x cols) matrix.  usf_linear_tf32x3: y = act(x W^T + bias) with three tcgen05.mma.kind::tf32 per K step

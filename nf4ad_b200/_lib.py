@@ -98,7 +98,6 @@ _PROTOS = {
     "usf_profile_end": (_int, [C.POINTER(_f32), C.POINTER(_int), C.POINTER(_int)]),
     "usf_debug_graph_stats": (_int, [C.POINTER(C.c_longlong), C.c_char_p, _int]),
     "usf_debug_tc_timeout": (_int, [C.POINTER(_int), _int]),
-    "usf_debug_tc_trace": (_int, [_int, C.POINTER(C.c_uint64), _int]),
     "usf_split_lo": (_int, [_vp, _i64, _vp, _i64, _i64, _i64, _vp]),
     "usf_linear_tf32x3": (_int, [_vp, _vp, _i64, _vp, _vp, _i64, _vp, _int, _vp, _vp, _i64, _i64, _i64, _i64, _vp]),
     "usf_linear_bf16": (_int, [_vp, _i64, _vp, _i64, _vp, _int, _vp, _i64, _int, _i64, _i64, _i64, _vp]),

@@ -151,10 +151,10 @@ int chain_gemm(int precision, const Buf& A, const usf_linear_desc& L, int64_t ro
   if (precision == USF_PREC_BF16)
     return tc_gemm(static_cast<const uint16_t*>(A.hi), A.ld, L.Wb, L.ldw, rows, N, L.K, bn, ep, s);
   if (precision == USF_PREC_TF32X3)
-    return tc3_gemm(static_cast<const float*>(A.hi), static_cast<const float*>(A.lo), A.ld, L.W, L.W + lo, L.ldw, rows, N,
-                    L.K, bn, ep, static_cast<float*>(out_lo), static_cast<float*>(ub_lo), s);
-  return tcb2_gemm(static_cast<const uint16_t*>(A.hi), static_cast<const uint16_t*>(A.lo), A.ld, L.Wb, L.Wb + lo, L.ldw,
-                   rows, N, L.K, bn, ep, static_cast<uint16_t*>(out_lo), static_cast<uint16_t*>(ub_lo), s);
+    return tc_split_gemm(static_cast<const float*>(A.hi), static_cast<const float*>(A.lo), A.ld, L.W, L.W + lo, L.ldw, rows,
+                         N, L.K, bn, ep, static_cast<float*>(out_lo), static_cast<float*>(ub_lo), s);
+  return tc_split_gemm(static_cast<const uint16_t*>(A.hi), static_cast<const uint16_t*>(A.lo), A.ld, L.Wb, L.Wb + lo, L.ldw,
+                       rows, N, L.K, bn, ep, static_cast<uint16_t*>(out_lo), static_cast<uint16_t*>(ub_lo), s);
 }
 
 int run_chain(const usf_stack_desc* st, const void* x, int64_t ldx, bool x_bf16, int64_t rows, int precision,
@@ -366,10 +366,6 @@ extern "C" const char* usf_gemm_kernel_name(int precision) {
 
 extern "C" int usf_debug_tc_timeout(int* flag, int reset) { return tc_timeout_flag(flag, reset); }
 
-extern "C" int usf_debug_tc_trace(int on, unsigned long long* out, int max_records) {
-  return tc_trace_ctl(on, out, max_records);
-}
-
 extern "C" int usf_linear_bf16(const uint16_t* x, int64_t ldx, const uint16_t* W, int64_t ldw, const float* bias,
                                int relu, void* y, int64_t ldy, int y_is_bf16, int64_t B, int64_t N, int64_t K,
                                usf_stream_t stream) {
@@ -399,7 +395,8 @@ extern "C" int usf_linear_tf32x3(const float* x, const float* x_lo, int64_t ldx,
   ep.out = y;
   ep.ldo = ldy;
   ep.out_bf16 = 0;
-  return tc3_gemm(x, x_lo, ldx, W, W_lo, ldw, B, N, K, tc_pick_bn(N), ep, y_lo, nullptr, as_stream(stream));
+  return tc_split_gemm(x, x_lo, ldx, W, W_lo, ldw, B, N, K, tc_pick_bn(N), ep, y_lo, static_cast<float*>(nullptr),
+                       as_stream(stream));
 }
 
 extern "C" int usf_profile_begin(int max_launches) {

@@ -117,12 +117,11 @@ int tc_gemm(const uint16_t* A, int64_t lda, const uint16_t* W, int64_t ldw, int6
             int64_t K, int bn, const EpiParams& ep, cudaStream_t stream);
 int tc_pick_bn(int64_t N);
 void tc_set_tile_order(int reverse);   // tile walk of the next tcgen05 launches of this thread: 0 first -> last, 1 last -> first
-// 3xTF32 GEMM (fp32 operands as hi + lo parts, fp32-grade accuracy on the tensor cores), see usf_tc3_gemm_kernel
-int tc3_gemm(const float* A, const float* Alo, int64_t lda, const float* W, const float* Wlo, int64_t ldw, int64_t M,
-             int64_t N, int64_t K, int bn, const EpiParams& ep, float* out_lo, float* ub_lo, cudaStream_t stream);
-// bf16x2 GEMM (operands as bf16 hi + lo pairs: fp32-grade at a third of the bf16 rate), see usf_tcb2_gemm_kernel
-int tcb2_gemm(const uint16_t* A, const uint16_t* Alo, int64_t lda, const uint16_t* W, const uint16_t* Wlo, int64_t ldw, int64_t M,
-              int64_t N, int64_t K, int bn, const EpiParams& ep, uint16_t* out_lo, uint16_t* ub_lo, cudaStream_t stream);
+// Split-operand GEMM (operands as hi + lo pairs: fp32-grade accuracy on the tensor cores).  T = float: 3xTF32
+// (usf_tc3_gemm_kernel); T = uint16_t: bf16x2, bf16 pairs at a third of the bf16 rate (usf_tcb2_gemm_kernel).
+template <class T>
+int tc_split_gemm(const T* A, const T* Alo, int64_t lda, const T* W, const T* Wlo, int64_t ldw, int64_t M, int64_t N,
+                  int64_t K, int bn, const EpiParams& ep, T* out_lo, T* ub_lo, cudaStream_t stream);
 int launch_split_rows_bf16x2(const float* x, int64_t ldx, uint16_t* hi, uint16_t* lo, int64_t ldy, int64_t B, int64_t D,
                              float* row_init, float init_value, cudaStream_t stream);
 // hi == NULL: lo against the truncated read of x; hi != NULL (may alias x): hi = x rounded to tf32, lo = x - hi
@@ -140,7 +139,6 @@ int trsm_rows_fast(const float* T, int64_t D, bool lower, bool unit, bool trans,
 int64_t lu_inverse_scratch_floats(int64_t D);
 int lu_inverse(const float* L_raw, const float* U_raw, int64_t D, float* A, float* scratch, cudaStream_t stream);
 int tc_timeout_flag(int* out, int reset);
-int tc_trace_ctl(int on, unsigned long long* out, int max_records);
 int trsm_rows(const float* T, int64_t D, bool lower, bool unit, bool trans, const float* rhs, int64_t ldr,
               const float* bias, float* X, int64_t ldx, int64_t B, cudaStream_t stream);
 

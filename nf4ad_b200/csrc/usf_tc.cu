@@ -2,12 +2,12 @@
 //
 //   acc[m, n] = sum_k A[m, k] * W[n, k]        A: activations (M x K, bf16), W: packed weights (N x K, bf16)
 //
-// Persistent, warp-specialised, 320 threads per CTA, one CTA per SM; by default two CTAs form a pair
-// (cluster of 2, tcgen05 cta_group::2) that owns a 256 x bn output tile:
+// Persistent, warp-specialised, 320 threads per CTA, one CTA per SM; two CTAs form a pair (cluster of 2, tcgen05
+// cta_group::2) that owns a 256 x bn output tile:
 //   warp 0   : TMA producer  -- cp.async.bulk.tensor (128B-swizzled boxes) into a 7-stage smem ring; each CTA of a
 //                               pair stages its own 128 rows of A and HALF of the W tile; both count on the
 //                               leader's mbarrier (one arrive.expect_tx for the pair's bytes)
-//   warp 1   : MMA issuer    -- the leader CTA issues tcgen05.mma (M=128*CG, N=bn<=256, K=16) into TMEM;
+//   warp 1   : MMA issuer    -- the leader CTA issues tcgen05.mma (M=256, N=bn<=256, K=16) into TMEM;
 //                               tcgen05.commit (multicast to both CTAs) releases smem stages / publishes the accumulator
 //   warps 2-9: epilogue      -- tcgen05.ld the fp32 accumulator (double-buffered in TMEM, 2 x 256 cols) and apply
 //                               the layer epilogue (bias / ReLU / coupling / base density); column vectors resident
@@ -17,8 +17,8 @@
 // griddepcontrol.launch_dependents at entry, griddepcontrol.wait after the prologue.
 // Pipelines: smem full/empty mbarriers (TMA <-> MMA), TMEM full/empty mbarriers (MMA <-> epilogue).
 // Every mbarrier wait is bounded (g_tc_timeout flag) so a protocol bug cannot hang the GPU.
-// USF_TC_CTA_GROUP=1 selects the single-CTA variant; DBG=true instantiations carry the pipeline trace and the
-// ablation switches (usf_debug_tc_trace), production launches carry neither.
+// The same CTA-pair pipeline also runs the fused conditioner chain (usf_tc_mlp_coupling_kernel) and, with operands
+// split into (hi, lo) pairs, the fp32-grade tiers (usf_tc3_gemm_kernel: 3xTF32, usf_tcb2_gemm_kernel: bf16x2).
 //
 // Measured bounds (profiles/r1b_*, DESIGN.md section 4): per SM the TMA unit delivers about one 128-byte box row per
 // 3 cycles (232 rows per k-block here = ~700 cycles against 416 of MMA at N=208); the tensor pipe is 65-68 % active
@@ -26,6 +26,8 @@
 #include <cuda.h>
 #include <cuda_fp16.h>
 #include <stdlib.h>
+
+#include <type_traits>
 
 #include "usf_common.cuh"
 
@@ -44,9 +46,8 @@ constexpr int TC_MAX_STAGES = 8;
 constexpr int TC_EPI_COLS = 1024;                    // per-column epilogue vectors resident in smem when N <= this
 constexpr uint32_t TC_EPI_BYTES = 3 * TC_EPI_COLS * 4;  // bias / loc / inv_scale (N <= 1024: whole vectors, staged once;
                                                         // wider outputs: [2 stages][3][256] re-staged per tile)
-// CG = CTAs per MMA (tcgen05 cta_group): 1 = one CTA owns a 128 x bn tile; 2 = a CTA pair (cluster of 2) owns a
-// 256 x bn tile, each CTA staging its own 128 rows of A and HALF of the W tile, which halves the L2->SMEM weight
-// traffic per CTA (the measured bound of the 1-CTA kernel) and the SMEM operand reads per MMA.
+// A CTA pair (cluster of 2) owns a 256 x bn tile, each CTA staging its own 128 rows of A and HALF of the W tile, which
+// halves the L2->SMEM weight traffic per CTA (the measured bound of a single-CTA kernel) and the SMEM operand reads per MMA.
 constexpr uint32_t TC_FIXED_BYTES = TC_BAR_BYTES + TC_EPI_BYTES + 1024;  // barriers + per-tile column vectors + alignment slack
 constexpr uint32_t TC_SMEM_BYTES = 227 * 1024;                           // whole carve-out; the operand ring takes what is left
 constexpr uint32_t TC_TMEM_COLS = 512;
@@ -79,12 +80,11 @@ __device__ __forceinline__ bool mbar_try_wait(uint32_t bar, uint32_t parity) {
 }
 // Bounded wait: returns false (and raises the global flag) if the barrier never completes.  The hot spin is
 // try_wait only; the clock and the global abort flag (an L2 round trip) are looked at once per 1024 failed polls.
-__device__ __forceinline__ bool mbar_wait(uint32_t bar, uint32_t parity, uint32_t backoff_ns = 0) {
+__device__ __forceinline__ bool mbar_wait(uint32_t bar, uint32_t parity) {
   if (mbar_try_wait(bar, parity)) return true;
   uint32_t spins = 0;
   long long t0 = 0;
   for (;;) {
-    if (backoff_ns != 0) __nanosleep(backoff_ns);   // waits off the critical path: do not burn issue slots / power
     if (mbar_try_wait(bar, parity)) return true;
     if ((++spins & 1023u) == 0u) {
       if (*reinterpret_cast<volatile int*>(&g_tc_timeout) != 0) return false;
@@ -98,47 +98,7 @@ __device__ __forceinline__ bool mbar_wait(uint32_t bar, uint32_t parity, uint32_
   }
 }
 
-// Wait with back-off: warps that are far from the critical path (epilogue warps waiting for a whole tile of MMAs, the
-// producer waiting for a ring slot) sleep between polls instead of competing with the MMA warp for the barrier unit.
-__device__ __forceinline__ bool mbar_wait_relaxed(uint32_t bar, uint32_t parity, uint32_t ns) {
-  if (mbar_try_wait(bar, parity)) return true;
-  uint32_t spins = 0;
-  long long t0 = 0;
-  for (;;) {
-    __nanosleep(ns);
-    if (mbar_try_wait(bar, parity)) return true;
-    if ((++spins & 1023u) == 0u) {
-      if (*reinterpret_cast<volatile int*>(&g_tc_timeout) != 0) return false;
-      const long long now = clock64();
-      if (t0 == 0) t0 = now;
-      else if (now - t0 > TC_WAIT_LIMIT_CYCLES) {
-        atomicExch(&g_tc_timeout, 1);
-        return false;
-      }
-    }
-  }
-}
-
-// TMA store of one box (shared -> global, bulk async-group completion); coordinates in elements: c0 = column, c1 = row.
-// Rows / columns outside the tensor are not written.
-__device__ __forceinline__ void tma_store_2d(const CUtensorMap* tmap, uint32_t src_smem, int c0, int c1) {
-  asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.bulk_group [%0, {%2, %3}], [%1];"
-               ::"l"(reinterpret_cast<uint64_t>(tmap)), "r"(src_smem), "r"(c0), "r"(c1)
-               : "memory");
-}
-__device__ __forceinline__ void tma_store_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
-// the staging tile may be overwritten once the stores issued so far have READ it
-__device__ __forceinline__ void tma_store_wait_read() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
-__device__ __forceinline__ void tma_store_wait_all() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
-
-__device__ __forceinline__ void tma_load_2d(uint32_t dst_smem, const CUtensorMap* tmap, uint32_t bar, int c0, int c1) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
-      ::"r"(dst_smem), "l"(reinterpret_cast<uint64_t>(tmap)), "r"(bar), "r"(c0), "r"(c1)
-      : "memory");
-}
-
-// 2-CTA variants: the load lands in this CTA's smem but signals the LEADER CTA's mbarrier (peer bit cleared).
+// TMA load of a CTA pair: the load lands in this CTA's smem but signals the LEADER CTA's mbarrier (peer bit cleared).
 __device__ __forceinline__ void tma_load_2d_2sm(uint32_t dst_smem, const CUtensorMap* tmap, uint32_t bar, int c0, int c1) {
   uint32_t leader_bar;   // shared::cluster address of the same-offset barrier in CTA 0 of the pair
   asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(leader_bar) : "r"(bar), "r"(0));
@@ -202,18 +162,6 @@ __device__ __forceinline__ uint64_t make_smem_desc(uint32_t smem_addr) {
 // kind::f16 instruction descriptor: D=f32, A=B=bf16, both K-major, M=m (128, or 256 for a CTA pair), N=n.
 __device__ __forceinline__ uint32_t make_idesc(uint32_t n, uint32_t m) {
   return (1u << 4) | (1u << 7) | (1u << 10) | ((n >> 3) << 17) | ((m >> 4) << 24);
-}
-
-__device__ __forceinline__ void umma_bf16(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-      ::"r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-__device__ __forceinline__ void umma_commit(uint32_t bar) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
 }
 
 __device__ __forceinline__ void umma_bf16_2sm(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc, uint32_t accumulate) {
@@ -381,48 +329,25 @@ struct TcArgs {
   int64_t M, N, K;
   int bn;        // N-tile width (multiple of 16, <= 256)
   int n_tiles;   // ceil(N / bn)
-  int m_tiles;   // ceil(M / (128 * CG))
+  int m_tiles;   // ceil(M / 256)
   int n_valid;   // valid output columns for fp32 stores / base density (<= N)
   int reverse;                // walk the tiles from the last row tile to the first (see tc_set_tile_order)
   int stages;                 // smem ring depth (<= TC_MAX_STAGES)
   uint32_t stage_bytes;       // bytes per stage (A tile + this CTA's W rows), multiple of 1024
-  uint32_t backoff_ns;        // sleep between polls of the epilogue / producer waits (0 = spin)
-  int dbg;                    // debug experiments (env USF_TC_DBG): 1 = copy-out without the global store, 2 = no copy-out
-  uint32_t out_stage_bytes;   // > 0: bf16 outputs leave through a staging tile in shared memory and TMA stores (see tmO)
-  unsigned long long* trace;  // debug: per-role timestamp records of CTA 0/1 (NULL = off), see usf_debug_tc_trace
   EpiParams ep;
 };
 
-// Debug tracing: record (role, tile, event) with an SM clock stamp.  3 roles x 2 CTAs x TC_TRACE_CAP records.
-constexpr int TC_TRACE_CAP = 2048;
-__device__ unsigned long long g_tc_trace[2 * 3 * TC_TRACE_CAP * 2];
-template <bool DBG>
-__device__ __forceinline__ void tc_trace(unsigned long long* buf, int& n, int tile, int ev) {
-  if (DBG && buf != nullptr && n < TC_TRACE_CAP) {
-    buf[2 * n] = ((unsigned long long)tile << 8) | (unsigned long long)ev;
-    buf[2 * n + 1] = (unsigned long long)clock64();
-    ++n;
-  }
-}
-
-// DBG = true: the instrumented variant (pipeline tracing + ablation switches); production launches use DBG = false, whose
-// producer / MMA loops carry no instrumentation at all (their instruction count is what bounds the MMA issue rate).
-template <int CG, bool DBG>
 __global__ void __launch_bounds__(TC_THREADS, 1)
-usf_tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmW,
-                   const __grid_constant__ CUtensorMap tmO, TcArgs args) {
-  // runtime ring geometry: a stage holds 128 rows of A and bn/CG rows of W (1 KB granularity), as many stages as fit
+usf_tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmW, TcArgs args) {
+  // runtime ring geometry: a stage holds 128 rows of A and bn/2 rows of W (1 KB granularity), as many stages as fit
   const int TC_STAGES = args.stages;
   const uint32_t TC_STAGE_BYTES = args.stage_bytes;
   extern __shared__ uint8_t smem_raw[];
   asm volatile("griddepcontrol.launch_dependents;" ::: "memory");   // the next kernel of the chain may start its prologue
   const uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;
-  // [ring][output staging tile: 128 rows x 64-column blocks of bf16, 16 KB each, 128B-swizzled like an operand tile][barriers]
-  const uint32_t ostage_base = smem_base + TC_STAGES * TC_STAGE_BYTES;
-  const uint32_t bar_base = ostage_base + args.out_stage_bytes;
-  const uint32_t cta_rank = CG == 2 ? cluster_ctarank() : 0u;   // 0 = leader of the pair (issues the MMAs)
-  const int unit = CG == 2 ? (int)(blockIdx.x >> 1) : (int)blockIdx.x;        // persistent work unit (CTA / CTA pair)
-  const int num_units = CG == 2 ? (int)(gridDim.x >> 1) : (int)gridDim.x;
+  const uint32_t bar_base = smem_base + TC_STAGES * TC_STAGE_BYTES;
+  const uint32_t cta_rank = cluster_ctarank();   // 0 = leader of the pair (issues the MMAs)
+  const int unit = (int)(blockIdx.x >> 1), num_units = (int)(gridDim.x >> 1);   // persistent work unit: a CTA pair
   // barrier layout (8 bytes each): full[STAGES], empty[STAGES], tmem_full[2], tmem_empty[2]; then tmem ptr
   auto full_bar = [&](int s) { return bar_base + 8u * s; };
   auto empty_bar = [&](int s) { return bar_base + 8u * (TC_STAGES + s); };
@@ -437,29 +362,22 @@ usf_tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
   if (warp == 0 && lane == 0) {
     for (int s = 0; s < TC_STAGES; ++s) {
       mbar_init(full_bar(s), 1);        // the leader's arrive.expect_tx; the peer's loads only add transaction bytes
-      mbar_init(empty_bar(s), 1);       // one tcgen05.commit (multicast to both CTAs of a pair)
+      mbar_init(empty_bar(s), 1);       // one tcgen05.commit (multicast to both CTAs of the pair)
     }
     for (int a = 0; a < 2; ++a) {
       mbar_init(tfull_bar(a), 1);
-      mbar_init(tempty_bar(a), 8 * CG);  // 8 epilogue warps per CTA, all arriving on the leader's barrier
+      mbar_init(tempty_bar(a), 16);     // 8 epilogue warps per CTA, all arriving on the leader's barrier
     }
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&tmA)) : "memory");
     asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&tmW)) : "memory");
-    if (args.out_stage_bytes != 0) asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&tmO)) : "memory");
   }
   if (warp == 1) {
-    if (CG == 1) {
-      asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(tmem_ptr_addr), "r"(TC_TMEM_COLS) : "memory");
-      asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    } else {
-      asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(tmem_ptr_addr), "r"(TC_TMEM_COLS) : "memory");
-      asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-    }
+    asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(tmem_ptr_addr), "r"(TC_TMEM_COLS) : "memory");
+    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
   }
   tc_fence_before();
-  if (CG == 2) cluster_sync_all();   // the peer's barriers must be initialised before any remote arrive / TMA signal
-  else __syncthreads();
+  cluster_sync_all();   // the peer's barriers must be initialised before any remote arrive / TMA signal
   tc_fence_after();
   uint32_t tmem_base;
   asm volatile("ld.shared.u32 %0, [%1];" : "=r"(tmem_base) : "r"(tmem_ptr_addr) : "memory");
@@ -470,20 +388,9 @@ usf_tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
   asm volatile("griddepcontrol.wait;" ::: "memory");
 
   const int total_tiles = args.m_tiles * args.n_tiles;
-  // trace region of this (CTA, role): only CTAs 0 and 1 record
-  int trn = 0;
-  unsigned long long* trb = nullptr;
-  if (DBG && args.trace != nullptr && blockIdx.x < 2) {
-    const int role = warp == 0 ? 0 : (warp == 1 ? 1 : 2);
-    if (warp <= 2 && lane == 0) trb = args.trace + (size_t)(blockIdx.x * 3 + role) * TC_TRACE_CAP * 2;
-  }
   const int num_kb = (int)((args.K + TC_BK - 1) / TC_BK);
-  // bytes landing per stage on the (leader's) full barrier: every CTA loads 128 rows of A and bn/CG rows of W
-  // debug ablations (usf_debug_tc_trace, bits 8+ of `on`): 1 = epilogue without global stores, 2 = epilogue only
-  // hands the accumulator back, 4 = producer skips the A loads, 8 = producer skips the W loads, 16 = no MMAs issued
-  // the uninstrumented variant honours only the producer-side load ablations (4, 8), requested with bit 0x200
-  const int dbg = DBG ? args.dbg : ((args.dbg & 0x200) ? (args.dbg & 12) : 0);
-  const uint32_t stage_tx = CG * (((dbg & 4) ? 0u : TC_A_BYTES) + ((dbg & 8) ? 0u : (uint32_t)(args.bn / CG) * TC_BK * 2));
+  // bytes landing per stage on the leader's full barrier: each CTA of the pair loads 128 rows of A and bn/2 rows of W
+  const uint32_t stage_tx = 2u * (TC_A_BYTES + (uint32_t)(args.bn / 2) * TC_BK * 2);
 
   if (warp == 0) {
     // ------------------------------------------------------------------ TMA producer (whole warp, one elected lane issues)
@@ -496,31 +403,20 @@ usf_tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
         const int mt = tt / args.n_tiles, nt = tt - mt * args.n_tiles;
         int width = (int)(args.N - (int64_t)nt * args.bn);
         if (width > args.bn) width = args.bn;
-        // a pair splits the tile's N columns evenly: CTA r stages W rows [n0 + r*width/2, +width/2)
-        const int w_row = nt * args.bn + (CG == 2 ? (int)cta_rank * (width >> 1) : 0);
-        const int a_row = (mt * CG + (int)cta_rank) * TC_BM;
+        // the pair splits the tile's N columns evenly: CTA r stages W rows [n0 + r*width/2, +width/2)
+        const int w_row = nt * args.bn + (int)cta_rank * (width >> 1);
+        const int a_row = (mt * 2 + (int)cta_rank) * TC_BM;
         for (int kb = 0; kb < num_kb; ++kb) {
-          if (kb == 0) tc_trace<DBG>(trb, trn, t, 0);
-          ok = (dbg & 32) ? mbar_wait_relaxed(empty_bar(s), ph ^ 1u, 40) : mbar_wait(empty_bar(s), ph ^ 1u, args.backoff_ns);
+          ok = mbar_wait(empty_bar(s), ph ^ 1u);
           if (!ok) break;
-          if (kb == 0) tc_trace<DBG>(trb, trn, t, 1);
-          if (kb == num_kb - 1) tc_trace<DBG>(trb, trn, t, 2);
-          tc_trace<DBG>(trb, trn, t, 4);   // slot acquired
           const uint32_t a_dst = smem_base + s * TC_STAGE_BYTES;
           if (elect_one()) {
-            if (CG == 1) {
-              mbar_expect_tx(full_bar(s), stage_tx);
-              if (!(dbg & 4)) tma_load_2d(a_dst, &tmA, full_bar(s), kb * TC_BK, a_row);
-              if (!(dbg & 8)) tma_load_2d(a_dst + TC_A_BYTES, &tmW, full_bar(s), kb * TC_BK, w_row);
-            } else {
-              // The peer's bytes can only land in the leader's CURRENT phase: its empty barrier for this slot was
-              // released by the commit that followed the MMAs which consumed the slot's previous contents.
-              if (cta_rank == 0) mbar_expect_tx(full_bar(s), stage_tx);
-              if (!(dbg & 4)) tma_load_2d_2sm(a_dst, &tmA, full_bar(s), kb * TC_BK, a_row);
-              if (!(dbg & 8)) tma_load_2d_2sm(a_dst + TC_A_BYTES, &tmW, full_bar(s), kb * TC_BK, w_row);
-            }
+            // The peer's bytes can only land in the leader's CURRENT phase: its empty barrier for this slot was
+            // released by the commit that followed the MMAs which consumed the slot's previous contents.
+            if (cta_rank == 0) mbar_expect_tx(full_bar(s), stage_tx);
+            tma_load_2d_2sm(a_dst, &tmA, full_bar(s), kb * TC_BK, a_row);
+            tma_load_2d_2sm(a_dst + TC_A_BYTES, &tmW, full_bar(s), kb * TC_BK, w_row);
           }
-          tc_trace<DBG>(trb, trn, t, 5);   // loads issued
           if (++s == TC_STAGES) { s = 0; ph ^= 1u; }
         }
       }
@@ -540,62 +436,41 @@ usf_tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
         const int nt = (args.reverse ? total_tiles - 1 - t : t) % args.n_tiles;
         int width = (int)(args.N - (int64_t)nt * args.bn);
         if (width > args.bn) width = args.bn;
-        const uint32_t idesc = make_idesc((uint32_t)width, TC_BM * CG);
-        tc_trace<DBG>(trb, trn, t, 0);
+        const uint32_t idesc = make_idesc((uint32_t)width, 2 * TC_BM);
         ok = mbar_wait(tempty_bar(a), aph ^ 1u);
         if (!ok) break;
-        tc_trace<DBG>(trb, trn, t, 1);
         tc_fence_after();
         const uint32_t d_tmem = tmem_base + (uint32_t)a * TC_MAX_BN;
         for (int kb = 0; kb < num_kb; ++kb) {
           // TMA (async proxy) -> mbarrier -> tcgen05.mma needs no further fence
-          if (DBG && (dbg & 64)) {
-            if (lane == 0) ok = mbar_wait(full_bar(s), ph);
-            ok = __shfl_sync(0xffffffffu, (int)ok, 0) != 0;
-          } else {
-            ok = mbar_wait(full_bar(s), ph);
-          }
+          ok = mbar_wait(full_bar(s), ph);
           if (!ok) break;
-          if (kb == 0) tc_trace<DBG>(trb, trn, t, 2);
-          if (kb == num_kb - 1) tc_trace<DBG>(trb, trn, t, 3);
-          tc_trace<DBG>(trb, trn, t, 4);   // operands landed
           if (elect_one()) {
             // descriptors advance by 32 bytes (2 x 16-byte units) per K=16 step inside the 128-byte swizzle row
             const uint64_t ad0 = desc_hi | (uint64_t)(desc_lo0 + (uint32_t)s * desc_stage);
             const uint64_t bd0 = ad0 + (TC_A_BYTES >> 4);
-            if (!(DBG && (dbg & 16))) {
-              if (kb + 1 < num_kb) {
+            if (kb + 1 < num_kb) {
 #pragma unroll
-                for (int k = 0; k < TC_BK / TC_UMMA_K; ++k) {
-                  if (CG == 1) umma_bf16(d_tmem, ad0 + 2u * k, bd0 + 2u * k, idesc, (kb | k) != 0 ? 1u : 0u);
-                  else umma_bf16_2sm(d_tmem, ad0 + 2u * k, bd0 + 2u * k, idesc, (kb | k) != 0 ? 1u : 0u);
-                }
-              } else {
-                for (int k = 0; k < tail_steps; ++k) {
-                  if (CG == 1) umma_bf16(d_tmem, ad0 + 2u * k, bd0 + 2u * k, idesc, (kb | k) != 0 ? 1u : 0u);
-                  else umma_bf16_2sm(d_tmem, ad0 + 2u * k, bd0 + 2u * k, idesc, (kb | k) != 0 ? 1u : 0u);
-                }
-              }
+              for (int k = 0; k < TC_BK / TC_UMMA_K; ++k)
+                umma_bf16_2sm(d_tmem, ad0 + 2u * k, bd0 + 2u * k, idesc, (kb | k) != 0 ? 1u : 0u);
+            } else {
+              for (int k = 0; k < tail_steps; ++k)
+                umma_bf16_2sm(d_tmem, ad0 + 2u * k, bd0 + 2u * k, idesc, (kb | k) != 0 ? 1u : 0u);
             }
-            if (CG == 1) umma_commit(empty_bar(s));  // smem stage reusable once these MMAs retire
-            else umma_commit_2sm(empty_bar(s));      // ... in both CTAs of the pair
+            umma_commit_2sm(empty_bar(s));   // smem stage reusable in both CTAs once these MMAs retire
           }
-          tc_trace<DBG>(trb, trn, t, 6);   // MMAs + commit issued
           if (++s == TC_STAGES) { s = 0; ph ^= 1u; }
         }
         if (!ok) break;
-        if (elect_one()) {
-          if (CG == 1) umma_commit(tfull_bar(a));    // accumulator ready for the epilogue
-          else umma_commit_2sm(tfull_bar(a));        // (each CTA of the pair holds its own 128 rows in its TMEM)
-        }
+        // accumulator ready for the epilogue (each CTA of the pair holds its own 128 rows in its TMEM)
+        if (elect_one()) umma_commit_2sm(tfull_bar(a));
         a ^= 1;
         if (a == 0) aph ^= 1u;
       }
     }
   } else {
     // ------------------------------------------------------------------ epilogue warps (2..9)
-    // Two warps per TMEM lane group (32 rows): `half` 0/1 takes the even/odd 64-column slabs (bf16 outputs, staged
-    // through a warp-private smem tile for coalesced global access) or the even/odd 16-column chunks (fp32 / density).
+    // Two warps per TMEM lane group (32 rows): `half` 0/1 takes the even/odd 16-column chunks.
     const int lane_grp = warp & 3;  // TMEM lanes [32*lane_grp, +32) are accessible to this warp
     const int half = (warp - 2) >> 2;
     const int et = (int)threadIdx.x - 64;  // 0..255 within the epilogue group
@@ -623,7 +498,7 @@ usf_tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
     for (int t = unit; t < total_tiles; t += num_units) {
       const int tt = args.reverse ? total_tiles - 1 - t : t;
       const int mt = tt / args.n_tiles, nt = tt - mt * args.n_tiles;
-      const int64_t row = (int64_t)(mt * CG + (int)cta_rank) * TC_BM + lane_grp * 32 + lane;
+      const int64_t row = (int64_t)(mt * 2 + (int)cta_rank) * TC_BM + lane_grp * 32 + lane;
       const bool rvalid = row < args.M;
       const int64_t n0 = (int64_t)nt * args.bn;
       int width = (int)(args.N - n0);
@@ -647,75 +522,13 @@ usf_tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
       // (2) coupling: request the first chunk of transformed coordinates of this thread's row (independent of the MMA)
       uint4 cq0 = make_uint4(0, 0, 0, 0), cq1 = cq0;
       if (is_cpl || is_add) cpl_load_u(ep, row, rvalid, nt * ep.C + half * 16, cq0, cq1);
-      tc_trace<DBG>(trb, trn, t, 0);
       if (!resident) asm volatile("bar.sync 1, 256;" ::: "memory");
-      tc_trace<DBG>(trb, trn, t, 1);
 
-      const bool ok = (dbg & 32) ? mbar_wait_relaxed(tfull_bar(a), aph, 100) : mbar_wait(tfull_bar(a), aph, args.backoff_ns);
-      tc_trace<DBG>(trb, trn, t, 2);
-      if (ok) {
+      if (mbar_wait(tfull_bar(a), aph)) {
         tc_fence_after();
         const uint32_t t_base = tmem_base + ((uint32_t)(lane_grp * 32) << 16) + (uint32_t)a * TC_MAX_BN;
-        bool released = false;
 
-        if (dbg & 2) {
-          // ablation: accumulator handed straight back
-        } else if ((ep.mode == EPI_BIAS || ep.mode == EPI_BIAS_RELU) && ep.out_bf16 && args.out_stage_bytes != 0) {
-          // bf16 activations through shared memory and TMA stores: every full 64-column block of the tile is written
-          // into a staging tile in the swizzled K-major layout (row-per-thread 16-byte pieces, conflict-free) and
-          // leaves as ONE bulk tensor store of 128 rows x 128 bytes; rows past M and columns past N are clipped by
-          // the tensor map.  The remainder of a tile that is not a multiple of 64 columns wide is stored directly.
-          const int nfull = width >> 6;
-          const int rloc = lane_grp * 32 + lane;
-          uint4* ost = reinterpret_cast<uint4*>(smem_raw + (ostage_base - smem_u32(smem_raw)));
-          // the previous tile's stores must have read the staging tile before it is overwritten
-          if (et == 0) tma_store_wait_read();
-          asm volatile("bar.sync 1, 256;" ::: "memory");
-          for (int c = half * 16; c < width; c += 32) {
-            float v[16];
-            tmem_ld16(t_base + c, v);
-            tmem_ld_wait();
-            const float4* bv = reinterpret_cast<const float4*>(ev + c);
-#pragma unroll
-            for (int j4 = 0; j4 < 4; ++j4) {
-              const float4 b4 = bv[j4];
-              v[4 * j4] += b4.x; v[4 * j4 + 1] += b4.y; v[4 * j4 + 2] += b4.z; v[4 * j4 + 3] += b4.w;
-            }
-            if (ep.mode == EPI_BIAS_RELU) {
-#pragma unroll
-              for (int j = 0; j < 16; ++j) v[j] = fmaxf(v[j], 0.f);
-            }
-            uint4 q0, q1;
-            q0.x = pack_bf16x2(v[0], v[1]);   q0.y = pack_bf16x2(v[2], v[3]);
-            q0.z = pack_bf16x2(v[4], v[5]);   q0.w = pack_bf16x2(v[6], v[7]);
-            q1.x = pack_bf16x2(v[8], v[9]);   q1.y = pack_bf16x2(v[10], v[11]);
-            q1.z = pack_bf16x2(v[12], v[13]); q1.w = pack_bf16x2(v[14], v[15]);
-            const int blk = c >> 6;
-            if (blk < nfull) {
-              const int p = (c & 63) >> 3;    // 16-byte piece within the 128-byte row of block `blk`
-              uint4* rowp = ost + (size_t)blk * (TC_A_BYTES / 16) + rloc * 8;
-              rowp[p ^ (rloc & 7)] = q0;
-              rowp[(p + 1) ^ (rloc & 7)] = q1;
-            } else if (rvalid) {
-              st_global_256(reinterpret_cast<uint16_t*>(ep.out) + row * ep.ldo + n0 + c, q0, q1);
-            }
-          }
-          // the accumulator is drained: hand the TMEM buffer back before the staging tile is synchronised and stored
-          tc_fence_before();
-          __syncwarp();
-          if (lane == 0) {
-            if (CG == 1 || cta_rank == 0) mbar_arrive(tempty_bar(a));
-            else mbar_arrive_cluster(tempty_bar(a), 0);
-          }
-          released = true;
-          asm volatile("fence.proxy.async.shared::cta;" ::: "memory");   // generic-proxy writes -> visible to the TMA store
-          asm volatile("bar.sync 1, 256;" ::: "memory");
-          if (et == 0) {
-            const int r0 = (mt * CG + (int)cta_rank) * TC_BM;
-            for (int b = 0; b < nfull; ++b) tma_store_2d(&tmO, ostage_base + (uint32_t)b * TC_A_BYTES, (int)n0 + b * 64, r0);
-            tma_store_commit();
-          }
-        } else if ((ep.mode == EPI_BIAS || ep.mode == EPI_BIAS_RELU) && ep.out_bf16) {
+        if ((ep.mode == EPI_BIAS || ep.mode == EPI_BIAS_RELU) && ep.out_bf16) {
           for (int c = half * 16; c < width; c += 32) {
             float v[16];
             tmem_ld16(t_base + c, v);
@@ -736,11 +549,10 @@ usf_tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
               q0.z = pack_bf16x2(v[4], v[5]);   q0.w = pack_bf16x2(v[6], v[7]);
               q1.x = pack_bf16x2(v[8], v[9]);   q1.y = pack_bf16x2(v[10], v[11]);
               q1.z = pack_bf16x2(v[12], v[13]); q1.w = pack_bf16x2(v[14], v[15]);
-              if (!(dbg & 1) || q0.x == 0x12345678u)
-                st_global_256(reinterpret_cast<uint16_t*>(ep.out) + row * ep.ldo + n0 + c, q0, q1);
+              st_global_256(reinterpret_cast<uint16_t*>(ep.out) + row * ep.ldo + n0 + c, q0, q1);
             }
           }
-        } else if (ep.mode == EPI_BIAS || ep.mode == EPI_BIAS_RELU) {
+        } else if (ep.mode == EPI_BIAS || ep.mode == EPI_BIAS_RELU) {   // fp32 output
           for (int c = half * 16; c < width; c += 32) {
             float v[16];
             tmem_ld16(t_base + c, v);
@@ -756,27 +568,16 @@ usf_tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
 #pragma unroll
                 for (int j = 0; j < 16; ++j) v[j] = fmaxf(v[j], 0.f);
               }
-              if (ep.out_bf16) {
-                uint4 q0, q1;
-                q0.x = pack_bf16x2(v[0], v[1]);   q0.y = pack_bf16x2(v[2], v[3]);
-                q0.z = pack_bf16x2(v[4], v[5]);   q0.w = pack_bf16x2(v[6], v[7]);
-                q1.x = pack_bf16x2(v[8], v[9]);   q1.y = pack_bf16x2(v[10], v[11]);
-                q1.z = pack_bf16x2(v[12], v[13]); q1.w = pack_bf16x2(v[14], v[15]);
-                uint4* dst = reinterpret_cast<uint4*>(reinterpret_cast<uint16_t*>(ep.out) + row * ep.ldo + n0 + c);
-                dst[0] = q0;
-                dst[1] = q1;
+              float* dst = reinterpret_cast<float*>(ep.out) + row * ep.ldo + n0 + c;
+              if (n0 + c + 16 <= args.n_valid && (reinterpret_cast<uintptr_t>(dst) & 15) == 0) {
+                // full, 16-byte aligned chunk (the training GEMMs: fp32 gradients / activations): 4 x 128-bit stores
+#pragma unroll
+                for (int j4 = 0; j4 < 4; ++j4)
+                  reinterpret_cast<float4*>(dst)[j4] = make_float4(v[4 * j4], v[4 * j4 + 1], v[4 * j4 + 2], v[4 * j4 + 3]);
               } else {
-                float* dst = reinterpret_cast<float*>(ep.out) + row * ep.ldo + n0 + c;
-                if (n0 + c + 16 <= args.n_valid && (reinterpret_cast<uintptr_t>(dst) & 15) == 0) {
-                  // full, 16-byte aligned chunk (the training GEMMs: fp32 gradients / activations): 4 x 128-bit stores
 #pragma unroll
-                  for (int j4 = 0; j4 < 4; ++j4)
-                    reinterpret_cast<float4*>(dst)[j4] = make_float4(v[4 * j4], v[4 * j4 + 1], v[4 * j4 + 2], v[4 * j4 + 3]);
-                } else {
-#pragma unroll
-                  for (int j = 0; j < 16; ++j)
-                    if (n0 + c + j < args.n_valid) dst[j] = v[j];
-                }
+                for (int j = 0; j < 16; ++j)
+                  if (n0 + c + j < args.n_valid) dst[j] = v[j];
               }
             }
           }
@@ -814,29 +615,23 @@ usf_tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
         }
 
         // accumulator drained: hand the TMEM buffer back to the MMA warp
-        if (!released) {
-          tc_fence_before();
-          __syncwarp();
-          if (lane == 0) {
-            if (CG == 1 || cta_rank == 0) mbar_arrive(tempty_bar(a));
-            else mbar_arrive_cluster(tempty_bar(a), 0);
-          }
+        tc_fence_before();
+        __syncwarp();
+        if (lane == 0) {
+          if (cta_rank == 0) mbar_arrive(tempty_bar(a));
+          else mbar_arrive_cluster(tempty_bar(a), 0);
         }
-        tc_trace<DBG>(trb, trn, t, 3);
       }
       a ^= 1;
       if (a == 0) aph ^= 1u;
     }
-    if (args.out_stage_bytes != 0 && et == 0) tma_store_wait_all();   // the last tile's bulk stores complete before exit
   }
 
   tc_fence_before();
-  if (CG == 2) cluster_sync_all();   // the peer may still be reading this CTA's smem / arriving on its barriers
-  else __syncthreads();
+  cluster_sync_all();   // the peer may still be reading this CTA's smem / arriving on its barriers
   if (warp == 1) {
     tc_fence_after();
-    if (CG == 1) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(TC_TMEM_COLS) : "memory");
-    else asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(TC_TMEM_COLS) : "memory");
+    asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(TC_TMEM_COLS) : "memory");
   }
 }
 
@@ -885,11 +680,8 @@ struct MlpArgs {
   const float* bias[MLP_MAX_LAYERS];
   EpiParams ep;                  // coupling epilogue of the last layer
   int reverse;                   // walk the row tiles from the last to the first (see tc_set_tile_order)
-  uint32_t backoff_ns;           // sleep between polls of the epilogue / producer waits (0 = spin)
-  unsigned long long* trace;     // debug timeline (see usf_debug_tc_trace); events use tile = (m_tile << 4) | gemm index
 };
 
-template <bool DBG>
 __global__ void __launch_bounds__(MLP_THREADS, 1)
 usf_tc_mlp_coupling_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ MlpMaps maps, MlpArgs args) {
   extern __shared__ uint8_t smem_raw[];
@@ -941,12 +733,6 @@ usf_tc_mlp_coupling_kernel(const __grid_constant__ CUtensorMap tmA, const __grid
   // the activation buffers, so wait for it to complete (a no-op when the launch carried no such dependency).
   asm volatile("griddepcontrol.wait;" ::: "memory");
   const int L = args.L;
-  int trn = 0;
-  unsigned long long* trb = nullptr;
-  if (DBG && args.trace != nullptr && blockIdx.x < 2) {
-    const int role = warp == 0 ? 0 : (warp == 1 ? 1 : 2);
-    if (warp <= 2 && lane == 0) trb = args.trace + (size_t)(blockIdx.x * 3 + role) * TC_TRACE_CAP * 2;
-  }
 
   if (warp == 0) {
     // ------------------------------------------------------------------ TMA producer (both CTAs; whole warp, elected lane issues)
@@ -956,7 +742,7 @@ usf_tc_mlp_coupling_kernel(const __grid_constant__ CUtensorMap tmA, const __grid
       bool ok = true;
       // one box into the next free slot; the pair's bytes are accounted on the leader's barrier
       auto load = [&](const CUtensorMap* tm, uint32_t bytes_per_cta, int c0, int c1) {
-        ok = mbar_wait(empty_bar(s), ph ^ 1u, args.backoff_ns);
+        ok = mbar_wait(empty_bar(s), ph ^ 1u);
         if (!ok) return;
         if (elect_one()) {
           if (cta_rank == 0) mbar_expect_tx(full_bar(s), 2u * bytes_per_cta);
@@ -1009,11 +795,8 @@ usf_tc_mlp_coupling_kernel(const __grid_constant__ CUtensorMap tmA, const __grid
             int width = args.N[l] - nt * args.bn[l];
             if (width > args.bn[l]) width = args.bn[l];
             const uint32_t idesc = make_idesc((uint32_t)width, TC_BM * 2);
-            const int gi = (t << 4) | (l * 4 + nt);
-            tc_trace<DBG>(trb, trn, gi, 0);
             ok = mbar_wait(tempty_bar(a), aph ^ 1u);
             if (!ok) break;
-            tc_trace<DBG>(trb, trn, gi, 1);
             tc_fence_after();
             const uint32_t d_tmem = tmem_base + (uint32_t)a * TC_MAX_BN;
             for (int kb = 0; kb < nkb; ++kb) {
@@ -1035,7 +818,6 @@ usf_tc_mlp_coupling_kernel(const __grid_constant__ CUtensorMap tmA, const __grid
               }
               ok = mbar_wait(full_bar(s), ph);
               if (!ok) break;
-              if (kb == 0) tc_trace<DBG>(trb, trn, gi, 2);
               int krem = args.K[l] - kb * TC_BK;
               if (krem > TC_BK) krem = TC_BK;
               const int ksteps = (krem + TC_UMMA_K - 1) / TC_UMMA_K;
@@ -1057,7 +839,6 @@ usf_tc_mlp_coupling_kernel(const __grid_constant__ CUtensorMap tmA, const __grid
             }
             if (!ok) break;
             if (elect_one()) umma_commit_2sm(tfull_bar(a));
-            tc_trace<DBG>(trb, trn, gi, 3);
             a ^= 1;
             if (a == 0) aph ^= 1u;
           }
@@ -1087,22 +868,18 @@ usf_tc_mlp_coupling_kernel(const __grid_constant__ CUtensorMap tmA, const __grid
       const int64_t row = (int64_t)((args.reverse ? args.m_tiles - 1 - t : t) * 2 + (int)cta_rank) * TC_BM + rloc;
       const bool rvalid = row < args.M;
       // accumulator hand-over: wait until the MMAs of the next GEMM of the chain are complete / give the buffer back
-      auto acquire = [&](int gi) -> bool {
-        tc_trace<DBG>(trb, trn, gi, 0);
-        const bool ok = mbar_wait(tfull_bar(a), aph, args.backoff_ns);
-        tc_trace<DBG>(trb, trn, gi, 2);
+      auto acquire = [&]() -> bool {
+        const bool ok = mbar_wait(tfull_bar(a), aph);
         if (ok) tc_fence_after();
         return ok;
       };
-      auto release = [&](int gi, bool hidden) {
+      auto release = [&]() {
         tc_fence_before();
         __syncwarp();
         if (lane == 0) {
           if (cta_rank == 0) mbar_arrive(tempty_bar(a));
           else mbar_arrive_cluster(tempty_bar(a), 0);
-          (void)hidden;
         }
-        tc_trace<DBG>(trb, trn, gi, 3);
       };
       auto advance = [&]() {
         a ^= 1;
@@ -1116,8 +893,7 @@ usf_tc_mlp_coupling_kernel(const __grid_constant__ CUtensorMap tmA, const __grid
       for (int l = 0; l + 1 < L; ++l) {
         const int width = args.N[l];
         const float* ev = epi + args.boff[l];
-        const int gi = (t << 4) | (l * 4);
-        if (acquire(gi)) {
+        if (acquire()) {
           const uint32_t t_base = tmem_base + ((uint32_t)(lane_grp * 32) << 16) + (uint32_t)a * TC_MAX_BN;
           // chunk i of this warp = columns [16*part + 64*i, +16): one 16-byte-pair piece of k-block i of the next
           // layer's operand A.  After each chunk the warp publishes its part of that k-block (hready[i]), so the MMA
@@ -1162,7 +938,7 @@ usf_tc_mlp_coupling_kernel(const __grid_constant__ CUtensorMap tmA, const __grid
               else mbar_arrive_cluster(hready_bar(i), 0);
             }
           }
-          release(gi, false);
+          release();
         }
         advance();
       }
@@ -1176,8 +952,7 @@ usf_tc_mlp_coupling_kernel(const __grid_constant__ CUtensorMap tmA, const __grid
       if (half * 16 >= C) {
         // no chunk of any tile belongs to this warp (narrow tiles): only hand the accumulators back
         for (int nt = 0; nt < ntl; ++nt) {
-          const int gi = (t << 4) | ((L - 1) * 4 + nt);
-          if (acquire(gi)) release(gi, false);
+          if (acquire()) release();
           advance();
         }
       } else {
@@ -1189,14 +964,13 @@ usf_tc_mlp_coupling_kernel(const __grid_constant__ CUtensorMap tmA, const __grid
           if (nc >= C) { nc = half * 16; nnt = nt + 1; }
           uint4 nq0 = make_uint4(0, 0, 0, 0), nq1 = nq0;
           if (nnt < ntl) cpl_load_u(ep, row, rvalid, nnt * C + nc, nq0, nq1);
-          const int gi = (t << 4) | ((L - 1) * 4 + nt);
           if (c == half * 16) {   // first chunk of the tile
-            ok = acquire(gi);
+            ok = acquire();
             t_tile = tmem_base + ((uint32_t)(lane_grp * 32) << 16) + (uint32_t)a * TC_MAX_BN;
           }
           if (ok) cpl_chunk_dispatch(ep.mode, t_tile, c, evl + nt * bnl, ep, k1, row, rvalid, nt * C + c, cq0, cq1, lsum);
           if (nnt != nt) {        // last chunk of the tile
-            if (ok) release(gi, false);
+            if (ok) release();
             advance();
           }
           cq0 = nq0;
@@ -1220,25 +994,27 @@ usf_tc_mlp_coupling_kernel(const __grid_constant__ CUtensorMap tmA, const __grid
 
 
 // ================================================================================================
-// 3xTF32 GEMM: fp32-grade accuracy on the tensor cores (the <= 1e-4 tier without the FFMA pipe).
-// Every fp32 operand is used as hi + lo, hi = the value the tensor core sees when it reads fp32 as tf32 (it drops the
-// low 13 mantissa bits), lo = a - hi (exact in fp32, precomputed by the producing kernel / at weight-pack time):
-//     a w ~= a_hi w_hi + a_hi w_lo + a_lo w_hi            (the dropped a_lo w_lo term is ~2^-21 relative)
-// three tcgen05.mma.kind::tf32 per K=8 step into the same fp32 TMEM accumulator.  Same CTA-pair structure as
-// usf_tc_gemm_kernel; a k-block is 32 fp32 columns (128-byte rows), a stage holds [A_hi | A_lo | W_hi | W_lo].
-// Epilogues write the fp32 result AND its low part (the next GEMM's A_lo), the coupling uses precise tanhf / expf.
+// Split-operand GEMMs: fp32-grade accuracy on the tensor cores.  Every operand is a pair hi + lo and each MMA step
+// issues three MMAs into the same fp32 TMEM accumulator:
+//     a w ~= a_hi w_hi + a_hi w_lo + a_lo w_hi
+// Same CTA-pair pipeline as usf_tc_gemm_kernel; a stage holds [A_hi | A_lo | W_hi | W_lo] of one k-block (128-byte
+// rows).  Epilogues write their results as (hi, lo) pairs again, the next GEMM's operands.  Two operand formats:
+//   3xTF32 (usf_tc3_gemm_kernel, the <= 1e-4 tier without the FFMA pipe): fp32 hi = the value the tensor core sees
+//     when it reads fp32 as tf32 (it drops the low 13 mantissa bits), lo = a - hi (exact in fp32, precomputed by the
+//     producing kernel / at weight-pack time).  k-blocks of 32 columns, kind::tf32 MMAs of K=8; the dropped
+//     a_lo w_lo term is ~2^-21 relative.
+//   bf16x2 (usf_tcb2_gemm_kernel: the bf16 rate / 3, twice the 3xTF32 rate at half its operand bytes): hi = bf16(v),
+//     lo = bf16(v - hi), 16 mantissa bits together.  k-blocks of 64 columns, kind::f16 MMAs of K=16; the dropped term
+//     is ~2^-16 relative.
 // ================================================================================================
-constexpr int T3_BK = 32;
-constexpr int T3_UMMA_K = 8;
-
-struct Tc3Args {
+template <class T>
+struct SplitArgs {
   int64_t M, N, K;
   int bn, n_tiles, m_tiles, n_valid, stages;
   uint32_t stage_bytes, w_bytes;   // w_bytes: this CTA's W rows of one k-block, rounded up to 1 KB
-  uint32_t backoff_ns;
   EpiParams ep;
-  float* out_lo;    // EPI_BIAS*: low part of the output (same leading dimension as ep.out), may be NULL
-  float* ub_lo;     // coupling modes: low part of the transformed columns (same leading dimension as ep.ub)
+  T* out_lo;    // EPI_BIAS*: low part of the output (same leading dimension as ep.out); NULL: plain fp32 output
+  T* ub_lo;     // coupling modes: low part of the transformed columns (same leading dimension as ep.ub)
 };
 
 __device__ __forceinline__ void umma_tf32_2sm(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc, uint32_t accumulate) {
@@ -1257,7 +1033,7 @@ __device__ __forceinline__ uint32_t make_idesc_tf32(uint32_t n, uint32_t m) {
 // lo = v - hi is exact in fp32 and at most 2^-12 |v|
 __device__ __forceinline__ float tf32_hi(float v) { return __uint_as_float((__float_as_uint(v) + 0x1000u) & 0xFFFFE000u); }
 
-// tanh / exp for the fp32-grade tier from two MUFU ops each instead of the ~25-instruction libm paths:
+// tanh / exp for the fp32-grade tiers from two MUFU ops each instead of the ~25-instruction libm paths:
 //   tanh(x) = 1 - 2 / (exp(2x) + 1)   (ex2.approx: 2^-22 relative; absolute error of the result ~1e-7, which is what
 //   the log-det sum sees; saturates correctly for |x| large: ex2 -> inf or 0)
 __device__ __forceinline__ float ex2_fast(float x) {
@@ -1273,313 +1049,6 @@ __device__ __forceinline__ void st16_f32(float* dst, const float (&v)[16]) {
     reinterpret_cast<float4*>(dst)[j4] = make_float4(v[4 * j4], v[4 * j4 + 1], v[4 * j4 + 2], v[4 * j4 + 3]);
 }
 
-__global__ void __launch_bounds__(TC_THREADS, 1)
-usf_tc3_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmAlo,
-                    const __grid_constant__ CUtensorMap tmW, const __grid_constant__ CUtensorMap tmWlo, Tc3Args args) {
-  const int STAGES = args.stages;
-  const uint32_t STAGE_BYTES = args.stage_bytes;
-  extern __shared__ uint8_t smem_raw[];
-  asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-  const uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;
-  const uint32_t bar_base = smem_base + STAGES * STAGE_BYTES;
-  const uint32_t cta_rank = cluster_ctarank();
-  const int unit = (int)(blockIdx.x >> 1), num_units = (int)(gridDim.x >> 1);
-  auto full_bar = [&](int s) { return bar_base + 8u * s; };
-  auto empty_bar = [&](int s) { return bar_base + 8u * (STAGES + s); };
-  auto tfull_bar = [&](int a) { return bar_base + 8u * (2 * STAGES + a); };
-  auto tempty_bar = [&](int a) { return bar_base + 8u * (2 * STAGES + 2 + a); };
-  const uint32_t tmem_ptr_addr = bar_base + 8u * (2 * STAGES + 4);
-  const uint32_t epi_base = bar_base + TC_BAR_BYTES;
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-
-  if (warp == 0 && lane == 0) {
-    for (int s = 0; s < STAGES; ++s) {
-      mbar_init(full_bar(s), 1);
-      mbar_init(empty_bar(s), 1);
-    }
-    for (int a = 0; a < 2; ++a) {
-      mbar_init(tfull_bar(a), 1);
-      mbar_init(tempty_bar(a), 16);
-    }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(tmem_ptr_addr), "r"(TC_TMEM_COLS) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-  }
-  tc_fence_before();
-  cluster_sync_all();
-  tc_fence_after();
-  uint32_t tmem_base;
-  asm volatile("ld.shared.u32 %0, [%1];" : "=r"(tmem_base) : "r"(tmem_ptr_addr) : "memory");
-  asm volatile("griddepcontrol.wait;" ::: "memory");
-
-  const int total_tiles = args.m_tiles * args.n_tiles;
-  const int num_kb = (int)((args.K + T3_BK - 1) / T3_BK);
-  const uint32_t w_rows_bytes = (uint32_t)(args.bn >> 1) * 128u;
-  const uint32_t stage_tx = 2u * (2u * TC_A_BYTES + 2u * w_rows_bytes);
-  const uint32_t off_alo = TC_A_BYTES, off_w = 2u * TC_A_BYTES, off_wlo = 2u * TC_A_BYTES + args.w_bytes;
-
-  if (warp == 0) {
-    int s = 0;
-    uint32_t ph = 0;
-    bool ok = true;
-    for (int t = unit; t < total_tiles && ok; t += num_units) {
-      const int mt = t / args.n_tiles, nt = t - mt * args.n_tiles;
-      int width = (int)(args.N - (int64_t)nt * args.bn);
-      if (width > args.bn) width = args.bn;
-      const int w_row = nt * args.bn + (int)cta_rank * (width >> 1);
-      const int a_row = (mt * 2 + (int)cta_rank) * TC_BM;
-      for (int kb = 0; kb < num_kb; ++kb) {
-        ok = mbar_wait(empty_bar(s), ph ^ 1u, args.backoff_ns);
-        if (!ok) break;
-        const uint32_t dst = smem_base + s * STAGE_BYTES;
-        if (elect_one()) {
-          if (cta_rank == 0) mbar_expect_tx(full_bar(s), stage_tx);
-          tma_load_2d_2sm(dst, &tmA, full_bar(s), kb * T3_BK, a_row);
-          tma_load_2d_2sm(dst + off_alo, &tmAlo, full_bar(s), kb * T3_BK, a_row);
-          tma_load_2d_2sm(dst + off_w, &tmW, full_bar(s), kb * T3_BK, w_row);
-          tma_load_2d_2sm(dst + off_wlo, &tmWlo, full_bar(s), kb * T3_BK, w_row);
-        }
-        if (++s == STAGES) { s = 0; ph ^= 1u; }
-      }
-    }
-  } else if (warp == 1) {
-    if (cta_rank == 0) {
-      int s = 0, a = 0;
-      uint32_t ph = 0, aph = 0;
-      bool ok = true;
-      const int tail_steps = ((int)args.K - (num_kb - 1) * T3_BK + T3_UMMA_K - 1) / T3_UMMA_K;
-      const uint64_t desc_hi = make_smem_desc(0);
-      const uint32_t lo0 = (smem_base & 0x3FFFFu) >> 4, stage16 = STAGE_BYTES >> 4;
-      for (int t = unit; t < total_tiles && ok; t += num_units) {
-        const int nt = t % args.n_tiles;
-        int width = (int)(args.N - (int64_t)nt * args.bn);
-        if (width > args.bn) width = args.bn;
-        const uint32_t idesc = make_idesc_tf32((uint32_t)width, 2 * TC_BM);
-        ok = mbar_wait(tempty_bar(a), aph ^ 1u);
-        if (!ok) break;
-        tc_fence_after();
-        const uint32_t d_tmem = tmem_base + (uint32_t)a * TC_MAX_BN;
-        for (int kb = 0; kb < num_kb; ++kb) {
-          ok = mbar_wait(full_bar(s), ph);
-          if (!ok) break;
-          if (elect_one()) {
-            const uint64_t ah = desc_hi | (uint64_t)(lo0 + (uint32_t)s * stage16);
-            const uint64_t al = ah + (off_alo >> 4), wh = ah + (off_w >> 4), wl = ah + (off_wlo >> 4);
-            const int ksteps = kb + 1 < num_kb ? T3_BK / T3_UMMA_K : tail_steps;
-            for (int k = 0; k < ksteps; ++k) {
-              umma_tf32_2sm(d_tmem, ah + 2u * k, wh + 2u * k, idesc, (kb | k) != 0 ? 1u : 0u);
-              umma_tf32_2sm(d_tmem, ah + 2u * k, wl + 2u * k, idesc, 1u);
-              umma_tf32_2sm(d_tmem, al + 2u * k, wh + 2u * k, idesc, 1u);
-            }
-            umma_commit_2sm(empty_bar(s));
-          }
-          if (++s == STAGES) { s = 0; ph ^= 1u; }
-        }
-        if (!ok) break;
-        if (elect_one()) umma_commit_2sm(tfull_bar(a));
-        a ^= 1;
-        if (a == 0) aph ^= 1u;
-      }
-    }
-  } else {
-    const int lane_grp = warp & 3;
-    const int half = (warp - 2) >> 2;
-    const int et = (int)threadIdx.x - 64;
-    const EpiParams& ep = args.ep;
-    float* epi = reinterpret_cast<float*>(smem_raw + (epi_base - smem_u32(smem_raw)));
-    const int mode = ep.mode;
-    const bool is_cpl = mode == EPI_COUPLING_INV || mode == EPI_COUPLING_FWD;
-    const bool is_add = mode == EPI_ADD_INV || mode == EPI_ADD_FWD;
-    const bool is_base = mode == EPI_BASE_NORMAL || mode == EPI_BASE_LAPLACE;
-    // column vectors resident for the whole kernel (host guarantees N <= TC_EPI_COLS)
-    for (int i = et; i < (int)args.N; i += 256) {
-      epi[i] = ep.bias != nullptr ? ep.bias[i] : 0.f;
-      if (is_base) {
-        const bool v2 = i < args.n_valid && ep.loc != nullptr;
-        epi[TC_EPI_COLS + i] = v2 ? ep.loc[i] : 0.f;
-        epi[2 * TC_EPI_COLS + i] = v2 ? ep.inv_scale[i] : 0.f;
-      }
-    }
-    asm volatile("bar.sync 1, 256;" ::: "memory");
-    int a = 0;
-    uint32_t aph = 0;
-    for (int t = unit; t < total_tiles; t += num_units) {
-      const int mt = t / args.n_tiles, nt = t - mt * args.n_tiles;
-      const int64_t row = (int64_t)(mt * 2 + (int)cta_rank) * TC_BM + lane_grp * 32 + lane;
-      const bool rvalid = row < args.M;
-      const int64_t n0 = (int64_t)nt * args.bn;
-      int width = (int)(args.N - n0);
-      if (width > args.bn) width = args.bn;
-      const float* ev = epi + n0;
-      const bool ok = mbar_wait(tfull_bar(a), aph, args.backoff_ns);
-      if (ok) {
-        tc_fence_after();
-        const uint32_t t_base = tmem_base + ((uint32_t)(lane_grp * 32) << 16) + (uint32_t)a * TC_MAX_BN;
-        if (mode == EPI_BIAS || mode == EPI_BIAS_RELU) {
-          for (int c = half * 16; c < width; c += 32) {
-            float v[16];
-            tmem_ld16(t_base + c, v);
-            tmem_ld_wait();
-            if (rvalid) {
-#pragma unroll
-              for (int j = 0; j < 16; ++j) {
-                v[j] += ev[c + j];
-                if (mode == EPI_BIAS_RELU) v[j] = fmaxf(v[j], 0.f);
-              }
-              float* dst = reinterpret_cast<float*>(ep.out) + row * ep.ldo + n0 + c;
-              // with a low-part twin the output travels as (hi, lo), hi + lo = v; without one it is v itself
-              float l[16];
-              if (args.out_lo != nullptr) {
-#pragma unroll
-                for (int j = 0; j < 16; ++j) {
-                  const float h = tf32_hi(v[j]);
-                  l[j] = v[j] - h;
-                  v[j] = h;
-                }
-              }
-              if (n0 + c + 16 <= args.n_valid && (reinterpret_cast<uintptr_t>(dst) & 15) == 0) {
-                st16_f32(dst, v);
-                if (args.out_lo != nullptr) st16_f32(args.out_lo + row * ep.ldo + n0 + c, l);
-              } else {
-#pragma unroll
-                for (int j = 0; j < 16; ++j)
-                  if (n0 + c + j < args.n_valid) {
-                    dst[j] = v[j];
-                    if (args.out_lo != nullptr) args.out_lo[row * ep.ldo + n0 + c + j] = l[j];
-                  }
-              }
-            }
-          }
-        } else if (is_cpl || is_add) {
-          const int C = ep.C;
-          float lsum = 0.f;
-          for (int c = half * 16; c < C; c += 32) {
-            float sv[16], tv[16];
-            if (is_cpl) {
-              tmem_ld16(t_base + c, sv);
-              tmem_ld16(t_base + C + c, tv);
-            } else {
-              tmem_ld16(t_base + c, tv);
-            }
-            tmem_ld_wait();
-            const int coord0 = nt * C + c;
-            if (rvalid && coord0 < ep.Db) {
-              float* up = reinterpret_cast<float*>(ep.ub) + row * ep.ldub + coord0;
-              float* ulo = args.ub_lo + row * ep.ldub + coord0;
-              const float* bt = is_cpl ? ev + C + c : ev + c;
-              const bool full = coord0 + 16 <= ep.Db && (reinterpret_cast<uintptr_t>(up) & 31) == 0;
-              float u[16];
-              if (full) {     // 64 contiguous bytes of this thread's row per array: two 256-bit loads each; u = hi + lo
-                uint4 q[4], ql[4];
-                ld_global_256(up, q[0], q[1]);
-                ld_global_256(up + 8, q[2], q[3]);
-                ld_global_256(ulo, ql[0], ql[1]);
-                ld_global_256(ulo + 8, ql[2], ql[3]);
-#pragma unroll
-                for (int i = 0; i < 4; ++i) {
-                  u[4 * i] = __uint_as_float(q[i].x) + __uint_as_float(ql[i].x);
-                  u[4 * i + 1] = __uint_as_float(q[i].y) + __uint_as_float(ql[i].y);
-                  u[4 * i + 2] = __uint_as_float(q[i].z) + __uint_as_float(ql[i].z);
-                  u[4 * i + 3] = __uint_as_float(q[i].w) + __uint_as_float(ql[i].w);
-                }
-              } else {
-#pragma unroll
-                for (int j = 0; j < 16; ++j) u[j] = coord0 + j < ep.Db ? up[j] + ulo[j] : 0.f;
-              }
-#pragma unroll
-              for (int j = 0; j < 16; ++j) {
-                const float tt = tv[j] + bt[j];
-                if (is_cpl) {
-                  const float ls = ep.clamp * tanh_mufu(sv[j] + ev[c + j]);   // padded coordinates: s = 0 -> ls = 0
-                  const float e = ex2_fast((mode == EPI_COUPLING_INV ? -ls : ls) * 1.4426950408889634f);
-                  u[j] = mode == EPI_COUPLING_INV ? (u[j] - tt) * e : fmaf(u[j], e, tt);
-                  lsum += ls;
-                } else {
-                  u[j] = mode == EPI_ADD_INV ? u[j] - tt : u[j] + tt;
-                }
-              }
-              float l[16];
-#pragma unroll
-              for (int j = 0; j < 16; ++j) {
-                const float h = tf32_hi(u[j]);
-                l[j] = u[j] - h;
-                u[j] = h;
-              }
-              if (full) {
-                st16_f32(up, u);
-                st16_f32(ulo, l);
-              } else {
-#pragma unroll
-                for (int j = 0; j < 16; ++j)
-                  if (coord0 + j < ep.Db) {
-                    up[j] = u[j];
-                    ulo[j] = l[j];
-                  }
-              }
-            }
-          }
-          if (is_cpl && rvalid && ep.row_acc != nullptr)
-            row_accumulate(ep, row, nt * 2 + half, mode == EPI_COUPLING_INV ? -lsum : lsum);
-        } else {   // base density
-          float lsum = 0.f;
-          const float* ev_loc = ev + TC_EPI_COLS;
-          const float* ev_isc = ev + 2 * TC_EPI_COLS;
-          for (int c = half * 16; c < width; c += 32) {
-            float v[16];
-            tmem_ld16(t_base + c, v);
-            tmem_ld_wait();
-            if (rvalid) {
-#pragma unroll
-              for (int j = 0; j < 16; ++j) {
-                const float z = v[j] + ev[c + j];
-                if (ep.out != nullptr && n0 + c + j < args.n_valid)
-                  reinterpret_cast<float*>(ep.out)[row * ep.ldo + n0 + c + j] = z;
-                const float d = (z - ev_loc[c + j]) * ev_isc[c + j];
-                lsum += (mode == EPI_BASE_NORMAL) ? -0.5f * d * d : -fabsf(d);
-              }
-            }
-          }
-          if (rvalid && ep.row_acc != nullptr && ep.loc != nullptr) row_accumulate(ep, row, nt * 2 + half, lsum);
-        }
-        tc_fence_before();
-        __syncwarp();
-        if (lane == 0) {
-          if (cta_rank == 0) mbar_arrive(tempty_bar(a));
-          else mbar_arrive_cluster(tempty_bar(a), 0);
-        }
-      }
-      a ^= 1;
-      if (a == 0) aph ^= 1u;
-    }
-  }
-
-  tc_fence_before();
-  cluster_sync_all();
-  if (warp == 1) {
-    tc_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(TC_TMEM_COLS) : "memory");
-  }
-}
-
-// ================================================================================================
-// bf16x2 GEMM: fp32-grade accuracy at the bf16 tensor-core rate / 3 (twice the 3xTF32 rate, half its operand bytes).
-// Every operand is a pair of bf16 values hi + lo, hi = bf16(v), lo = bf16(v - hi): 16 mantissa bits together.
-//     a w ~= a_hi w_hi + a_hi w_lo + a_lo w_hi           (the dropped a_lo w_lo term is ~2^-16 relative)
-// three tcgen05.mma.kind::f16 per K=16 step into one fp32 TMEM accumulator; same CTA-pair pipeline as the 3xTF32 kernel
-// (a stage = [A_hi | A_lo | W_hi | W_lo] of one 64-column k-block); epilogues write (hi, lo) bf16 pairs for the next GEMM.
-// ================================================================================================
-struct Tcb2Args {
-  int64_t M, N, K;
-  int bn, n_tiles, m_tiles, n_valid, stages;
-  uint32_t stage_bytes, w_bytes;
-  uint32_t backoff_ns;
-  EpiParams ep;
-  uint16_t* out_lo;   // EPI_BIAS*: low part of the bf16 output (same leading dimension as ep.out); NULL: fp32 output
-  uint16_t* ub_lo;    // coupling modes: low part of the transformed columns
-};
-
 // (a, b) -> packed bf16x2 of the high parts and of the low parts
 __device__ __forceinline__ void split_bf16x2_pair(float a, float b, uint32_t& hi, uint32_t& lo) {
   const __nv_bfloat16 ha = __float2bfloat16_rn(a), hb = __float2bfloat16_rn(b);
@@ -1587,9 +1056,117 @@ __device__ __forceinline__ void split_bf16x2_pair(float a, float b, uint32_t& hi
   lo = pack_bf16x2(a - __bfloat162float(ha), b - __bfloat162float(hb));
 }
 
-__global__ void __launch_bounds__(TC_THREADS, 1)
-usf_tcb2_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmAlo,
-                    const __grid_constant__ CUtensorMap tmW, const __grid_constant__ CUtensorMap tmWlo, Tcb2Args args) {
+// Operand formats of split_gemm.  Each gives the element type T, the k-block and MMA-step widths, the three MMAs of one
+// step, and the epilogue's 16-value row accesses: load16 reads hi + lo, store16 splits v into (hi, lo) and writes both.
+// Both take `full` (one vector access per array) or else touch only the first n values; out_full / ub_full are the
+// format's conditions for a full chunk of the bias output and of the coupling's transformed columns.
+struct Tf32x3 {
+  using T = float;
+  static constexpr int BK = 32, UMMA_K = 8;
+  __device__ static uint32_t idesc(uint32_t n) { return make_idesc_tf32(n, 2 * TC_BM); }
+  __device__ static void mma3(uint32_t d, uint64_t ah, uint64_t al, uint64_t wh, uint64_t wl, uint32_t idesc, uint32_t acc) {
+    umma_tf32_2sm(d, ah, wh, idesc, acc);
+    umma_tf32_2sm(d, ah, wl, idesc, 1u);
+    umma_tf32_2sm(d, al, wh, idesc, 1u);
+  }
+  __device__ static bool out_full(const float* hi, int n) { return n >= 16 && (reinterpret_cast<uintptr_t>(hi) & 15) == 0; }
+  // 64 contiguous bytes of the row per array: two 256-bit loads each, which need 32-byte alignment
+  __device__ static bool ub_full(const float* hi, int n) { return n >= 16 && (reinterpret_cast<uintptr_t>(hi) & 31) == 0; }
+  __device__ static void load16(const float* hi, const float* lo, bool full, int n, float (&u)[16]) {
+    if (full) {
+      uint4 q[4], ql[4];
+      ld_global_256(hi, q[0], q[1]);
+      ld_global_256(hi + 8, q[2], q[3]);
+      ld_global_256(lo, ql[0], ql[1]);
+      ld_global_256(lo + 8, ql[2], ql[3]);
+#pragma unroll
+      for (int i = 0; i < 4; ++i) {
+        u[4 * i] = __uint_as_float(q[i].x) + __uint_as_float(ql[i].x);
+        u[4 * i + 1] = __uint_as_float(q[i].y) + __uint_as_float(ql[i].y);
+        u[4 * i + 2] = __uint_as_float(q[i].z) + __uint_as_float(ql[i].z);
+        u[4 * i + 3] = __uint_as_float(q[i].w) + __uint_as_float(ql[i].w);
+      }
+    } else {
+#pragma unroll
+      for (int j = 0; j < 16; ++j) u[j] = j < n ? hi[j] + lo[j] : 0.f;
+    }
+  }
+  __device__ static void store16(float* hi, float* lo, bool full, int n, float (&v)[16]) {
+    float l[16];
+#pragma unroll
+    for (int j = 0; j < 16; ++j) {
+      const float h = tf32_hi(v[j]);
+      l[j] = v[j] - h;
+      v[j] = h;
+    }
+    if (full) {
+      st16_f32(hi, v);
+      st16_f32(lo, l);
+    } else {
+#pragma unroll
+      for (int j = 0; j < 16; ++j)
+        if (j < n) {
+          hi[j] = v[j];
+          lo[j] = l[j];
+        }
+    }
+  }
+};
+
+struct Bf16x2 {
+  using T = uint16_t;
+  static constexpr int BK = TC_BK, UMMA_K = TC_UMMA_K;
+  __device__ static uint32_t idesc(uint32_t n) { return make_idesc(n, 2 * TC_BM); }
+  __device__ static void mma3(uint32_t d, uint64_t ah, uint64_t al, uint64_t wh, uint64_t wl, uint32_t idesc, uint32_t acc) {
+    umma_bf16_2sm(d, ah, wh, idesc, acc);
+    umma_bf16_2sm(d, ah, wl, idesc, 1u);
+    umma_bf16_2sm(d, al, wh, idesc, 1u);
+  }
+  // the (hi, lo) outputs are activation rows padded to the N tile: every chunk is stored whole
+  __device__ static bool out_full(const uint16_t*, int) { return true; }
+  // 16 coordinates = 32 bytes of the row per array: one 256-bit load each
+  __device__ static bool ub_full(const uint16_t*, int n) { return n >= 16; }
+  __device__ static void load16(const uint16_t* hi, const uint16_t* lo, bool full, int n, float (&u)[16]) {
+    if (full) {
+      uint4 q0, q1, l0, l1;
+      float uh[16], ul[16];
+      ld_global_256(hi, q0, q1);
+      ld_global_256(lo, l0, l1);
+      unpack_bf16x8(q0, uh);
+      unpack_bf16x8(q1, uh + 8);
+      unpack_bf16x8(l0, ul);
+      unpack_bf16x8(l1, ul + 8);
+#pragma unroll
+      for (int j = 0; j < 16; ++j) u[j] = uh[j] + ul[j];
+    } else {
+#pragma unroll
+      for (int j = 0; j < 16; ++j)
+        u[j] = j < n ? __uint_as_float((uint32_t)hi[j] << 16) + __uint_as_float((uint32_t)lo[j] << 16) : 0.f;
+    }
+  }
+  __device__ static void store16(uint16_t* hi, uint16_t* lo, bool full, int n, float (&v)[16]) {
+    if (full) {
+      uint32_t ph[8], pl[8];
+#pragma unroll
+      for (int j = 0; j < 8; ++j) split_bf16x2_pair(v[2 * j], v[2 * j + 1], ph[j], pl[j]);
+      st_global_256(hi, make_uint4(ph[0], ph[1], ph[2], ph[3]), make_uint4(ph[4], ph[5], ph[6], ph[7]));
+      st_global_256(lo, make_uint4(pl[0], pl[1], pl[2], pl[3]), make_uint4(pl[4], pl[5], pl[6], pl[7]));
+    } else {
+#pragma unroll
+      for (int j = 0; j < 16; ++j)
+        if (j < n) {
+          const __nv_bfloat16 h = __float2bfloat16_rn(v[j]);
+          hi[j] = __bfloat16_as_ushort(h);
+          lo[j] = __bfloat16_as_ushort(__float2bfloat16_rn(v[j] - __bfloat162float(h)));
+        }
+    }
+  }
+};
+
+template <class F>
+__device__ __forceinline__ void split_gemm(const CUtensorMap& tmA, const CUtensorMap& tmAlo, const CUtensorMap& tmW,
+                                           const CUtensorMap& tmWlo, const SplitArgs<typename F::T>& args) {
+  using T = typename F::T;
   const int STAGES = args.stages;
   const uint32_t STAGE_BYTES = args.stage_bytes;
   extern __shared__ uint8_t smem_raw[];
@@ -1629,7 +1206,7 @@ usf_tcb2_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_const
   asm volatile("griddepcontrol.wait;" ::: "memory");
 
   const int total_tiles = args.m_tiles * args.n_tiles;
-  const int num_kb = (int)((args.K + TC_BK - 1) / TC_BK);
+  const int num_kb = (int)((args.K + F::BK - 1) / F::BK);
   const uint32_t w_rows_bytes = (uint32_t)(args.bn >> 1) * 128u;
   const uint32_t stage_tx = 2u * (2u * TC_A_BYTES + 2u * w_rows_bytes);
   const uint32_t off_alo = TC_A_BYTES, off_w = 2u * TC_A_BYTES, off_wlo = 2u * TC_A_BYTES + args.w_bytes;
@@ -1645,15 +1222,15 @@ usf_tcb2_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_const
       const int w_row = nt * args.bn + (int)cta_rank * (width >> 1);
       const int a_row = (mt * 2 + (int)cta_rank) * TC_BM;
       for (int kb = 0; kb < num_kb; ++kb) {
-        ok = mbar_wait(empty_bar(s), ph ^ 1u, args.backoff_ns);
+        ok = mbar_wait(empty_bar(s), ph ^ 1u);
         if (!ok) break;
         const uint32_t dst = smem_base + s * STAGE_BYTES;
         if (elect_one()) {
           if (cta_rank == 0) mbar_expect_tx(full_bar(s), stage_tx);
-          tma_load_2d_2sm(dst, &tmA, full_bar(s), kb * TC_BK, a_row);
-          tma_load_2d_2sm(dst + off_alo, &tmAlo, full_bar(s), kb * TC_BK, a_row);
-          tma_load_2d_2sm(dst + off_w, &tmW, full_bar(s), kb * TC_BK, w_row);
-          tma_load_2d_2sm(dst + off_wlo, &tmWlo, full_bar(s), kb * TC_BK, w_row);
+          tma_load_2d_2sm(dst, &tmA, full_bar(s), kb * F::BK, a_row);
+          tma_load_2d_2sm(dst + off_alo, &tmAlo, full_bar(s), kb * F::BK, a_row);
+          tma_load_2d_2sm(dst + off_w, &tmW, full_bar(s), kb * F::BK, w_row);
+          tma_load_2d_2sm(dst + off_wlo, &tmWlo, full_bar(s), kb * F::BK, w_row);
         }
         if (++s == STAGES) { s = 0; ph ^= 1u; }
       }
@@ -1663,14 +1240,14 @@ usf_tcb2_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_const
       int s = 0, a = 0;
       uint32_t ph = 0, aph = 0;
       bool ok = true;
-      const int tail_steps = ((int)args.K - (num_kb - 1) * TC_BK + TC_UMMA_K - 1) / TC_UMMA_K;
+      const int tail_steps = ((int)args.K - (num_kb - 1) * F::BK + F::UMMA_K - 1) / F::UMMA_K;
       const uint64_t desc_hi = make_smem_desc(0);
       const uint32_t lo0 = (smem_base & 0x3FFFFu) >> 4, stage16 = STAGE_BYTES >> 4;
       for (int t = unit; t < total_tiles && ok; t += num_units) {
         const int nt = t % args.n_tiles;
         int width = (int)(args.N - (int64_t)nt * args.bn);
         if (width > args.bn) width = args.bn;
-        const uint32_t idesc = make_idesc((uint32_t)width, 2 * TC_BM);
+        const uint32_t idesc = F::idesc((uint32_t)width);
         ok = mbar_wait(tempty_bar(a), aph ^ 1u);
         if (!ok) break;
         tc_fence_after();
@@ -1679,14 +1256,12 @@ usf_tcb2_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_const
           ok = mbar_wait(full_bar(s), ph);
           if (!ok) break;
           if (elect_one()) {
+            // one MMA step is 32 bytes of the 128-byte swizzle row: the descriptors advance by 2 x 16-byte units
             const uint64_t ah = desc_hi | (uint64_t)(lo0 + (uint32_t)s * stage16);
             const uint64_t al = ah + (off_alo >> 4), wh = ah + (off_w >> 4), wl = ah + (off_wlo >> 4);
-            const int ksteps = kb + 1 < num_kb ? TC_BK / TC_UMMA_K : tail_steps;
-            for (int k = 0; k < ksteps; ++k) {
-              umma_bf16_2sm(d_tmem, ah + 2u * k, wh + 2u * k, idesc, (kb | k) != 0 ? 1u : 0u);
-              umma_bf16_2sm(d_tmem, ah + 2u * k, wl + 2u * k, idesc, 1u);
-              umma_bf16_2sm(d_tmem, al + 2u * k, wh + 2u * k, idesc, 1u);
-            }
+            const int ksteps = kb + 1 < num_kb ? F::BK / F::UMMA_K : tail_steps;
+            for (int k = 0; k < ksteps; ++k)
+              F::mma3(d_tmem, ah + 2u * k, al + 2u * k, wh + 2u * k, wl + 2u * k, idesc, (kb | k) != 0 ? 1u : 0u);
             umma_commit_2sm(empty_bar(s));
           }
           if (++s == STAGES) { s = 0; ph ^= 1u; }
@@ -1727,7 +1302,7 @@ usf_tcb2_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_const
       int width = (int)(args.N - n0);
       if (width > args.bn) width = args.bn;
       const float* ev = epi + n0;
-      const bool ok = mbar_wait(tfull_bar(a), aph, args.backoff_ns);
+      const bool ok = mbar_wait(tfull_bar(a), aph);
       if (ok) {
         tc_fence_after();
         const uint32_t t_base = tmem_base + ((uint32_t)(lane_grp * 32) << 16) + (uint32_t)a * TC_MAX_BN;
@@ -1742,23 +1317,20 @@ usf_tcb2_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_const
                 v[j] += ev[c + j];
                 if (mode == EPI_BIAS_RELU) v[j] = fmaxf(v[j], 0.f);
               }
+              const int64_t off = row * ep.ldo + n0 + c;
+              const int n = args.n_valid - (int)(n0 + c);   // valid columns of this chunk
               if (args.out_lo != nullptr) {
-                // the output travels as a (hi, lo) pair of bf16 rows, hi + lo = v to 16 mantissa bits: the next GEMM's A
-                uint16_t* dh = reinterpret_cast<uint16_t*>(ep.out) + row * ep.ldo + n0 + c;
-                uint16_t* dl = args.out_lo + row * ep.ldo + n0 + c;
-                uint32_t ph[8], pl[8];
-#pragma unroll
-                for (int j = 0; j < 8; ++j) split_bf16x2_pair(v[2 * j], v[2 * j + 1], ph[j], pl[j]);
-                st_global_256(dh, make_uint4(ph[0], ph[1], ph[2], ph[3]), make_uint4(ph[4], ph[5], ph[6], ph[7]));
-                st_global_256(dl, make_uint4(pl[0], pl[1], pl[2], pl[3]), make_uint4(pl[4], pl[5], pl[6], pl[7]));
+                // the output travels as (hi, lo), hi + lo = v: the next GEMM's A
+                T* dh = reinterpret_cast<T*>(ep.out) + off;
+                F::store16(dh, args.out_lo + off, F::out_full(dh, n), n, v);
               } else {
-                float* dst = reinterpret_cast<float*>(ep.out) + row * ep.ldo + n0 + c;
-                if (n0 + c + 16 <= args.n_valid && (reinterpret_cast<uintptr_t>(dst) & 15) == 0) {
+                float* dst = reinterpret_cast<float*>(ep.out) + off;
+                if (n >= 16 && (reinterpret_cast<uintptr_t>(dst) & 15) == 0) {
                   st16_f32(dst, v);
                 } else {
 #pragma unroll
                   for (int j = 0; j < 16; ++j)
-                    if (n0 + c + j < args.n_valid) dst[j] = v[j];
+                    if (j < n) dst[j] = v[j];
                 }
               }
             }
@@ -1777,27 +1349,13 @@ usf_tcb2_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_const
             tmem_ld_wait();
             const int coord0 = nt * C + c;
             if (rvalid && coord0 < ep.Db) {
-              uint16_t* up = reinterpret_cast<uint16_t*>(ep.ub) + row * ep.ldub + coord0;
-              uint16_t* ulo = args.ub_lo + row * ep.ldub + coord0;
+              T* up = reinterpret_cast<T*>(ep.ub) + row * ep.ldub + coord0;
+              T* ulo = args.ub_lo + row * ep.ldub + coord0;
               const float* bt = is_cpl ? ev + C + c : ev + c;
-              const bool full = coord0 + 16 <= ep.Db;
+              const int n = ep.Db - coord0;   // valid coordinates of this chunk
+              const bool full = F::ub_full(up, n);
               float u[16];
-              if (full) {     // 16 coordinates = 32 bytes of this thread's row per array: one 256-bit load each; u = hi + lo
-                uint4 q0, q1, l0, l1;
-                float uh[16], ul[16];
-                ld_global_256(up, q0, q1);
-                ld_global_256(ulo, l0, l1);
-                unpack_bf16x8(q0, uh);
-                unpack_bf16x8(q1, uh + 8);
-                unpack_bf16x8(l0, ul);
-                unpack_bf16x8(l1, ul + 8);
-#pragma unroll
-                for (int j = 0; j < 16; ++j) u[j] = uh[j] + ul[j];
-              } else {
-#pragma unroll
-                for (int j = 0; j < 16; ++j)
-                  u[j] = coord0 + j < ep.Db ? __uint_as_float((uint32_t)up[j] << 16) + __uint_as_float((uint32_t)ulo[j] << 16) : 0.f;
-              }
+              F::load16(up, ulo, full, n, u);
 #pragma unroll
               for (int j = 0; j < 16; ++j) {
                 const float tt = tv[j] + bt[j];
@@ -1810,21 +1368,7 @@ usf_tcb2_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_const
                   u[j] = mode == EPI_ADD_INV ? u[j] - tt : u[j] + tt;
                 }
               }
-              if (full) {
-                uint32_t ph[8], pl[8];
-#pragma unroll
-                for (int j = 0; j < 8; ++j) split_bf16x2_pair(u[2 * j], u[2 * j + 1], ph[j], pl[j]);
-                st_global_256(up, make_uint4(ph[0], ph[1], ph[2], ph[3]), make_uint4(ph[4], ph[5], ph[6], ph[7]));
-                st_global_256(ulo, make_uint4(pl[0], pl[1], pl[2], pl[3]), make_uint4(pl[4], pl[5], pl[6], pl[7]));
-              } else {
-#pragma unroll
-                for (int j = 0; j < 16; ++j)
-                  if (coord0 + j < ep.Db) {
-                    const __nv_bfloat16 h = __float2bfloat16_rn(u[j]);
-                    up[j] = __bfloat16_as_ushort(h);
-                    ulo[j] = __bfloat16_as_ushort(__float2bfloat16_rn(u[j] - __bfloat162float(h)));
-                  }
-              }
+              F::store16(up, ulo, full, n, u);
             }
           }
           if (is_cpl && rvalid && ep.row_acc != nullptr)
@@ -1868,6 +1412,18 @@ usf_tcb2_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_const
     tc_fence_after();
     asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(TC_TMEM_COLS) : "memory");
   }
+}
+
+__global__ void __launch_bounds__(TC_THREADS, 1)
+usf_tc3_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmAlo,
+                    const __grid_constant__ CUtensorMap tmW, const __grid_constant__ CUtensorMap tmWlo, SplitArgs<float> args) {
+  split_gemm<Tf32x3>(tmA, tmAlo, tmW, tmWlo, args);
+}
+
+__global__ void __launch_bounds__(TC_THREADS, 1)
+usf_tcb2_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmAlo,
+                     const __grid_constant__ CUtensorMap tmW, const __grid_constant__ CUtensorMap tmWlo, SplitArgs<uint16_t> args) {
+  split_gemm<Bf16x2>(tmA, tmAlo, tmW, tmWlo, args);
 }
 
 // (hi, lo) split of a (rows x cols) fp32 matrix: hi = x rounded to tf32 (written to `hi`, which may alias x, or skipped
@@ -1959,41 +1515,36 @@ int make_tmap(CUtensorMap* tm, const void* base, int64_t rows, int64_t cols, int
 
 const char* const kTcGemmKernelName = "usf_tc_gemm_kernel";
 
-int g_trace_on = 0;   // 1: trace plain GEMM launches, 2: trace fused conditioner launches
-int g_tc_dbg = -1;    // debug ablation bits (see usf_tc_gemm_kernel); -1 = read USF_TC_DBG once
-
-// CTAs per MMA: 2 (CTA pairs, tcgen05 cta_group::2) unless USF_TC_CTA_GROUP=1 selects the single-CTA kernel.
-int tc_cta_group() {
-  static int cg = 0;
-  if (cg == 0) {
-    const char* e = getenv("USF_TC_CTA_GROUP");
-    cg = (e != nullptr && e[0] == '1') ? 1 : 2;
-  }
-  return cg;
-}
-
-// USF_TC_BACKOFF_NS: sleep between polls of the waits that are off the critical path (epilogue warps waiting for a
-// tile of MMAs, producers waiting for a ring slot).
-static uint32_t tc_backoff_ns() {
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("USF_TC_BACKOFF_NS"); v = e ? atoi(e) : 0; if (v < 0) v = 0; }
-  return (uint32_t)v;
-}
-
-// USF_TC_TMA_STORE=1: bf16 outputs of the plain GEMM through a shared-memory staging tile and TMA stores (UTMASTG).
-// Default off: measured on the affine GEMM of C2 (65536 x 784 x 784, profiles/r2/ab_tma_store.txt) 72.3 us against
-// 68.4 us with direct 256-bit stores -- the 48 KB staging tile costs two of the seven ring stages (5 stages alone:
-// 70.7 us) and the two block-wide barriers per tile the rest; the stores themselves were never the bound.
-static bool tc_tma_store() {
-  const char* e = getenv("USF_TC_TMA_STORE");      // read per launch: a test switches it within one process
-  return e != nullptr && e[0] == '1';
-}
-
 // USF_PDL=0 disables programmatic dependent launch of the tensor-core kernels.
 static bool tc_pdl() {
   static int v = -1;
   if (v < 0) { const char* e = getenv("USF_PDL"); v = (e != nullptr && e[0] == '0') ? 0 : 1; }
   return v == 1;
+}
+
+// Launch of a persistent CTA-pair kernel: one cluster of 2 CTAs per two SMs (at most one per work unit), with
+// programmatic dependent launch unless USF_PDL=0.
+template <class... Params, class... Args>
+static int launch_pairs(void (*kernel)(Params...), int64_t units, int threads, uint32_t smem_bytes, cudaStream_t stream,
+                        const Args&... args) {
+  int64_t pairs = num_sms() / 2;
+  if (pairs > units) pairs = units;
+  cudaLaunchConfig_t cfg{};
+  cfg.gridDim = dim3((unsigned)(2 * pairs));
+  cfg.blockDim = dim3(threads);
+  cfg.dynamicSmemBytes = smem_bytes;
+  cfg.stream = stream;
+  cudaLaunchAttribute attr[2];
+  attr[0].id = cudaLaunchAttributeClusterDimension;
+  attr[0].val.clusterDim.x = 2;
+  attr[0].val.clusterDim.y = 1;
+  attr[0].val.clusterDim.z = 1;
+  attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+  attr[1].val.programmaticStreamSerializationAllowed = 1;
+  cfg.attrs = attr;
+  cfg.numAttrs = tc_pdl() ? 2 : 1;
+  USF_CUDA(cudaLaunchKernelEx(&cfg, kernel, args...));
+  return USF_OK;
 }
 
 // Tile order of the next tensor-core launches on this thread.  A launch chain alternates it kernel by kernel
@@ -2034,18 +1585,15 @@ int tc_gemm(const uint16_t* A, int64_t lda, const uint16_t* W, int64_t ldw, int6
                       (ep.ldub % 16) == 0,
                   "tc_gemm: additive tile must be [t(C <= 128)] and the b-part 32-byte aligned");
 
-  const int cg = tc_cta_group();
   static bool attr_set = false;
   if (!attr_set) {
-    USF_CUDA(cudaFuncSetAttribute(usf_tc_gemm_kernel<1, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TC_SMEM_BYTES));
-    USF_CUDA(cudaFuncSetAttribute(usf_tc_gemm_kernel<2, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TC_SMEM_BYTES));
-    USF_CUDA(cudaFuncSetAttribute(usf_tc_gemm_kernel<2, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TC_SMEM_BYTES));
+    USF_CUDA(cudaFuncSetAttribute(usf_tc_gemm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TC_SMEM_BYTES));
     attr_set = true;
   }
   CUtensorMap tmA, tmW;
   int rc = make_tmap(&tmA, A, M, K, lda, TC_BM);
   if (rc) return rc;
-  rc = make_tmap(&tmW, W, N, K, ldw, bn / cg);
+  rc = make_tmap(&tmW, W, N, K, ldw, bn / 2);
   if (rc) return rc;
 
   TcArgs args;
@@ -2054,97 +1602,52 @@ int tc_gemm(const uint16_t* A, int64_t lda, const uint16_t* W, int64_t ldw, int6
   args.K = K;
   args.bn = bn;
   args.n_tiles = (int)ceil_div(N, bn);
-  args.m_tiles = (int)ceil_div(M, TC_BM * cg);
+  args.m_tiles = (int)ceil_div(M, 2 * TC_BM);
   args.n_valid = ep.n_valid > 0 ? ep.n_valid : (int)N;
   args.ep = ep;
   args.reverse = g_tile_reverse;
-  args.stage_bytes = TC_A_BYTES + (uint32_t)round_up((int64_t)(bn / cg) * TC_BK * 2, 1024);
-  // bf16 activations leave through a staging tile + TMA stores when the ring keeps >= 4 stages beside it (ring depth
-  // >= 4 is flat, profiles/r1_run9) and the output qualifies as a tensor map (USF_TC_TMA_STORE=0: direct 256-bit stores)
-  args.out_stage_bytes = 0;
-  CUtensorMap tmO;
-  memset(&tmO, 0, sizeof(tmO));
-  if ((ep.mode == EPI_BIAS || ep.mode == EPI_BIAS_RELU) && ep.out_bf16 && bn >= 64 && tc_tma_store() && cg == 2) {
-    const uint32_t want = (uint32_t)(bn / 64) * TC_A_BYTES;
-    if ((TC_SMEM_BYTES - TC_FIXED_BYTES - want) / args.stage_bytes >= 4) {
-      if (make_tmap(&tmO, ep.out, M, N, ep.ldo, TC_BM) == USF_OK) args.out_stage_bytes = want;
-    }
-  }
-  args.stages = (int)((TC_SMEM_BYTES - TC_FIXED_BYTES - args.out_stage_bytes) / args.stage_bytes);
+  args.stage_bytes = TC_A_BYTES + (uint32_t)round_up((int64_t)(bn / 2) * TC_BK * 2, 1024);
+  args.stages = (int)((TC_SMEM_BYTES - TC_FIXED_BYTES) / args.stage_bytes);
   if (args.stages > TC_MAX_STAGES) args.stages = TC_MAX_STAGES;
-  {
-    static int cap = -1;   // tuning knob: USF_TC_MAX_STAGES caps the ring depth
-    if (cap < 0) { const char* e = getenv("USF_TC_MAX_STAGES"); cap = e ? atoi(e) : TC_MAX_STAGES; }
-    if (cap >= 2 && args.stages > cap) args.stages = cap;
-  }
   if (args.stages < 2) { set_error("tc_gemm: tile does not fit in shared memory"); return USF_E_ARG; }
-  if (g_tc_dbg < 0) { const char* e = getenv("USF_TC_DBG"); g_tc_dbg = e ? atoi(e) : 0; }
-  args.dbg = g_tc_dbg;
-  args.backoff_ns = tc_backoff_ns();
-  args.trace = nullptr;
-  if (g_trace_on == 1) {
-    void* p = nullptr;
-    USF_CUDA(cudaGetSymbolAddress(&p, g_tc_trace));
-    USF_CUDA(cudaMemsetAsync(p, 0, sizeof(unsigned long long) * 2 * 3 * TC_TRACE_CAP * 2, stream));
-    args.trace = reinterpret_cast<unsigned long long*>(p);
-  }
-  const int64_t total = (int64_t)args.m_tiles * args.n_tiles;
-  if (cg == 1) {
-    int grid = num_sms();
-    if (grid > total) grid = (int)total;
-    usf_tc_gemm_kernel<1, false><<<grid, TC_THREADS, TC_SMEM_BYTES, stream>>>(tmA, tmW, tmO, args);
-    USF_LAUNCH_CHECK("usf_tc_gemm_kernel<1>");
-    return USF_OK;
-  }
-  int64_t pairs = num_sms() / 2;
-  if (pairs > total) pairs = total;
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = dim3((unsigned)(2 * pairs));
-  cfg.blockDim = dim3(TC_THREADS);
-  cfg.dynamicSmemBytes = TC_SMEM_BYTES;
-  cfg.stream = stream;
-  cudaLaunchAttribute attr[2];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = 2;
-  attr[0].val.clusterDim.y = 1;
-  attr[0].val.clusterDim.z = 1;
-  attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[1].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = tc_pdl() ? 2 : 1;
-  if (args.trace != nullptr || (args.dbg != 0 && !(args.dbg & 0x200))) USF_CUDA(cudaLaunchKernelEx(&cfg, usf_tc_gemm_kernel<2, true>, tmA, tmW, tmO, args));
-  else USF_CUDA(cudaLaunchKernelEx(&cfg, usf_tc_gemm_kernel<2, false>, tmA, tmW, tmO, args));
-  return USF_OK;
+  return launch_pairs(usf_tc_gemm_kernel, (int64_t)args.m_tiles * args.n_tiles, TC_THREADS, TC_SMEM_BYTES, stream, tmA, tmW,
+                      args);
 }
 
-
-// 3xTF32 GEMM launcher (see usf_tc3_gemm_kernel).  A, Alo: (M, lda) fp32; W, Wlo: (N, ldw) fp32; leading dimensions
-// multiples of 4 (16-byte pitches), N multiple of 16 and <= TC_EPI_COLS.
-int tc3_gemm(const float* A, const float* Alo, int64_t lda, const float* W, const float* Wlo, int64_t ldw, int64_t M,
-             int64_t N, int64_t K, int bn, const EpiParams& ep, float* out_lo, float* ub_lo, cudaStream_t stream) {
+// Split-operand GEMM launcher (see split_gemm): T = float runs 3xTF32 (usf_tc3_gemm_kernel), T = uint16_t bf16x2
+// (usf_tcb2_gemm_kernel).  A, Alo: (M, lda); W, Wlo: (N, ldw); leading dimensions of 16-byte pitches, N multiple of 16
+// and <= TC_EPI_COLS.
+template <class T>
+int tc_split_gemm(const T* A, const T* Alo, int64_t lda, const T* W, const T* Wlo, int64_t ldw, int64_t M, int64_t N,
+                  int64_t K, int bn, const EpiParams& ep, T* out_lo, T* ub_lo, cudaStream_t stream) {
+  constexpr bool t3 = std::is_same<T, float>::value;
+  void (*kernel)(CUtensorMap, CUtensorMap, CUtensorMap, CUtensorMap, SplitArgs<T>);
+  if constexpr (t3) kernel = usf_tc3_gemm_kernel;
+  else kernel = usf_tcb2_gemm_kernel;
   if (M <= 0 || N <= 0) return USF_OK;
-  USF_CHECK_ARG(A && Alo && W && Wlo, "tc3_gemm: null operand");
-  USF_CHECK_ARG((lda % 4) == 0 && (ldw % 4) == 0, "tc3_gemm: leading dimensions must be multiples of 4");
+  USF_CHECK_ARG(A && Alo && W && Wlo, "tc_split_gemm: null operand");
+  USF_CHECK_ARG((lda * sizeof(T)) % 16 == 0 && (ldw * sizeof(T)) % 16 == 0,
+                "tc_split_gemm: leading dimensions must be multiples of 16 bytes");
   USF_CHECK_ARG(((reinterpret_cast<uintptr_t>(A) | reinterpret_cast<uintptr_t>(Alo) | reinterpret_cast<uintptr_t>(W) |
-                  reinterpret_cast<uintptr_t>(Wlo)) & 15) == 0, "tc3_gemm: operands must be 16-byte aligned");
+                  reinterpret_cast<uintptr_t>(Wlo)) & 15) == 0, "tc_split_gemm: operands must be 16-byte aligned");
   USF_CHECK_ARG(bn >= 16 && bn <= TC_MAX_BN && (bn % 16) == 0 && (N % 16) == 0 && K > 0 && N <= TC_EPI_COLS,
-                "tc3_gemm: bad tile/shape (bn=%d N=%lld K=%lld)", bn, (long long)N, (long long)K);
+                "tc_split_gemm: bad tile/shape (bn=%d N=%lld K=%lld)", bn, (long long)N, (long long)K);
   const bool cpl = ep.mode == EPI_COUPLING_INV || ep.mode == EPI_COUPLING_FWD;
   const bool add = ep.mode == EPI_ADD_INV || ep.mode == EPI_ADD_FWD;
-  if (cpl) USF_CHECK_ARG(bn == 2 * ep.C && (N % bn) == 0 && ub_lo != nullptr && !ep.ub_bf16, "tc3_gemm: bad coupling tile");
-  if (add) USF_CHECK_ARG(bn == ep.C && (N % bn) == 0 && ub_lo != nullptr && !ep.ub_bf16, "tc3_gemm: bad additive tile");
+  if (cpl) USF_CHECK_ARG(bn == 2 * ep.C && (N % bn) == 0 && ub_lo != nullptr && !ep.ub_bf16 == t3, "tc_split_gemm: bad coupling tile");
+  if (add) USF_CHECK_ARG(bn == ep.C && (N % bn) == 0 && ub_lo != nullptr && !ep.ub_bf16 == t3, "tc_split_gemm: bad additive tile");
   static bool attr_set = false;
   if (!attr_set) {
-    USF_CUDA(cudaFuncSetAttribute(usf_tc3_gemm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TC_SMEM_BYTES));
+    USF_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TC_SMEM_BYTES));
     attr_set = true;
   }
   CUtensorMap tmA, tmAlo, tmW, tmWlo;
-  int rc = make_tmap(&tmA, A, M, K, lda, TC_BM, 4);
-  if (!rc) rc = make_tmap(&tmAlo, Alo, M, K, lda, TC_BM, 4);
-  if (!rc) rc = make_tmap(&tmW, W, N, K, ldw, bn / 2, 4);
-  if (!rc) rc = make_tmap(&tmWlo, Wlo, N, K, ldw, bn / 2, 4);
+  int rc = make_tmap(&tmA, A, M, K, lda, TC_BM, sizeof(T));
+  if (!rc) rc = make_tmap(&tmAlo, Alo, M, K, lda, TC_BM, sizeof(T));
+  if (!rc) rc = make_tmap(&tmW, W, N, K, ldw, bn / 2, sizeof(T));
+  if (!rc) rc = make_tmap(&tmWlo, Wlo, N, K, ldw, bn / 2, sizeof(T));
   if (rc) return rc;
-  Tc3Args args;
+  SplitArgs<T> args;
   memset(&args, 0, sizeof(args));
   args.M = M; args.N = N; args.K = K; args.bn = bn;
   args.n_tiles = (int)ceil_div(N, bn);
@@ -2157,90 +1660,14 @@ int tc3_gemm(const float* A, const float* Alo, int64_t lda, const float* W, cons
   args.stage_bytes = 2u * TC_A_BYTES + 2u * args.w_bytes;
   args.stages = (int)((TC_SMEM_BYTES - TC_FIXED_BYTES) / args.stage_bytes);
   if (args.stages > TC_MAX_STAGES) args.stages = TC_MAX_STAGES;
-  if (args.stages < 2) { set_error("tc3_gemm: tile does not fit in shared memory"); return USF_E_ARG; }
-  args.backoff_ns = tc_backoff_ns();
-  const int64_t total = (int64_t)args.m_tiles * args.n_tiles;
-  int64_t pairs = num_sms() / 2;
-  if (pairs > total) pairs = total;
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = dim3((unsigned)(2 * pairs));
-  cfg.blockDim = dim3(TC_THREADS);
-  cfg.dynamicSmemBytes = TC_SMEM_BYTES;
-  cfg.stream = stream;
-  cudaLaunchAttribute attr[2];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = 2;
-  attr[0].val.clusterDim.y = 1;
-  attr[0].val.clusterDim.z = 1;
-  attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[1].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = tc_pdl() ? 2 : 1;
-  USF_CUDA(cudaLaunchKernelEx(&cfg, usf_tc3_gemm_kernel, tmA, tmAlo, tmW, tmWlo, args));
-  return USF_OK;
+  if (args.stages < 2) { set_error("tc_split_gemm: tile does not fit in shared memory"); return USF_E_ARG; }
+  return launch_pairs(kernel, (int64_t)args.m_tiles * args.n_tiles, TC_THREADS, TC_SMEM_BYTES, stream, tmA, tmAlo, tmW,
+                      tmWlo, args);
 }
-
-// bf16x2 GEMM launcher (see usf_tcb2_gemm_kernel).  A, Alo: (M, lda) bf16; W, Wlo: (N, ldw) bf16; leading dimensions
-// multiples of 8 (16-byte pitches), N multiple of 16 and <= TC_EPI_COLS.
-int tcb2_gemm(const uint16_t* A, const uint16_t* Alo, int64_t lda, const uint16_t* W, const uint16_t* Wlo, int64_t ldw, int64_t M,
-              int64_t N, int64_t K, int bn, const EpiParams& ep, uint16_t* out_lo, uint16_t* ub_lo, cudaStream_t stream) {
-  if (M <= 0 || N <= 0) return USF_OK;
-  USF_CHECK_ARG(A && Alo && W && Wlo, "tcb2_gemm: null operand");
-  USF_CHECK_ARG((lda % 8) == 0 && (ldw % 8) == 0, "tcb2_gemm: leading dimensions must be multiples of 8");
-  USF_CHECK_ARG(((reinterpret_cast<uintptr_t>(A) | reinterpret_cast<uintptr_t>(Alo) | reinterpret_cast<uintptr_t>(W) |
-                  reinterpret_cast<uintptr_t>(Wlo)) & 15) == 0, "tcb2_gemm: operands must be 16-byte aligned");
-  USF_CHECK_ARG(bn >= 16 && bn <= TC_MAX_BN && (bn % 16) == 0 && (N % 16) == 0 && K > 0 && N <= TC_EPI_COLS,
-                "tcb2_gemm: bad tile/shape (bn=%d N=%lld K=%lld)", bn, (long long)N, (long long)K);
-  const bool cpl = ep.mode == EPI_COUPLING_INV || ep.mode == EPI_COUPLING_FWD;
-  const bool add = ep.mode == EPI_ADD_INV || ep.mode == EPI_ADD_FWD;
-  if (cpl) USF_CHECK_ARG(bn == 2 * ep.C && (N % bn) == 0 && ub_lo != nullptr && ep.ub_bf16, "tcb2_gemm: bad coupling tile");
-  if (add) USF_CHECK_ARG(bn == ep.C && (N % bn) == 0 && ub_lo != nullptr && ep.ub_bf16, "tcb2_gemm: bad additive tile");
-  static bool attr_set = false;
-  if (!attr_set) {
-    USF_CUDA(cudaFuncSetAttribute(usf_tcb2_gemm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TC_SMEM_BYTES));
-    attr_set = true;
-  }
-  CUtensorMap tmA, tmAlo, tmW, tmWlo;
-  int rc = make_tmap(&tmA, A, M, K, lda, TC_BM, 2);
-  if (!rc) rc = make_tmap(&tmAlo, Alo, M, K, lda, TC_BM, 2);
-  if (!rc) rc = make_tmap(&tmW, W, N, K, ldw, bn / 2, 2);
-  if (!rc) rc = make_tmap(&tmWlo, Wlo, N, K, ldw, bn / 2, 2);
-  if (rc) return rc;
-  Tcb2Args args;
-  memset(&args, 0, sizeof(args));
-  args.M = M; args.N = N; args.K = K; args.bn = bn;
-  args.n_tiles = (int)ceil_div(N, bn);
-  args.m_tiles = (int)ceil_div(M, 2 * TC_BM);
-  args.n_valid = ep.n_valid > 0 ? ep.n_valid : (int)N;
-  args.ep = ep;
-  args.out_lo = out_lo;
-  args.ub_lo = ub_lo;
-  args.w_bytes = (uint32_t)round_up((int64_t)(bn / 2) * 128, 1024);
-  args.stage_bytes = 2u * TC_A_BYTES + 2u * args.w_bytes;
-  args.stages = (int)((TC_SMEM_BYTES - TC_FIXED_BYTES) / args.stage_bytes);
-  if (args.stages > TC_MAX_STAGES) args.stages = TC_MAX_STAGES;
-  if (args.stages < 2) { set_error("tcb2_gemm: tile does not fit in shared memory"); return USF_E_ARG; }
-  args.backoff_ns = tc_backoff_ns();
-  const int64_t total = (int64_t)args.m_tiles * args.n_tiles;
-  int64_t pairs = num_sms() / 2;
-  if (pairs > total) pairs = total;
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = dim3((unsigned)(2 * pairs));
-  cfg.blockDim = dim3(TC_THREADS);
-  cfg.dynamicSmemBytes = TC_SMEM_BYTES;
-  cfg.stream = stream;
-  cudaLaunchAttribute attr[2];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = 2;
-  attr[0].val.clusterDim.y = 1;
-  attr[0].val.clusterDim.z = 1;
-  attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[1].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = tc_pdl() ? 2 : 1;
-  USF_CUDA(cudaLaunchKernelEx(&cfg, usf_tcb2_gemm_kernel, tmA, tmAlo, tmW, tmWlo, args));
-  return USF_OK;
-}
+template int tc_split_gemm<float>(const float*, const float*, int64_t, const float*, const float*, int64_t, int64_t,
+                                  int64_t, int64_t, int, const EpiParams&, float*, float*, cudaStream_t);
+template int tc_split_gemm<uint16_t>(const uint16_t*, const uint16_t*, int64_t, const uint16_t*, const uint16_t*, int64_t,
+                                     int64_t, int64_t, int64_t, int, const EpiParams&, uint16_t*, uint16_t*, cudaStream_t);
 
 // fp32 rows -> (hi, lo) bf16 pairs in the activation layout (pad columns zero), optional per-row accumulator seed.
 // HBM-bound (4 D bytes read, 4 ldy written per row): 8 columns per thread, 16-byte loads when the source row allows,
@@ -2295,7 +1722,7 @@ int launch_split_lo(const float* x, int64_t ldx, float* hi, float* lo, int64_t l
 // Fused conditioner chain + coupling (see usf_tc_mlp_coupling_kernel).  Returns USF_E_UNSUPPORTED when the shapes do
 // not fit the fused kernel (the caller then runs the layer-by-layer chain).
 bool tc_mlp_supported(int n_layers, const int* N, const int* K, int Da) {
-  if (tc_cta_group() != 2 || n_layers < 2 || n_layers > MLP_MAX_LAYERS) return false;
+  if (n_layers < 2 || n_layers > MLP_MAX_LAYERS) return false;
   if (K[0] != Da || Da <= 0) return false;
   int total_n = 0;
   for (int l = 0; l < n_layers; ++l) total_n += N[l];
@@ -2315,8 +1742,7 @@ int tc_mlp_coupling(const uint16_t* A, int64_t lda, int64_t M, int n_layers, con
   USF_CHECK_ARG((lda % 8) == 0 && (reinterpret_cast<uintptr_t>(A) & 15) == 0, "tc_mlp_coupling: bad activation layout");
   static bool attr_set = false;
   if (!attr_set) {
-    USF_CUDA(cudaFuncSetAttribute(usf_tc_mlp_coupling_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)MLP_SMEM_BYTES));
-    USF_CUDA(cudaFuncSetAttribute(usf_tc_mlp_coupling_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)MLP_SMEM_BYTES));
+    USF_CUDA(cudaFuncSetAttribute(usf_tc_mlp_coupling_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)MLP_SMEM_BYTES));
     attr_set = true;
   }
   MlpArgs args;
@@ -2352,46 +1778,7 @@ int tc_mlp_coupling(const uint16_t* A, int64_t lda, int64_t M, int n_layers, con
                   "tc_mlp_coupling: bad additive tile");
   args.ep = ep;
   args.reverse = g_tile_reverse;
-  args.backoff_ns = tc_backoff_ns();
-  args.trace = nullptr;
-  if (g_trace_on == 2) {
-    void* tp = nullptr;
-    USF_CUDA(cudaGetSymbolAddress(&tp, g_tc_trace));
-    USF_CUDA(cudaMemsetAsync(tp, 0, sizeof(unsigned long long) * 2 * 3 * TC_TRACE_CAP * 2, stream));
-    args.trace = reinterpret_cast<unsigned long long*>(tp);
-  }
-  int64_t pairs = num_sms() / 2;
-  if (pairs > args.m_tiles) pairs = args.m_tiles;
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = dim3((unsigned)(2 * pairs));
-  cfg.blockDim = dim3(MLP_THREADS);
-  cfg.dynamicSmemBytes = MLP_SMEM_BYTES;
-  cfg.stream = stream;
-  cudaLaunchAttribute attr[2];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = 2;
-  attr[0].val.clusterDim.y = 1;
-  attr[0].val.clusterDim.z = 1;
-  attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[1].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = tc_pdl() ? 2 : 1;
-  if (args.trace != nullptr) USF_CUDA(cudaLaunchKernelEx(&cfg, usf_tc_mlp_coupling_kernel<true>, tmA, maps, args));
-  else USF_CUDA(cudaLaunchKernelEx(&cfg, usf_tc_mlp_coupling_kernel<false>, tmA, maps, args));
-  return USF_OK;
-}
-
-// Debug: enable tracing for subsequent launches (on != 0) / read back the records of the LAST launch.
-int tc_trace_ctl(int on, unsigned long long* out, int max_records) {
-  g_trace_on = on & 0xFF;
-  if (out == nullptr) g_tc_dbg = (on >> 8) & 0x3FF;   // bits 8+: ablation switches for subsequent plain-GEMM launches
-  if (out != nullptr) {
-    const size_t n = (size_t)2 * 3 * TC_TRACE_CAP * 2;
-    const size_t want = (size_t)max_records * 2 < n ? (size_t)max_records * 2 : n;
-    cudaError_t e = cudaMemcpyFromSymbol(out, g_tc_trace, sizeof(unsigned long long) * want);
-    if (e != cudaSuccess) return cuda_fail(e, "cudaMemcpyFromSymbol(g_tc_trace)");
-  }
-  return USF_OK;
+  return launch_pairs(usf_tc_mlp_coupling_kernel, args.m_tiles, MLP_THREADS, MLP_SMEM_BYTES, stream, tmA, maps, args);
 }
 
 int tc_timeout_flag(int* out, int reset) {
