@@ -286,7 +286,8 @@ int usf_set_deterministic(int on);
 
 /* 1 if usf_stack_run serves this stack at this precision with ONE whole-stack kernel (small event shapes: D + ctx_dim
  * <= 64, every layer width <= 128, fp32 weights; rows stay in shared memory across all layers, deterministic row sums),
- * 0 if it runs the launch chain. */
+ * 0 if it runs the launch chain.  USF_SMALL_STACK=0 in the environment turns this path off (and that of
+ * usf_stack_log_prob_grad, usf_stack_grad_is_single_kernel). */
 int usf_stack_is_single_kernel(const usf_stack_desc* st, int precision);
 
 /* usf_stack_run (precision USF_PREC_BF16) on rows that are bf16 already: x_bf16:(B,D) with ldx in bf16 elements.  The bf16
@@ -313,18 +314,29 @@ typedef struct {
 } usf_stack_grad_desc;
 
 /* Workspace bytes usf_stack_log_prob_grad needs for up to B rows (0 on a bad descriptor).  Rows are processed in chunks
- * of at most 16384, so the size stops growing there. */
+ * of at most 16384, so the size stops growing there.  On the one-kernel path (usf_stack_grad_is_single_kernel) the size
+ * does not depend on B: 256 bytes, plus -- when the saved block output rows do not fit in shared memory -- those rows for
+ * two CTAs per SM (n_blocks x 64 rows each). */
 size_t usf_stack_grad_workspace_bytes(const usf_stack_desc* st, const usf_stack_grad_desc* gd, int64_t B, int precision);
 
 /* log p(x) (out_logprob, (B)) and g = d log p(x) / dx (out_grad, (B, D) with leading dimension ldg) of an inverse-direction
  * stack with a base density, x:(B, D + ctx_dim).  precision: USF_PREC_FP32 (SIMT chain) or USF_PREC_BF16X2.  A forward
  * chain that keeps every block's output row and hidden activations is followed by the reverse chain on the same GEMM
- * kernels.  No atomics touch the gradient (bit-identical run to run); out_logprob follows usf_set_deterministic as in
- * usf_stack_run and equals its result bit for bit in deterministic mode at the same precision on the launch chain.  The
- * context gradient is not formed.  gpu_launches (optional) receives the number of kernels enqueued. */
+ * kernels.  No atomics touch the gradient (bit-identical run to run, whatever the row count of the call); out_logprob
+ * follows usf_set_deterministic as in usf_stack_run and equals its result bit for bit in deterministic mode at the same
+ * precision on the launch chain.  At USF_PREC_FP32, a stack that usf_stack_grad_is_single_kernel accepts runs in ONE
+ * kernel instead: the whole-stack kernel of usf_stack_run followed, per tile of 64 rows, by the reverse pass; its
+ * out_logprob equals usf_stack_run's bit for bit in any mode (usf_stack_run takes the same kernel there).  The context
+ * gradient is not formed.  gpu_launches (optional) receives the number of kernels enqueued. */
 int usf_stack_log_prob_grad(const usf_stack_desc* st, const usf_stack_grad_desc* gd, const float* x, int64_t ldx, int64_t B,
                             float* out_logprob, float* out_grad, int64_t ldg, void* workspace, size_t workspace_bytes,
                             int precision, int* gpu_launches, usf_stream_t stream);
+
+/* 1 if usf_stack_log_prob_grad serves this stack at this precision with ONE kernel: the stacks usf_stack_is_single_kernel
+ * accepts, unless the gradient kernel's saved state and transposed staging exceed the 227 KB of shared memory of a block
+ * (for example 8 conditioner layers 128 wide) or a transposed pack does not have the layout described above; those keep
+ * the launch chain.  0 also on a bad descriptor. */
+int usf_stack_grad_is_single_kernel(const usf_stack_desc* st, const usf_stack_grad_desc* gd, int precision);
 
 /* HOST function (no CUDA call): dst[r, c] = bf16(src[r, c]), round-to-nearest-even, NaN -> 0x7FFF -- the bit pattern the
  * device conversion produces.  src/dst are host pointers (pinned or not), leading dimensions in elements; `threads`

@@ -94,6 +94,7 @@ _PROTOS = {
     "usf_stack_grad_workspace_bytes": (_sz, [C.POINTER(StackDesc), C.POINTER(StackGradDesc), _i64, _int]),
     "usf_stack_log_prob_grad": (_int, [C.POINTER(StackDesc), C.POINTER(StackGradDesc), _vp, _i64, _i64, _vp, _vp, _i64,
                                        _vp, _sz, _int, C.POINTER(_int), _vp]),
+    "usf_stack_grad_is_single_kernel": (_int, [C.POINTER(StackDesc), C.POINTER(StackGradDesc), _int]),
     "usf_profile_begin": (_int, [_int]),
     "usf_profile_end": (_int, [C.POINTER(_f32), C.POINTER(_int), C.POINTER(_int)]),
     "usf_debug_graph_stats": (_int, [C.POINTER(C.c_longlong), C.c_char_p, _int]),

@@ -146,6 +146,12 @@ int trsm_rows(const float* T, int64_t D, bool lower, bool unit, bool trans, cons
 bool small_stack_supported(const usf_stack_desc* st, int precision);
 int small_stack_run(const usf_stack_desc* st, const float* x, int64_t ldx, int64_t B, float* out_logprob, float* out_y,
                     int64_t ldy, float* out_ladj, cudaStream_t stream);
+// its gradient twin (usf_stack_log_prob_grad at fp32): log p and d log p / dx in one launch
+bool small_grad_supported(const usf_stack_desc* st, const usf_stack_grad_desc* gd, int precision);
+size_t small_grad_workspace_bytes(const usf_stack_desc* st, const usf_stack_grad_desc* gd);
+int small_grad_run(const usf_stack_desc* st, const usf_stack_grad_desc* gd, const float* x, int64_t ldx, int64_t B,
+                   float* out_logprob, float* out_grad, int64_t ldg, void* workspace, size_t workspace_bytes,
+                   cudaStream_t stream);
 
 // ---- small helpers launched by the stack runner ---------------------------------------------
 int launch_convert_rows(const float* x, int64_t ldx, uint16_t* y_bf16, float* y_f32, int64_t ldy,

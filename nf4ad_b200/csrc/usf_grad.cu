@@ -2,7 +2,8 @@
 // row and hidden activations kept in per-block slots, followed by the reverse (vector-Jacobian) chain on the same GEMM
 // kernels.  The reverse GEMMs are plain products with the transposed packed weights (usf_stack_grad_desc); the steps
 // between them -- base-density gradient, coupling VJP, ReLU gate, pass-through residual -- are small element-wise
-// kernels over the saved rows.  Nothing on the gradient is summed with atomics.
+// kernels over the saved rows.  Nothing on the gradient is summed with atomics.  Small event shapes at fp32 take the
+// one-kernel path of usf_small.cu instead (usf_small_stack_grad_kernel), as usf_stack_run takes usf_small_stack_kernel.
 #include <vector>
 
 #include "usf_common.cuh"
@@ -186,7 +187,14 @@ extern "C" size_t usf_stack_grad_workspace_bytes(const usf_stack_desc* st, const
   GradPlan p;
   const int64_t rows = B < kGradChunkRows ? (B > 0 ? B : 1) : kGradChunkRows;
   if (plan_grad(st, gd, rows, precision, &p) != USF_OK) return 0;
+  if (small_grad_supported(st, gd, precision)) return small_grad_workspace_bytes(st, gd);
   return p.total;
+}
+
+extern "C" int usf_stack_grad_is_single_kernel(const usf_stack_desc* st, const usf_stack_grad_desc* gd, int precision) {
+  GradPlan p;
+  if (plan_grad(st, gd, 1, precision, &p) != USF_OK) return 0;
+  return small_grad_supported(st, gd, precision) ? 1 : 0;
 }
 
 extern "C" int usf_stack_log_prob_grad(const usf_stack_desc* st, const usf_stack_grad_desc* gd, const float* x, int64_t ldx,
@@ -201,6 +209,12 @@ extern "C" int usf_stack_log_prob_grad(const usf_stack_desc* st, const usf_stack
   const int64_t d_in = (int64_t)st->D + st->ctx_dim;
   USF_CHECK_ARG(ldx >= d_in && ldg >= st->D, "usf_stack_log_prob_grad: leading dimension too small");
   if (B == 0) return USF_OK;
+  if (small_grad_supported(st, gd, precision)) {
+    if ((rc = small_grad_run(st, gd, x, ldx, B, out_logprob, out_grad, ldg, workspace, workspace_bytes, as_stream(stream))))
+      return rc;
+    if (gpu_launches) *gpu_launches = 1;
+    return USF_OK;
+  }
   if (workspace == nullptr || workspace_bytes < p.total) {
     set_error("usf_stack_log_prob_grad: workspace too small (%zu < %zu bytes)", workspace_bytes, p.total);
     return USF_E_WORKSPACE;

@@ -354,6 +354,11 @@ class CompiledStack:
         """True when usf_stack_run serves this stack with the one whole-stack kernel (small event shapes)."""
         return bool(lib().usf_stack_is_single_kernel(C.byref(self.desc), self.precision))
 
+    @property
+    def grad_single_kernel(self):
+        """True when `run_grad` is served by the one-kernel gradient path (small event shapes at fp32)."""
+        return bool(lib().usf_stack_grad_is_single_kernel(C.byref(self.desc), C.byref(self.grad_desc), self.precision))
+
     def run(self, x, want_logprob=False, want_y=False, want_ladj=False, deterministic=False):
         """`deterministic`: per-row sums without atomics (usf_set_deterministic): bit-identical results run to run.
         x: (B, D) fp32 CUDA -- or bf16 rows for the bf16 tier (usf_stack_run_bf16in: bit-identical to fp32 rows that
@@ -417,7 +422,8 @@ class CompiledStack:
         return gd
 
     def run_grad(self, x, deterministic=False):
-        """log p(x) and d log p(x) / dx of rows x:(B, D + ctx_dim) on the reverse launch chain (`grad_desc`).
+        """log p(x) and d log p(x) / dx of rows x:(B, D + ctx_dim): one kernel where `grad_single_kernel`, else the
+        reverse launch chain (`grad_desc`).
         Returns (logprob (B,), grad (B, D) fp32, n_launches)."""
         _lib.require_cuda(x)
         if x.dim() != 2 or x.shape[1] != self.D + self.ctx_dim:
