@@ -16,7 +16,7 @@ CUDA tensors only -- a CPU tensor raises (`USFError`); the CPU restatement lives
 """
 import contextlib
 import os
-from typing import Any, Dict, List, Optional, Type
+from typing import Any, Dict, List, NamedTuple, Optional, Type
 
 import torch
 
@@ -90,6 +90,22 @@ def _default_precision():
     if p not in _REQUESTS:
         raise ValueError(f"USF_PRECISION must be one of {sorted(_REQUESTS)}, got {p!r}")
     return p
+
+
+class _TierDecision(NamedTuple):
+    """`Flow._tier_cache`: `want` resolved to `tier` on the weights `key`; not `calibrated`: answered without rows."""
+    key: tuple
+    want: str
+    tier: str
+    calibrated: bool
+    err: Optional[float]        # max-row error of the bf16 calibration, None where it did not run
+
+
+class _SmallDecision(NamedTuple):
+    """`Flow._small_cache`: does the one-kernel path take the stack on the weights `key`, and its widest layer."""
+    key: tuple
+    eligible: bool
+    widest: int
 
 
 class Flow(torch.nn.Module):
@@ -222,17 +238,19 @@ class Flow(torch.nn.Module):
             self._key_slots = None
         return super().train(mode)
 
-    # ---- which tier a grad-free call really runs ---------------------------------------------------------------
+    # ---- which tier a fused call really runs ---------------------------------------------------------------------
     # `precision = "bf16"` promises log_prob within 1e-2 of the fp64 result (BASELINE.json north star).  bf16 operands
     # hold that on the large trained-flow-like stacks (D >= 128: 1e-3 .. 6e-3) but not on every stack: the small ADBench /
     # GMM shapes (D < 128) and ill-conditioned untrained stacks amplify the 2^-9 operand rounding past it (4e-2 at D = 6).
     # So the tier is not taken on trust:
     #   * small event shapes (D + context <= 64, widths <= 128) run the ONE-kernel fp32 path (csrc/usf_small.cu) whatever
     #     tier was asked for -- those shapes are launch-latency bound, it is both the fastest and the most accurate form;
-    #   * other stacks with D < 128 run the 3xTF32 kernels (fp32-grade; the tensor-core rate does not matter there);
+    #   * other stacks with D < 128 run the FP32_GRADE_TC kernels (the tensor-core rate does not matter there);
     #   * for the rest the first scoring call after every weight change scores its first rows (<= 256) at both tiers and
     #     keeps bf16 only if the two agree within `BF16_CALIBRATION_TOL` on every row.
     # `effective_precision` reports the outcome; USF_BF16_CALIBRATE=0 / `bf16_trust` run the bf16 kernels regardless.
+    # `log_prob_and_grad` runs the tier `log_prob` runs on the same rows, "bf16" / "tf32x3" raised to "bf16x2", and never
+    # starts the calibration: it does not need to know whether bf16 would have held.
     BF16_CALIBRATION_TOL = 5e-3
     BF16_MIN_DIM = 128
     SMALL_MAX_DIM = 64
@@ -255,51 +273,64 @@ class Flow(torch.nn.Module):
             return False
         key = self._weights_key()
         hit = self.__dict__.get("_small_cache")
-        if hit is None or hit[0] != key:
+        if hit is None or hit.key != key:
             cs = self._stack(True, device, "fp32")
-            if cs is None or not cs.single_kernel:
-                hit = (key, False, 0)
-            else:
-                widest = 0
+            eligible, widest = cs is not None and cs.single_kernel, 0
+            if eligible:
                 for j in range(cs.desc.n_blocks):
                     blk = cs.blocks[j]
                     widest = max([widest, blk.G.N] + [blk.mlp[l].N for l in range(blk.n_mlp - 1)])
-                hit = (key, True, widest)
-            self.__dict__["_small_cache"] = hit
-        _, eligible, widest = hit
-        if not eligible:
+            hit = self.__dict__["_small_cache"] = _SmallDecision(key, eligible, widest)
+        if not hit.eligible:
             return False
-        return rows is None or self.SMALL_ALWAYS or rows <= self.SMALL_MAX_ROWS or widest <= 32
+        return rows is None or self.SMALL_ALWAYS or rows <= self.SMALL_MAX_ROWS or hit.widest <= 32
 
-    def _tier(self, x2=None, context_rows=None):
-        want = self.precision
-        if want == "auto":
-            want = self.FP32_GRADE_TC if self.event_dim >= self.BF16_MIN_DIM else "fp32"
-        if want == "fp32" or (want == "bf16" and self.__dict__.get("bf16_trust", False)) or \
-                (want == "bf16" and os.environ.get("USF_BF16_CALIBRATE", "1") == "0"):
-            self.effective_precision = want
-            return want
+    def _requested(self):
+        """`precision` with "auto" resolved: FP32_GRADE_TC from BF16_MIN_DIM coordinates on, "fp32" below."""
+        if self.precision != "auto":
+            return self.precision
+        return self.FP32_GRADE_TC if self.event_dim >= self.BF16_MIN_DIM else "fp32"
+
+    def _tier(self, x2=None, context=None, grad=False):
+        """The tier a fused call on the rows `x2` (None: the generative direction) runs, `context` as `_soft_context`
+        left it.  A grad-free call reports it in `effective_precision`.  `grad`: the tier of `log_prob_and_grad`."""
+        want = self._requested()
+        if want == "fp32" or (want == "bf16" and (self.__dict__.get("bf16_trust", False) or
+                                                  os.environ.get("USF_BF16_CALIBRATE", "1") == "0")):
+            tier = want
+        else:
+            device = x2.device if x2 is not None else next(self.parameters()).device
+            if self._small_ok(device, None if x2 is None else x2.shape[0]):     # (depends on the batch size: not cached)
+                tier = "fp32"
+            elif grad:
+                tier = want
+            else:
+                tier = self._calibrated_tier(want, x2, context, device)
+        if grad:
+            return "bf16x2" if tier in ("bf16", "tf32x3") else tier     # a bf16-operand gradient would be of little use
+        self.effective_precision = tier
+        return tier
+
+    def _calibrated_tier(self, want, x2, context, device):
+        """The tier a tensor-core request `want` runs on the current weights (the bf16 calibration), cached per weight
+        version in `_tier_cache`."""
         key = self._weights_key()
-        device = x2.device if x2 is not None else next(self.parameters()).device
-        if self._small_ok(device, None if x2 is None else x2.shape[0]):     # (depends on the batch size: not cached below)
-            self.effective_precision = "fp32"
-            return "fp32"
         hit = self.__dict__.get("_tier_cache")
-        if hit is not None and hit[0] == (key, want) and (hit[2] or x2 is None):
-            self.effective_precision = hit[1]
-            return hit[1]
+        if hit is not None and hit.key == key and hit.want == want and (hit.calibrated or x2 is None):
+            return hit.tier
         tier, calibrated, err = want, False, None
         if want in ("tf32x3", "bf16x2"):
             calibrated = True
         elif self.event_dim < self.BF16_MIN_DIM:
             tier, calibrated = self.FP32_GRADE_TC, True
         elif x2 is not None and x2.shape[0] > 0 and not self._needs_grad(x2):
-            rows = (x2 if context_rows is None else context_rows)[:256]
             lo = self._stack(True, device, "bf16")
             hi = self._stack(True, device, self.FP32_GRADE_TC) or self._stack(True, device, "fp32")
-            if lo is None or lo.desc.base_kind < 0 or hi is None:
+            rows = self._fused_input(x2, context)      # the rows log_prob runs
+            if lo is None or lo.desc.base_kind < 0 or hi is None or rows is None:
                 calibrated = True                      # no fused bf16 path at all / nothing to compare with
             else:
+                rows = rows[:256]
                 a = lo.run(rows, want_logprob=True)[0].double()
                 b = hi.run(rows.float(), want_logprob=True)[0].double()
                 err = float(((a - b).abs() / b.abs().clamp_min(1.0)).nan_to_num(nan=float("inf")).max())
@@ -311,8 +342,7 @@ class Flow(torch.nn.Module):
         if tier in ("tf32x3", "bf16x2") and self._stack(True, device, tier) is None and \
                 self._stack(True, device, "fp32") is not None:
             tier = "fp32"                              # shapes the split-operand kernels do not take (N > 1024)
-        self.__dict__["_tier_cache"] = ((key, want), tier, calibrated, err)
-        self.effective_precision = tier
+        self.__dict__["_tier_cache"] = _TierDecision(key, want, tier, calibrated, err)
         self.bf16_calibration_err = err
         return tier
 
@@ -321,26 +351,18 @@ class Flow(torch.nn.Module):
         if self.precision == "fp32":
             return "fp32"
         hit = self.__dict__.get("_tier_cache")
-        return hit[1] if hit is not None and hit[2] and hit[0][0] == self._weights_key() else None
+        return hit.tier if hit is not None and hit.calibrated and hit.key == self._weights_key() else None
 
     def resolve_precision(self, x):
         """The tier grad-free calls on these weights run at ("bf16" may resolve to "tf32x3" / "fp32", see above);
         `x`: a few device rows to calibrate on when that has not happened since the last weight change."""
         x2, _ = self._prep(x)
-        ctx = self._soft_context(x2, None)
-        if self.context_dim() > 0 and ctx is not None:
-            xin = torch.cat([x2.float(), ctx.expand(x2.shape[0], self.context_dim())], dim=1)
-        else:
-            xin = None
-        return self._tier(x2, xin)
+        return self._tier(x2, self._soft_context(x2, None))
 
     def _stack(self, inverse, device, precision=None, grad=False):
         """Compiled (packed) stack for this direction / precision / weight version, or None.  `grad`: the same stack with
         the transposed matrices of the reverse chain built (`log_prob_and_grad`), or None where they cannot be."""
-        precision = precision or self.precision
-        if precision == "auto":
-            precision = self.FP32_GRADE_TC if self.event_dim >= self.BF16_MIN_DIM else "fp32"
-        prec = _PRECISIONS[precision]
+        prec = _PRECISIONS[self._requested() if precision in (None, "auto") else precision]
         slot = (bool(inverse), prec)
         key = (self._weights_key(), str(device))
         hit = self._compiled.get(slot)
@@ -384,33 +406,43 @@ class Flow(torch.nn.Module):
         ev = self.event_shape
         return rows if len(ev) == 1 else rows.reshape(rows.shape[0], *ev)
 
-    def _fused(self, x2, context, inverse):
-        """-> (compiled stack | None, input rows incl. context columns).  The fused launch chain serves the grad-free
-        calls of flat-event flows; a conditional flow carries its context as extra activation columns."""
-        if self._needs_grad(x2):
-            return None, x2
+    def _fused_input(self, x2, context):
+        """The input rows of the fused chain for the rows `x2` and a context as `_soft_context` left it: `x2` as given for
+        an unconditional flow (bf16 rows reach usf_stack_run_bf16in), else the fp32 rows with the context columns
+        appended (a conditional flow carries its context as extra activation columns).  None: a context handed to an
+        unconditional flow, whose conditioners are then evaluated as given, layer-wise."""
         cd = self.context_dim()
-        if cd == 0 and context is not None:
-            return None, x2                   # unconditional conditioners handed a context: evaluated as given, layer-wise
-        if cd > 0 and context is None:
+        if cd == 0:
+            return x2 if context is None else None
+        if context is None:
             raise ValueError("this flow's conditioners take a context (ConditionalDenseNN): pass `context=` or build the "
                              "flow with soft_training=True")
-        xin = x2
-        if cd > 0:
-            ctx = context if context.dim() == 2 else context.reshape(-1, cd)
-            xin = torch.cat([x2.to(torch.float32), ctx.to(torch.float32).expand(x2.shape[0], cd)], dim=1)
-        tier = self._tier(x2 if inverse else None, xin if inverse else None)
-        cs = self._stack(inverse, x2.device, tier)
-        if cs is None or cs.ctx_dim != cd:
-            return None, x2
-        return cs, xin
+        ctx = context if context.dim() == 2 else context.reshape(-1, cd)
+        return torch.cat([x2.to(torch.float32), ctx.to(torch.float32).expand(x2.shape[0], cd)], dim=1)
+
+    def _fused(self, x, context, inverse=True, grad=False):
+        """The prologue of the public calls: -> (rows (B, prod(event)), leading batch shape, context after
+        `_soft_context`, compiled stack | None, its input rows).  The stack serves the grad-free calls and, with `grad`,
+        `log_prob_and_grad` (its transposed matrices built; fp32 where the tier's cannot be).  None: the layer-wise pass
+        (autograd, image-shaped events -- `_stack` refuses them --, stacks the fused kernels do not take)."""
+        x2, lead = self._prep(x)
+        context = self._soft_context(x2, context)
+        cs = xin = None
+        if grad or not self._needs_grad(x2):
+            xin = self._fused_input(x2, context)
+        if xin is not None:
+            tier = self._tier(x2, context, grad) if inverse else self._tier()
+            cs = self._stack(inverse, x2.device, tier, grad)
+            if cs is None and grad and tier != "fp32":
+                cs = self._stack(True, x2.device, "fp32", grad=True)
+            if cs is not None and cs.ctx_dim != self.context_dim():
+                cs = None
+        return x2, lead, context, cs, xin
 
     # ------------------------------------------------------------------ density path
     @_on_device
     def log_prob(self, x, context=None):
-        x2, lead = self._prep(x)
-        context = self._soft_context(x2, context)
-        cs, xin = self._fused(x2, context, True)
+        x2, lead, context, cs, xin = self._fused(x, context)
         if cs is not None and cs.desc.base_kind >= 0:
             lp, _, _, n = cs.run(xin, want_logprob=True, deterministic=self.deterministic)
             self.last_launches = n
@@ -430,15 +462,15 @@ class Flow(torch.nn.Module):
         sign(0) = 0 for a Laplace base); builds no autograd graph, touches no `p.grad`, works under `torch.no_grad()`.
         The gradient is the per-feature attribution of the anomaly score -log p (the context gradient is not formed).
 
-        Flat-event stacks run the reverse launch chain of the fused path in one library call: at bf16x2 when the request
-        is "auto" with D >= BF16_MIN_DIM, or "bf16x2" / "bf16" / "tf32x3" (a gradient at bf16 operand precision would be
-        of little use), else on the fp32 SIMT kernels.  Other flows (image-shaped events, opaque conditioners, softplus
-        scales, a context handed to an unconditional flow) differentiate the layer-wise pass with autograd.
+        Flat-event stacks run the reverse launch chain of the fused path in one library call, at the tier `log_prob`
+        runs on these rows (`_tier`), with "bf16" / "tf32x3" raised to bf16x2 (a gradient at bf16 operand precision
+        would be of little use) and fp32 where the bf16x2 chain does not take the stack.  So a small stack that
+        `log_prob` scores in one kernel gets its gradient in one kernel too, and `lp` is `log_prob`'s (bit for bit in
+        deterministic mode).  Other flows (image-shaped events, opaque conditioners, softplus scales, a context handed to
+        an unconditional flow) differentiate the layer-wise pass with autograd.
         `last_grad_precision` reports which: "bf16x2", "fp32" or "autograd"."""
-        x2, lead = self._prep(x)
-        ctx = self._soft_context(x2, context)
-        cs, xin = self._grad_stack(x2, ctx)
-        if cs is None:
+        _, lead, _, cs, xin = self._fused(x, context, grad=True)
+        if cs is None or cs.desc.base_kind < 0:
             self.last_grad_precision = "autograd"
             with torch.enable_grad():
                 xr = x.detach().to(torch.float32).requires_grad_(True)
@@ -449,27 +481,6 @@ class Flow(torch.nn.Module):
         self.last_grad_precision = "bf16x2" if cs.precision == _lib.USF_PREC_BF16X2 else "fp32"
         self.last_launches = n
         return lp.reshape(lead), g.reshape(x.shape)
-
-    def _grad_stack(self, x2, context):
-        """-> (compiled stack with its transposed matrices | None, input rows incl. context columns) for
-        `log_prob_and_grad`, by the tier rule there."""
-        cd = self.context_dim()
-        if len(self.event_shape) != 1 or (cd == 0 and context is not None):
-            return None, x2
-        if cd > 0 and context is None:
-            raise ValueError("this flow's conditioners take a context (ConditionalDenseNN): pass `context=` or build the "
-                             "flow with soft_training=True")
-        xin = x2.to(torch.float32)
-        if cd > 0:
-            ctx = context if context.dim() == 2 else context.reshape(-1, cd)
-            xin = torch.cat([xin, ctx.to(torch.float32).expand(x2.shape[0], cd)], dim=1)
-        want = self.precision
-        tc = (want == "auto" and self.event_dim >= self.BF16_MIN_DIM) or want in ("bf16x2", "bf16", "tf32x3")
-        for tier in (("bf16x2", "fp32") if tc else ("fp32",)):
-            cs = self._stack(True, x2.device, tier, grad=True)
-            if cs is not None and cs.ctx_dim == cd and cs.desc.base_kind >= 0:
-                return cs, xin
-        return None, x2
 
     def _prefetch_lu_inverses(self, y):
         """Mixed-precision training: the dense inverses of all LU layers this pass will apply are independent of the
@@ -745,9 +756,7 @@ class Flow(torch.nn.Module):
     @_on_device
     def backward(self, x, context=None):
         """data -> latent."""
-        x2, lead = self._prep(x)
-        context = self._soft_context(x2, context)
-        cs, xin = self._fused(x2, context, True)
+        x2, lead, context, cs, xin = self._fused(x, context)
         if cs is not None:
             _, z, _, n = cs.run(xin, want_y=True)
             self.last_launches = n
@@ -757,9 +766,7 @@ class Flow(torch.nn.Module):
 
     @_on_device
     def latent_to_data(self, z, context=None):
-        z2, lead = self._prep(z)
-        context = self._soft_context(z2, context)
-        cs, zin = self._fused(z2, context, False)
+        z2, lead, context, cs, zin = self._fused(z, context, inverse=False)
         if cs is not None:
             _, x, _, n = cs.run(zin, want_y=True)
             self.last_launches = n

@@ -363,30 +363,49 @@ class CompiledStack:
         """`deterministic`: per-row sums without atomics (usf_set_deterministic): bit-identical results run to run.
         x: (B, D) fp32 CUDA -- or bf16 rows for the bf16 tier (usf_stack_run_bf16in: bit-identical to fp32 rows that
         round to them).  Returns (logprob | None, y | None, ladj | None, n_launches)."""
+        if want_logprob and self.desc.base_kind < 0:
+            raise _lib.USFError("this stack was compiled without a supported base distribution")
+        bf16_rows = x.dtype == torch.bfloat16 and self.precision == _lib.USF_PREC_BF16
+        return self._call("usf_stack_run_bf16in" if bf16_rows else "usf_stack_run", x, want_logprob, want_y, want_ladj,
+                          deterministic)
+
+    def _call(self, entry, x, want_lp, want_rows, want_ladj, deterministic):
+        """One library call of `entry` on the rows x:(B, D + ctx_dim), `deterministic` mode set for it: the fp32 outputs
+        it writes are a (B,) log p, (B, D) rows (y, or the gradient of usf_stack_log_prob_grad, which has no ladj) and a
+        (B,) ladj.  -> (lp | None, rows | None, ladj | None, n_launches)."""
+        grad = entry == "usf_stack_log_prob_grad"
+        bf16_rows = entry == "usf_stack_run_bf16in"
         _lib.require_cuda(x)
-        x_bf16 = x.dtype == torch.bfloat16 and self.precision == _lib.USF_PREC_BF16 and x.dim() == 2
         if x.dim() != 2 or x.shape[1] != self.D + self.ctx_dim:
             raise ValueError(f"expected rows of {self.D} coordinates (+ {self.ctx_dim} context columns), got shape {tuple(x.shape)}")
-        if x_bf16:
+        if bf16_rows:
             if x.stride(1) != 1 or (x.shape[0] > 1 and x.stride(0) < x.shape[1]):
                 x = x.contiguous()
             ldx = x.stride(0) if x.shape[0] > 1 else max(x.shape[1], 1)
         else:
             x, ldx = ops._rows(x)
-        B = x.shape[0]
-        dev = x.device
-        lp = torch.empty(B, device=dev, dtype=torch.float32) if want_logprob else None
-        y = torch.empty(B, self.D, device=dev, dtype=torch.float32) if want_y else None
+        B, dev = x.shape[0], x.device
+        lp = torch.empty(B, device=dev, dtype=torch.float32) if want_lp else None
+        rows = torch.empty(B, self.D, device=dev, dtype=torch.float32) if want_rows else None
         ladj = torch.empty(B, device=dev, dtype=torch.float32) if want_ladj else None
         if B == 0:
-            return lp, y, ladj, 0
-        if want_logprob and self.desc.base_kind < 0:
-            raise _lib.USFError("this stack was compiled without a supported base distribution")
-        prev = lib().usf_set_deterministic(int(bool(deterministic)))
+            return lp, rows, ladj, 0
+        descs = (C.byref(self.desc), C.byref(self.grad_desc)) if grad else (C.byref(self.desc),)
+        query = "usf_stack_grad_workspace_bytes" if grad else "usf_stack_workspace_bytes"
+        outs = (ptr(lp), ptr(rows), self.D) if grad else (ptr(lp), ptr(rows), self.D, ptr(ladj))
+        tier = () if bf16_rows else (self.precision,)          # (usf_stack_run_bf16in runs the bf16 tier)
+        L = lib()
+        prev = L.usf_set_deterministic(int(bool(deterministic)))
         try:
-            return self._run(x, x_bf16, ldx, B, lp, y, ladj)
+            nbytes = getattr(L, query)(*descs, B, self.precision)
+            if nbytes == 0:
+                raise _lib.USFError(f"{query} failed: " + L.usf_last_error().decode())
+            ws = torch.empty(nbytes, device=dev, dtype=torch.uint8)
+            n = C.c_int(0)
+            check(getattr(L, entry)(*descs, ptr(x), ldx, B, *outs, ptr(ws), nbytes, *tier, C.byref(n), stream()), entry)
         finally:
-            lib().usf_set_deterministic(prev)
+            L.usf_set_deterministic(prev)
+        return lp, rows, ladj, n.value
 
     @property
     def grad_desc(self):
@@ -425,40 +444,5 @@ class CompiledStack:
         """log p(x) and d log p(x) / dx of rows x:(B, D + ctx_dim): one kernel where `grad_single_kernel`, else the
         reverse launch chain (`grad_desc`).
         Returns (logprob (B,), grad (B, D) fp32, n_launches)."""
-        _lib.require_cuda(x)
-        if x.dim() != 2 or x.shape[1] != self.D + self.ctx_dim:
-            raise ValueError(f"expected rows of {self.D} coordinates (+ {self.ctx_dim} context columns), got shape {tuple(x.shape)}")
-        x, ldx = ops._rows(x)
-        B, dev = x.shape[0], x.device
-        lp = torch.empty(B, device=dev, dtype=torch.float32)
-        g = torch.empty(B, self.D, device=dev, dtype=torch.float32)
-        if B == 0:
-            return lp, g, 0
-        prev = lib().usf_set_deterministic(int(bool(deterministic)))
-        try:
-            nbytes = lib().usf_stack_grad_workspace_bytes(C.byref(self.desc), C.byref(self.grad_desc), B, self.precision)
-            if nbytes == 0:
-                raise _lib.USFError("usf_stack_grad_workspace_bytes failed: " + lib().usf_last_error().decode())
-            ws = torch.empty(nbytes, device=dev, dtype=torch.uint8)
-            n = C.c_int(0)
-            check(lib().usf_stack_log_prob_grad(C.byref(self.desc), C.byref(self.grad_desc), ptr(x), ldx, B, ptr(lp), ptr(g),
-                                                self.D, ptr(ws), nbytes, self.precision, C.byref(n), stream()),
-                  "usf_stack_log_prob_grad")
-        finally:
-            lib().usf_set_deterministic(prev)
-        return lp, g, n.value
-
-    def _run(self, x, x_bf16, ldx, B, lp, y, ladj):
-        dev = x.device
-        nbytes = lib().usf_stack_workspace_bytes(C.byref(self.desc), B, self.precision)
-        if nbytes == 0:
-            raise _lib.USFError("usf_stack_workspace_bytes failed: " + lib().usf_last_error().decode())
-        ws = torch.empty(nbytes, device=dev, dtype=torch.uint8)
-        n = C.c_int(0)
-        if x_bf16:
-            check(lib().usf_stack_run_bf16in(C.byref(self.desc), ptr(x), ldx, B, ptr(lp), ptr(y), self.D, ptr(ladj), ptr(ws),
-                                             nbytes, C.byref(n), stream()), "usf_stack_run_bf16in")
-        else:
-            check(lib().usf_stack_run(C.byref(self.desc), ptr(x), ldx, B, ptr(lp), ptr(y), self.D, ptr(ladj), ptr(ws),
-                                      nbytes, self.precision, C.byref(n), stream()), "usf_stack_run")
-        return lp, y, ladj, n.value
+        lp, g, _, n = self._call("usf_stack_log_prob_grad", x, True, True, False, deterministic)
+        return lp, g, n

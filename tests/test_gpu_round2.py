@@ -381,7 +381,7 @@ def test_small_stack_single_kernel(O, P, cfg):
     with torch.no_grad():
         big = torch.randn(70000, D, generator=g).cuda()
         lp = fp.log_prob(big)
-        big_tier = fp.effective_precision        # wide layers at this batch size go to the 3xTF32 chain (Flow._small_ok)
+        big_tier = fp.effective_precision        # wide layers at this batch size go to the FP32_GRADE_TC chain (Flow._small_ok)
         part = fp.log_prob(big[12345:12400].contiguous())
         if big_tier == "fp32":
             assert fp.last_launches == 1 and torch.equal(lp[12345:12400], part)

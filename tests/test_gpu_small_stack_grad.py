@@ -136,16 +136,20 @@ def test_query_is_fp32_only(K, O, P):
 # ------------------------------------------------------------------------------------------------------------------
 # Flow level
 # ------------------------------------------------------------------------------------------------------------------
-@pytest.mark.parametrize("name", ["C4-D6", "fixture-D32"])
-def test_flow_auto(O, P, name):
-    """Flow.log_prob_and_grad under "auto": one launch at fp32, lp torch.equal to the fused log_prob (no_grad: with
-    trainable parameters and grad mode on, log_prob differentiates the layer-wise pass instead), both within the bounds
-    of test_full_depth_against_oracle; ADBenchFlow.score_gradients is -g."""
+@pytest.mark.parametrize("name,precision", [
+    pytest.param(name, precision, id=name if precision == "auto" else f"{name}-{precision}")
+    for name in ("C4-D6", "fixture-D32") for precision in ("auto", "bf16x2", "bf16", "tf32x3")])
+def test_flow_auto(O, P, name, precision):
+    """Flow.log_prob_and_grad under every request log_prob serves with the one-kernel path: one launch at fp32, lp
+    torch.equal to the fused log_prob (no_grad: with trainable parameters and grad mode on, log_prob differentiates the
+    layer-wise pass instead) and one compiled stack for both, both within the bounds of test_full_depth_against_oracle;
+    ADBenchFlow.score_gradients is -g."""
     from test_gpu_log_prob_grad import FP32_TOL, GRAD_TOL, oracle_grad, rel, row_err
     from nf4ad_b200.adbench import ADBenchFlow
     case_flow(O, P, name)
     fo, fp = base._FLOWS[name]
-    fp.precision = "auto"
+    fp.invalidate_cache()
+    fp.precision = precision
     D = CASES[name][1]
     x = torch.randn(256, D, generator=torch.Generator().manual_seed(5))
     xc = x.cuda()
@@ -154,6 +158,7 @@ def test_flow_auto(O, P, name):
     with torch.no_grad():
         lq = fp.log_prob(xc)
     assert fp.last_launches == 1 and torch.equal(lp, lq)
+    assert len(fp._compiled) == 1, list(fp._compiled)
     lp_ref, g_ref, kink = oracle_grad(fo, x)
     e = row_err(g, g_ref)
     bad = e > GRAD_TOL
