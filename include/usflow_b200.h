@@ -2,7 +2,7 @@
  * usflow_b200.h -- C ABI of the B200-native USFlows density path.
  *
  * This is the drop-in boundary: a plain-C shared library (libusflow_b200.so,
- * sm_100a only) that the Python mirror of the USFlows module API
+ * sm_100a only, 54 entry points) that the Python mirror of the USFlows module API
  * (nf4ad_b200/, import names `src.usflows.*`) binds with ctypes.  There are no
  * torch types in any signature: raw device pointers, int64 sizes / leading
  * dimensions (in elements), a cudaStream_t passed as void*.
@@ -296,6 +296,25 @@ int usf_stack_is_single_kernel(const usf_stack_desc* st, int precision);
 int usf_stack_run_bf16in(const usf_stack_desc* st, const uint16_t* x_bf16, int64_t ldx, int64_t B, float* out_logprob,
                          float* out_y, int64_t ldy, float* out_ladj, void* workspace, size_t workspace_bytes,
                          int* gpu_launches, usf_stream_t stream);
+
+/* ---- the terms of log p: what the base density and each coupling contribute, from the same pass ---------------------
+ * log p(x) = const_term + sum_j t_j(x) + b(x) for an inverse-direction stack with a base density: t_j is block j's
+ * coupling log-det term (-sum clamp tanh(s); 0 for an additive block), b the data-dependent part of the base log-density
+ * (Normal: sum -((z - loc) / scale)^2 / 2; Laplace: sum -|z - loc| / scale).  usf_stack_log_prob_terms runs usf_stack_run's
+ * pass in its deterministic form (whatever usf_set_deterministic says) and writes, besides log p and z:
+ *   out_terms : (n_blocks + 1) rows of B floats, leading dimension ldt >= B.  Row j < n_blocks is t_j of block j in
+ *               EXECUTION order (block j inverts coupling n_blocks - 1 - j of the generative layer list), row n_blocks
+ *               is b.  Every row is written (0.0 for an additive block); columns [B, ldt) are not touched.
+ *   out_logprob (B, optional): usf_stack_run's log p in deterministic mode, bit for bit; out_z (B, D) ldz (optional): z.
+ * const_term is in no row.  On the launch chain the slot sums of each block are added from 0 into its row in the same
+ * last kernel that adds all slots for log p; on the one-kernel path (usf_stack_is_single_kernel) the terms are the values
+ * that kernel adds to log p, so const_term + row 0 + ... + row n_blocks, added in that order in fp32, is out_logprob bit
+ * for bit.  Every precision is accepted; at most 255 blocks.  The workspace is usf_stack_terms_workspace_bytes (the
+ * deterministic slot area included). */
+size_t usf_stack_terms_workspace_bytes(const usf_stack_desc* st, int64_t B, int precision);
+int usf_stack_log_prob_terms(const usf_stack_desc* st, const float* x, int64_t ldx, int64_t B, float* out_logprob,
+                             float* out_terms, int64_t ldt, float* out_z, int64_t ldz, void* workspace,
+                             size_t workspace_bytes, int precision, int* gpu_launches, usf_stream_t stream);
 
 /* ---- input gradient of log p: log p(x) and d log p(x) / dx per row in one call ---------------------------------------
  * The reverse (vector-Jacobian) chain of an inverse-direction stack, with the weights treated as constants.  It needs

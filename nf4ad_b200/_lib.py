@@ -91,6 +91,9 @@ _PROTOS = {
     "usf_set_deterministic": (_int, [_int]),
     "usf_stack_run": (_int, [C.POINTER(StackDesc), _vp, _i64, _i64, _vp, _vp, _i64, _vp, _vp, _sz, _int,
                              C.POINTER(_int), _vp]),
+    "usf_stack_terms_workspace_bytes": (_sz, [C.POINTER(StackDesc), _i64, _int]),
+    "usf_stack_log_prob_terms": (_int, [C.POINTER(StackDesc), _vp, _i64, _i64, _vp, _vp, _i64, _vp, _i64, _vp, _sz, _int,
+                                        C.POINTER(_int), _vp]),
     "usf_stack_grad_workspace_bytes": (_sz, [C.POINTER(StackDesc), C.POINTER(StackGradDesc), _i64, _int]),
     "usf_stack_log_prob_grad": (_int, [C.POINTER(StackDesc), C.POINTER(StackGradDesc), _vp, _i64, _i64, _vp, _vp, _i64,
                                        _vp, _sz, _int, C.POINTER(_int), _vp]),

@@ -106,6 +106,26 @@ class ADBenchFlow:
                 out[i:i + chunk_rows] = (-g).cpu().numpy()
             return out
 
+    def score_terms(self, X_test: np.ndarray, chunk_rows: int = 65536) -> dict:
+        """The anomaly score split by the part of the model that produces it (`Flow.log_prob_terms`), in score sign
+        (-log p): {"score": (N,), "base": (N,) -log p_Z(z), "couplings": (N, K) one column per coupling in the order of
+        `flow.layers`, "affine": float, the affine layers' share}.  score = base + couplings.sum(1) + affine up to the order
+        of the fp32 adds.  Rows go to the device `chunk_rows` at a time."""
+        with torch.cuda.device(self.device):
+            X = torch.as_tensor(np.asarray(X_test), dtype=torch.float32)
+            self.flow_model.eval()
+            parts = {"score": [], "base": [], "couplings": []}
+            affine = 0.0
+            for i in range(0, max(X.shape[0], 1), chunk_rows):
+                t = self.flow_model.log_prob_terms(X[i:i + chunk_rows].to(self.device))
+                parts["score"].append((-t.log_prob).cpu().numpy())
+                parts["base"].append((-t.base).cpu().numpy())
+                parts["couplings"].append((-t.couplings).cpu().numpy())
+                affine = -float(t.affine)
+            out = {k: np.concatenate(v) for k, v in parts.items()}
+            out["affine"] = affine
+            return out
+
     def predict(self, X_test: np.ndarray, threshold: Optional[float] = None) -> np.ndarray:
         """1 = anomaly.  Default threshold: median score (adbench_wrapper.py:435-449)."""
         scores = self.predict_score(X_test)

@@ -166,7 +166,13 @@ int run_chain(const usf_stack_desc* st, const void* x, int64_t ldx, bool x_bf16,
   const int64_t d_in = (int64_t)st->D + st->ctx_dim;   // input row = D coordinates + the context columns
   // deterministic mode: the accumulating launches store into consecutive slots instead of adding atomically
   float* det = io.row_acc != nullptr ? io.det : nullptr;
+  USF_CHECK_ARG(io.terms == nullptr || (det != nullptr && io.density && st->n_blocks < kMaxTermRows),
+                "stack: log p terms need the deterministic slots of a density pass");
   int det_cursor = 0;
+  SlotTerms tm{};   // (io.terms: the slot range of every block and of the base density)
+  tm.out = io.terms;
+  tm.ldt = io.ldt;
+  tm.n = st->n_blocks + 1;
   auto det_assign = [&](EpiParams& ep, int n) {
     if (det == nullptr || n == 0) return;
     ep.row_part = det;
@@ -241,6 +247,7 @@ int run_chain(const usf_stack_desc* st, const void* x, int64_t ldx, bool x_bf16,
     cp.clamp = blk.clamp;
     cp.row_acc = io.row_acc;
     det_assign(cp, det_slots(st, b, precision));
+    if (tm.out != nullptr) tm.end[b] = det_cursor;
     void* ub_lo = u.lo != nullptr ? static_cast<uint8_t*>(u.lo) + (size_t)blk.b_off * esz : nullptr;
     const int k0 = k;
     k += blk.n_mlp - 1;
@@ -304,6 +311,7 @@ int run_chain(const usf_stack_desc* st, const void* x, int64_t ldx, bool x_bf16,
       ep.inv_scale = st->inv_scale;
       ep.row_acc = io.row_acc;
       det_assign(ep, det_slots(st, st->n_blocks, precision));
+      if (tm.out != nullptr) tm.end[st->n_blocks] = det_cursor;
     } else {
       USF_CHECK_ARG(io.out != nullptr, "usf_stack_run: nothing to compute (no output requested)");
       ep.mode = EPI_BIAS;
@@ -317,7 +325,7 @@ int run_chain(const usf_stack_desc* st, const void* x, int64_t ldx, bool x_bf16,
   ++*launches;
   // deterministic mode: the slots, added in slot order, on top of the seeded accumulator
   if (det != nullptr && det_cursor > 0) {
-    rc = launch_sum_row_parts(io.row_acc, det, rows, det_cursor, rows, s);
+    rc = launch_sum_row_parts(io.row_acc, det, rows, det_cursor, rows, tm, s);
     if (rc) return rc;
     ++*launches;
   }
@@ -438,12 +446,15 @@ extern "C" size_t usf_stack_workspace_bytes(const usf_stack_desc* st, int64_t B,
 }
 
 // x_bf16: x points to bf16 rows (ldx in bf16 elements) instead of fp32 ones -- usf_stack_run_bf16in
+// out_terms (ldt): the log p terms of usf_stack_log_prob_terms (deterministic mode), or nullptr
 static int stack_run_eager(const usf_stack_desc* st, const float* x, int64_t ldx, int64_t B, float* out_logprob,
                            float* out_y, int64_t ldy, float* out_ladj, void* workspace, size_t workspace_bytes,
-                           int precision, int* gpu_launches, usf_stream_t stream, int x_bf16) {
+                           int precision, int* gpu_launches, usf_stream_t stream, int x_bf16, float* out_terms,
+                           int64_t ldt) {
   USF_CHECK_ARG(st != nullptr && x != nullptr && B >= 0, "usf_stack_run: bad arguments");
   USF_CHECK_ARG(!x_bf16 || precision == USF_PREC_BF16, "usf_stack_run_bf16in: bf16 rows need the bf16 precision tier");
-  USF_CHECK_ARG(!(out_logprob && (st->base_kind < 0 || !st->inverse)),
+  const bool density = out_logprob != nullptr || out_terms != nullptr;
+  USF_CHECK_ARG(!(density && (st->base_kind < 0 || !st->inverse)),
                 "usf_stack_run: log_prob needs the inverse direction and a base distribution");
   USF_CHECK_ARG(!(out_logprob && out_ladj), "usf_stack_run: request log_prob or ladj, not both");
   const int64_t d_in = (int64_t)st->D + st->ctx_dim;   // input row = D coordinates + the context columns
@@ -453,11 +464,11 @@ static int stack_run_eager(const usf_stack_desc* st, const float* x, int64_t ldx
   // small event shapes (D + context <= 64, widths <= 128; fp32 weights): the whole stack in ONE kernel, rows resident
   // in shared memory across all layers (usf_small.cu) -- the chain below would be 8-40 launches of a few microseconds
   if (!x_bf16 && small_stack_supported(st, precision)) {
-    USF_CHECK_ARG(out_logprob != nullptr || out_y != nullptr || out_ladj != nullptr, "usf_stack_run: nothing to compute (no output requested)");
+    USF_CHECK_ARG(density || out_y != nullptr || out_ladj != nullptr, "usf_stack_run: nothing to compute (no output requested)");
     int rc1;
     {
       ProfScope ps(as_stream(stream), 6);
-      rc1 = small_stack_run(st, x, ldx, B, out_logprob, out_y, ldy, out_ladj, as_stream(stream));
+      rc1 = small_stack_run(st, x, ldx, B, out_logprob, out_y, ldy, out_ladj, out_terms, ldt, as_stream(stream));
     }
     if (rc1 == USF_OK && gpu_launches) *gpu_launches = 1;
     return rc1;
@@ -470,13 +481,13 @@ static int stack_run_eager(const usf_stack_desc* st, const float* x, int64_t ldx
     set_error("usf_stack_run: workspace too small (%zu < %zu bytes)", workspace_bytes, p.total);
     return USF_E_WORKSPACE;
   }
-  // two ping-pong activation and hidden buffers, the (unused) accumulator region, the split-K scratch, the low-part
-  // twins of the four buffers (3xTF32 / bf16x2), the deterministic slot area
+  // two ping-pong activation and hidden buffers, the accumulator region (log p of a terms call without out_logprob), the
+  // split-K scratch, the low-part twins of the four buffers (3xTF32 / bf16x2), the deterministic slot area
   Arena ws(workspace);
   Buf act[2], hid[2];
   for (Buf& a : act) a = {ws.take(p.act_bytes), nullptr, p.ld_act};
   for (Buf& h : hid) h = {ws.take(p.hid_bytes), nullptr, p.ld_hid};
-  ws.take(p.acc_bytes);
+  float* const acc_ws = static_cast<float*>(ws.take(p.acc_bytes));
   ChainIO io{};
   io.scratch = p.small_bytes ? static_cast<float*>(ws.take(p.small_bytes)) : nullptr;
   io.scratch_floats = p.small_bytes / sizeof(float);
@@ -490,15 +501,17 @@ static int stack_run_eager(const usf_stack_desc* st, const float* x, int64_t ldx
   io.n_act = 2;
   io.hid = hid;
   io.n_hid = 2;
-  io.density = out_logprob != nullptr;
+  io.density = density;
   io.ldo = ldy;
-  io.acc_init = out_logprob ? st->const_term : 0.f;
+  io.acc_init = density ? st->const_term : 0.f;
+  io.ldt = ldt;
   float* acc = out_logprob ? out_logprob : out_ladj;
   int launches = 0;
   for (int64_t r0 = 0; r0 < B; r0 += kChunkRows) {
     const int64_t rows = (B - r0) < kChunkRows ? (B - r0) : kChunkRows;
     io.out = out_y ? out_y + r0 * ldy : nullptr;
-    io.row_acc = acc ? acc + r0 : nullptr;
+    io.row_acc = acc ? acc + r0 : (out_terms ? acc_ws : nullptr);
+    io.terms = out_terms ? out_terms + r0 : nullptr;
     const void* xr = x_bf16 ? static_cast<const void*>(reinterpret_cast<const uint16_t*>(x) + r0 * ldx) : x + r0 * ldx;
     rc = run_chain(st, xr, ldx, x_bf16, rows, precision, io, &launches, as_stream(stream));
     if (rc) return rc;
@@ -560,17 +573,20 @@ extern "C" int usf_debug_graph_stats(long long* stats4, char* last_failure, int 
 
 static int stack_run_cached(const usf_stack_desc* st, const float* x, int64_t ldx, int64_t B, float* out_logprob,
                             float* out_y, int64_t ldy, float* out_ladj, void* workspace, size_t workspace_bytes,
-                            int precision, int* gpu_launches, usf_stream_t stream, int x_bf16) {
+                            int precision, int* gpu_launches, usf_stream_t stream, int x_bf16, float* out_terms,
+                            int64_t ldt) {
   if (st == nullptr || !graphs_enabled() || g_prof.on || B <= 0 || st->n_blocks < 0 ||
       (st->n_blocks > 0 && st->blocks == nullptr))
     return stack_run_eager(st, x, ldx, B, out_logprob, out_y, ldy, out_ladj, workspace, workspace_bytes, precision,
-                           gpu_launches, stream, x_bf16);
+                           gpu_launches, stream, x_bf16, out_terms, ldt);
   // key material = every descriptor byte and every call argument; the 64-bit hash only pre-filters, a hit compares
-  // the bytes themselves (a hash collision must never replay another chain)
-  const uint64_t extra[9] = {(uint64_t)(uintptr_t)x, (uint64_t)ldx, (uint64_t)B, (uint64_t)(uintptr_t)out_logprob,
-                             (uint64_t)(uintptr_t)out_y, (uint64_t)ldy, (uint64_t)(uintptr_t)out_ladj,
-                             (uint64_t)(uintptr_t)workspace,
-                             (uint64_t)workspace_bytes * 16u + (uint64_t)precision + (x_bf16 ? 4u : 0u) + (g_deterministic ? 8u : 0u)};
+  // the bytes themselves (a hash collision must never replay another chain).  A terms call (out_terms, bit 16) and a
+  // plain run never share a key.
+  const uint64_t extra[11] = {(uint64_t)(uintptr_t)x, (uint64_t)ldx, (uint64_t)B, (uint64_t)(uintptr_t)out_logprob,
+                              (uint64_t)(uintptr_t)out_y, (uint64_t)ldy, (uint64_t)(uintptr_t)out_ladj,
+                              (uint64_t)(uintptr_t)workspace, (uint64_t)(uintptr_t)out_terms, (uint64_t)ldt,
+                              (uint64_t)workspace_bytes * 32u + (uint64_t)precision + (x_bf16 ? 4u : 0u) +
+                                  (g_deterministic ? 8u : 0u) + (out_terms ? 16u : 0u)};
   const size_t nb_bytes = st->n_blocks > 0 ? sizeof(usf_block_desc) * (size_t)st->n_blocks : 0;
   thread_local std::vector<unsigned char> kb;
   kb.resize(sizeof(*st) + nb_bytes + sizeof(extra));
@@ -603,7 +619,7 @@ static int stack_run_cached(const usf_stack_desc* st, const float* x, int64_t ld
     victim->stamp = ++g_graph_clock;
     ++g_graph_stats[3];
     return stack_run_eager(st, x, ldx, B, out_logprob, out_y, ldy, out_ladj, workspace, workspace_bytes, precision,
-                           gpu_launches, stream, x_bf16);
+                           gpu_launches, stream, x_bf16, out_terms, ldt);
   }
   // second identical call: capture the chain, instantiate, replay
   slot->stamp = ++g_graph_clock;
@@ -611,17 +627,17 @@ static int stack_run_cached(const usf_stack_desc* st, const float* x, int64_t ld
       cudaStreamCreateWithFlags(&g_capture_stream, cudaStreamNonBlocking) != cudaSuccess) {
     cudaGetLastError();
     return stack_run_eager(st, x, ldx, B, out_logprob, out_y, ldy, out_ladj, workspace, workspace_bytes, precision,
-                           gpu_launches, stream, x_bf16);
+                           gpu_launches, stream, x_bf16, out_terms, ldt);
   }
   int launches = 0;
   cudaGraph_t graph = nullptr;
   if (cudaStreamBeginCapture(g_capture_stream, cudaStreamCaptureModeThreadLocal) != cudaSuccess) {
     cudaGetLastError();
     return stack_run_eager(st, x, ldx, B, out_logprob, out_y, ldy, out_ladj, workspace, workspace_bytes, precision,
-                           gpu_launches, stream, x_bf16);
+                           gpu_launches, stream, x_bf16, out_terms, ldt);
   }
   const int rc = stack_run_eager(st, x, ldx, B, out_logprob, out_y, ldy, out_ladj, workspace, workspace_bytes, precision,
-                                 &launches, g_capture_stream, x_bf16);
+                                 &launches, g_capture_stream, x_bf16, out_terms, ldt);
   const cudaError_t ce = cudaStreamEndCapture(g_capture_stream, &graph);
   cudaGraphExec_t exec = nullptr;
   cudaError_t ie = cudaSuccess;
@@ -634,7 +650,7 @@ static int stack_run_cached(const usf_stack_desc* st, const float* x, int64_t ld
     if (graph != nullptr) cudaGraphDestroy(graph);
     slot->key = 0;   // do not try again with this key
     return stack_run_eager(st, x, ldx, B, out_logprob, out_y, ldy, out_ladj, workspace, workspace_bytes, precision,
-                           gpu_launches, stream, x_bf16);
+                           gpu_launches, stream, x_bf16, out_terms, ldt);
   }
   cudaGraphDestroy(graph);
   ++g_graph_stats[1];
@@ -659,12 +675,49 @@ extern "C" int usf_stack_run(const usf_stack_desc* st, const float* x, int64_t l
                              float* out_y, int64_t ldy, float* out_ladj, void* workspace, size_t workspace_bytes,
                              int precision, int* gpu_launches, usf_stream_t stream) {
   return stack_run_cached(st, x, ldx, B, out_logprob, out_y, ldy, out_ladj, workspace, workspace_bytes, precision,
-                          gpu_launches, stream, 0);
+                          gpu_launches, stream, 0, nullptr, 0);
 }
 
 extern "C" int usf_stack_run_bf16in(const usf_stack_desc* st, const uint16_t* x_bf16, int64_t ldx, int64_t B,
                                     float* out_logprob, float* out_y, int64_t ldy, float* out_ladj, void* workspace,
                                     size_t workspace_bytes, int* gpu_launches, usf_stream_t stream) {
   return stack_run_cached(st, reinterpret_cast<const float*>(x_bf16), ldx, B, out_logprob, out_y, ldy, out_ladj, workspace,
-                          workspace_bytes, USF_PREC_BF16, gpu_launches, stream, 1);
+                          workspace_bytes, USF_PREC_BF16, gpu_launches, stream, 1, nullptr, 0);
+}
+
+namespace {
+// usf_stack_log_prob_terms runs the slot form of the chain whatever usf_set_deterministic says
+struct DeterministicScope {
+  int prev;
+  DeterministicScope() : prev(g_deterministic) { g_deterministic = 1; }
+  ~DeterministicScope() { g_deterministic = prev; }
+};
+}  // namespace
+
+extern "C" size_t usf_stack_terms_workspace_bytes(const usf_stack_desc* st, int64_t B, int precision) {
+  DeterministicScope det;
+  return usf_stack_workspace_bytes(st, B, precision);
+}
+
+extern "C" int usf_stack_log_prob_terms(const usf_stack_desc* st, const float* x, int64_t ldx, int64_t B,
+                                        float* out_logprob, float* out_terms, int64_t ldt, float* out_z, int64_t ldz,
+                                        void* workspace, size_t workspace_bytes, int precision, int* gpu_launches,
+                                        usf_stream_t stream) {
+  USF_CHECK_ARG(st != nullptr && x != nullptr && out_terms != nullptr && B >= 0, "usf_stack_log_prob_terms: bad arguments");
+  USF_CHECK_ARG(st->inverse && st->base_kind >= 0,
+                "usf_stack_log_prob_terms: needs the inverse direction and a base distribution");
+  USF_CHECK_ARG(st->n_blocks >= 0 && st->n_blocks < kMaxTermRows, "usf_stack_log_prob_terms: at most %d blocks",
+                kMaxTermRows - 1);
+  USF_CHECK_ARG(ldt >= B && (out_z == nullptr || ldz >= st->D), "usf_stack_log_prob_terms: leading dimension too small");
+  if (gpu_launches) *gpu_launches = 0;
+  if (B == 0) return USF_OK;
+  DeterministicScope det;
+  const size_t need = usf_stack_workspace_bytes(st, B, precision);
+  if (need == 0) return USF_E_ARG;   // (plan_stack has set the message)
+  if (workspace == nullptr || workspace_bytes < need) {
+    set_error("usf_stack_log_prob_terms: workspace too small (%zu < %zu bytes)", workspace_bytes, need);
+    return USF_E_WORKSPACE;
+  }
+  return stack_run_cached(st, x, ldx, B, out_logprob, out_z, ldz, nullptr, workspace, workspace_bytes, precision,
+                          gpu_launches, stream, 0, out_terms, ldt);
 }

@@ -144,8 +144,10 @@ int trsm_rows(const float* T, int64_t D, bool lower, bool unit, bool trans, cons
 
 // ---- whole-stack kernel for small event shapes (usf_small.cu): one launch instead of the chain ------------------
 bool small_stack_supported(const usf_stack_desc* st, int precision);
+// out_terms (optional, n_blocks + 1 rows of ldt floats): usf_stack_log_prob_terms -- what each block and the base density
+// add to a row's log p, from the kernel's terms instance
 int small_stack_run(const usf_stack_desc* st, const float* x, int64_t ldx, int64_t B, float* out_logprob, float* out_y,
-                    int64_t ldy, float* out_ladj, cudaStream_t stream);
+                    int64_t ldy, float* out_ladj, float* out_terms, int64_t ldt, cudaStream_t stream);
 // its gradient twin (usf_stack_log_prob_grad at fp32): log p and d log p / dx in one launch
 bool small_grad_supported(const usf_stack_desc* st, const usf_stack_grad_desc* gd, int precision);
 size_t small_grad_workspace_bytes(const usf_stack_desc* st, const usf_stack_grad_desc* gd);
@@ -158,8 +160,19 @@ int launch_convert_rows(const float* x, int64_t ldx, uint16_t* y_bf16, float* y_
                         int64_t B, int64_t D, float* row_init, float init_value, cudaStream_t stream);
 int launch_copy_rows_bf16(const uint16_t* x, int64_t ldx, uint16_t* y, int64_t ldy, int64_t B, int64_t D, float* row_init,
                           float init_value, cudaStream_t stream);
-// out[r] += sum over slots (in slot order) of part[s * ld + r]: the end of a deterministic launch chain
-int launch_sum_row_parts(float* out, const float* part, int64_t ld, int slots, int64_t rows, cudaStream_t stream);
+// usf_stack_log_prob_terms: the slots of the deterministic chain split into n consecutive ranges (range j ends before slot
+// end[j], end[n - 1] is the slot count); out == nullptr: no terms.
+constexpr int kMaxTermRows = 256;
+struct SlotTerms {
+  float* out;     // range j's sum, added from 0 in slot order, goes to out[j * ldt + row]
+  int64_t ldt;
+  int n;
+  int end[kMaxTermRows];
+};
+// out[r] += sum over slots (in slot order) of part[s * ld + r]: the end of a deterministic launch chain; with tm.out, in the
+// same pass each range of slots summed on its own into its row of tm.out
+int launch_sum_row_parts(float* out, const float* part, int64_t ld, int slots, int64_t rows, const SlotTerms& tm,
+                         cudaStream_t stream);
 int launch_bf16_to_f32(const uint16_t* x, int64_t ldx, float* y, int64_t ldy, int64_t B, int64_t D,
                        cudaStream_t stream);
 
@@ -198,6 +211,8 @@ struct ChainIO {
   int det_n;
   float* scratch;            // fp32 split-K accumulator (chain_gemm), or nullptr
   size_t scratch_floats;
+  float* terms;              // deterministic mode only: per block, then the base density, its slots' sum (ldt apart)
+  int64_t ldt;
 };
 
 // The forward chain over `rows` rows of x (fp32 rows, or bf16 rows when x_bf16) at `precision`: input pack, per block

@@ -320,20 +320,36 @@ __global__ void usf_simt_epilogue_kernel(const float* __restrict__ acc, int64_t 
   }
 }
 
-// out[r] += part[0][r] + part[1][r] + ... in slot order (deterministic mode: the end of the launch chain)
-__global__ void usf_sum_row_parts_kernel(float* out, const float* __restrict__ part, int64_t ld, int slots, int64_t rows) {
+// out[r] += part[0][r] + part[1][r] + ... in slot order (deterministic mode: the end of the launch chain).  With tm.out the
+// same adds, in the same order, also go range by range into a sum of their own that starts from 0 (the log p terms).
+__global__ void usf_sum_row_parts_kernel(float* out, const float* __restrict__ part, int64_t ld, int slots, int64_t rows,
+                                         const __grid_constant__ SlotTerms tm) {
   for (int64_t r = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; r < rows; r += (int64_t)gridDim.x * blockDim.x) {
     float v = out[r];
-    for (int s = 0; s < slots; ++s) v += part[(int64_t)s * ld + r];
+    if (tm.out == nullptr) {
+      for (int s = 0; s < slots; ++s) v += part[(int64_t)s * ld + r];
+    } else {
+      int s = 0;
+      for (int j = 0; j < tm.n; ++j) {
+        float t = 0.f;
+        for (; s < tm.end[j]; ++s) {
+          const float p = part[(int64_t)s * ld + r];
+          v += p;
+          t += p;
+        }
+        tm.out[(int64_t)j * tm.ldt + r] = t;
+      }
+    }
     out[r] = v;
   }
 }
 
-int launch_sum_row_parts(float* out, const float* part, int64_t ld, int slots, int64_t rows, cudaStream_t stream) {
+int launch_sum_row_parts(float* out, const float* part, int64_t ld, int slots, int64_t rows, const SlotTerms& tm,
+                         cudaStream_t stream) {
   if (rows <= 0 || slots <= 0) return USF_OK;
   int64_t blocks = (rows + 255) / 256;
   if (blocks > 148 * 8) blocks = 148 * 8;
-  usf_sum_row_parts_kernel<<<(unsigned)blocks, 256, 0, stream>>>(out, part, ld, slots, rows);
+  usf_sum_row_parts_kernel<<<(unsigned)blocks, 256, 0, stream>>>(out, part, ld, slots, rows, tm);
   USF_LAUNCH_CHECK("usf_sum_row_parts_kernel");
   return USF_OK;
 }

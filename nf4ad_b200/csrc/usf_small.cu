@@ -96,6 +96,12 @@ struct SsArgsT {
 };
 using SsArgs = SsArgsT<SS_MAX_OPS>;
 using SsGradArgs = SsArgsT<SS_MAX_GRAD_OPS>;
+// the terms instance (usf_stack_log_prob_terms): row j < n_blocks of out_terms receives what block j adds to log p, row
+// n_blocks the base log-density sum
+struct SsTermsArgs : SsArgs {
+  float* out_terms;
+  int64_t ldt;
+};
 
 __device__ __forceinline__ float half_warp_sum(float v) {
   // the 16 column lanes of one row group are 16 consecutive lanes of a warp
@@ -186,10 +192,17 @@ struct SsLayerCtx {
   float* save;
 };
 
+// TERMS: a value the row's log p accumulator just took, stored into row `term` of out_terms
+template <class A>
+__device__ __forceinline__ void store_term(const A& args, const SsLayerCtx& cx, int term, int r, float v) {
+  if (r < cx.nrows) args.out_terms[(int64_t)term * args.ldt + cx.row0 + r] = v;
+}
+
 // One layer on this thread's 4 x (16 JN) register tile: GEMM against the staged weights, then the layer's epilogue.
 // GRAD: the gradient kernel's instance -- the same GEMM and forward epilogues, which also keep what the reverse pass
-// reads (block output rows, dL/dz), plus the reverse epilogues.
-template <int JN, bool GRAD, class A>
+// reads (block output rows, dL/dz), plus the reverse epilogues.  TERMS: the terms instance -- the same arithmetic, and
+// every term added to a row's log p also stored on its own (store_term).
+template <int JN, bool GRAD, bool TERMS = false, class A>
 __device__ __forceinline__ void ss_layer(const A& args, const SsOp& op, const SsLayerCtx& cx) {
   const int jn = cx.jn, tx = cx.tx, ty = cx.ty, lda = cx.lda;
   const float* bbuf = cx.bbuf;
@@ -334,7 +347,12 @@ __device__ __forceinline__ void ss_layer(const A& args, const SsOp& op, const Ss
       for (int i = 0; i < 4; ++i) {
         const float s = half_warp_sum(lsum[i]);
         if (tx == 0) cx.racc[ty * 4 + i] += args.inverse ? -s : s;   // one writer per row, fixed order: deterministic
+        if constexpr (TERMS)
+          if (tx == 0) store_term(args, cx, op.slot, ty * 4 + i, args.inverse ? -s : s);
       }
+    } else if constexpr (TERMS) {
+      if (tx == 0)
+        for (int i = 0; i < 4; ++i) store_term(args, cx, op.slot, ty * 4 + i, 0.f);   // an additive block adds nothing
     }
   } else {  // SS_FINAL: natural column order, optional store, optional base log-density
     float lsum[4] = {0.f, 0.f, 0.f, 0.f};
@@ -368,6 +386,8 @@ __device__ __forceinline__ void ss_layer(const A& args, const SsOp& op, const Ss
       for (int i = 0; i < 4; ++i) {
         const float s = half_warp_sum(lsum[i]);
         if (tx == 0) cx.racc[ty * 4 + i] += s;
+        if constexpr (TERMS)
+          if (tx == 0) store_term(args, cx, args.n_blocks, ty * 4 + i, s);
       }
     }
   }
@@ -377,7 +397,7 @@ __device__ __forceinline__ void ss_layer(const A& args, const SsOp& op, const Ss
 // its log p is usf_small_stack_kernel's bit for bit -- and then its reverse ops on the tile, last block first, before
 // the next tile.  Shared memory: the scoring kernel's buffers (nhs hidden slots instead of 2), then, GRAD only and when
 // they fit, the saved block output rows (else args.save, this CTA's part).
-template <bool GRAD, class A>
+template <bool GRAD, bool TERMS = false, class A>
 __device__ __forceinline__ void ss_body(const A& args) {
   extern __shared__ float4 smem4[];
   float* smem = reinterpret_cast<float*>(smem4);
@@ -469,10 +489,10 @@ __device__ __forceinline__ void ss_body(const A& args) {
         float* const aux = rbuf(op.aux, op.slot, ldx);
         SsLayerCtx cx{in, ldi, wbuf, bbuf, ldw, K4, jn, nullptr, nullptr, out, lda, ldo,
                       racc, locs, iscs, row0, nrows, tx, ty, aux, ldx, save};
-        if (jn <= 1) ss_layer<1, GRAD>(args, op, cx);
-        else if (jn == 2) ss_layer<2, GRAD>(args, op, cx);
-        else if (jn <= 4) ss_layer<4, GRAD>(args, op, cx);
-        else ss_layer<8, GRAD>(args, op, cx);
+        if (jn <= 1) ss_layer<1, GRAD, TERMS>(args, op, cx);
+        else if (jn == 2) ss_layer<2, GRAD, TERMS>(args, op, cx);
+        else if (jn <= 4) ss_layer<4, GRAD, TERMS>(args, op, cx);
+        else ss_layer<8, GRAD, TERMS>(args, op, cx);
       } else {
         const float* in;
         int ldi = lda;
@@ -481,10 +501,10 @@ __device__ __forceinline__ void ss_body(const A& args) {
         else { in = hp ? hid1 : hid0; ldi = ldh; }
         SsLayerCtx cx{in, ldi, wbuf, bbuf, ldw, K4, jn, actc, cur ? act0 : act1, (op.first || hp) ? hid0 : hid1, lda, ldh,
                       racc, locs, iscs, row0, nrows, tx, ty, cur ? act0 : act1, lda, save};   // (aux: dL/dz of the final op)
-        if (jn <= 1) ss_layer<1, GRAD>(args, op, cx);
-        else if (jn == 2) ss_layer<2, GRAD>(args, op, cx);
-        else if (jn <= 4) ss_layer<4, GRAD>(args, op, cx);
-        else ss_layer<8, GRAD>(args, op, cx);
+        if (jn <= 1) ss_layer<1, GRAD, TERMS>(args, op, cx);
+        else if (jn == 2) ss_layer<2, GRAD, TERMS>(args, op, cx);
+        else if (jn <= 4) ss_layer<4, GRAD, TERMS>(args, op, cx);
+        else ss_layer<8, GRAD, TERMS>(args, op, cx);
         if (op.kind == SS_AFFINE) cur ^= 1;
         else if (op.kind == SS_HIDDEN) hp = (op.first || hp) ? 0 : 1;
         else if (op.kind == SS_COUPLING) hp = 0;
@@ -503,6 +523,11 @@ __device__ __forceinline__ void ss_body(const A& args) {
 
 __global__ void __launch_bounds__(SS_THREADS, 2) usf_small_stack_kernel(const __grid_constant__ SsArgs args) {
   ss_body<false>(args);
+}
+
+// usf_small_stack_kernel that also stores the terms of log p (usf_stack_log_prob_terms)
+__global__ void __launch_bounds__(SS_THREADS, 2) usf_small_stack_terms_kernel(const __grid_constant__ SsTermsArgs args) {
+  ss_body<false, true>(args);
 }
 
 // log p and d log p / dx of a tile in one launch: the forward ops of usf_small_stack_kernel, then the reverse ops.
@@ -745,14 +770,37 @@ size_t small_grad_workspace_bytes(const usf_stack_desc* st, const usf_stack_grad
   return 256 + grad_saved_bytes(a, L);
 }
 
+// The scoring launch of `kernel` (its own shared-memory attribute, set once per thread: one flag per instance of A).
+template <class A>
+int small_launch(void (*kernel)(A), const A& a, int64_t B, const char* name, cudaStream_t stream) {
+  const size_t smem = smem_bytes(a);
+  static thread_local bool attr_set = false;
+  if (smem > 48 * 1024 && !attr_set) {
+    USF_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(227 * 1024)));
+    attr_set = true;
+  }
+  int per_sm = 1;
+  if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, SS_THREADS, smem) != cudaSuccess || per_sm < 1) {
+    cudaGetLastError();
+    per_sm = 1;
+  }
+  const int64_t tiles = ceil_div(B, SS_ROWS);
+  int64_t grid = (int64_t)num_sms() * per_sm;
+  if (grid > tiles) grid = tiles;
+  kernel<<<(unsigned)grid, SS_THREADS, smem, stream>>>(a);
+  const cudaError_t e = cudaGetLastError();
+  return e != cudaSuccess ? cuda_fail(e, name) : USF_OK;
+}
+
 int small_stack_run(const usf_stack_desc* st, const float* x, int64_t ldx, int64_t B, float* out_logprob, float* out_y,
-                    int64_t ldy, float* out_ladj, cudaStream_t stream) {
-  static thread_local SsArgs a;
+                    int64_t ldy, float* out_ladj, float* out_terms, int64_t ldt, cudaStream_t stream) {
+  static thread_local SsTermsArgs a;
   USF_CHECK_ARG(build_args(st, &a), "small_stack_run: unsupported stack");
+  const bool density = out_logprob != nullptr || out_terms != nullptr;
   a.d_in = st->D + st->ctx_dim;
   a.D = st->D;
   a.inverse = st->inverse;
-  a.base_kind = out_logprob != nullptr ? st->base_kind : -1;
+  a.base_kind = density ? st->base_kind : -1;
   a.B = B;
   a.x = x;
   a.ldx = ldx;
@@ -761,26 +809,15 @@ int small_stack_run(const usf_stack_desc* st, const float* x, int64_t ldx, int64
   a.out_y = out_y;
   a.ldy = ldy;
   a.out_ladj = out_ladj;
-  a.acc_init = out_logprob != nullptr ? st->const_term : 0.f;
+  a.acc_init = density ? st->const_term : 0.f;
   a.loc = st->loc;
   a.inv_scale = st->inv_scale;
-  const size_t smem = smem_bytes(a);
-  static thread_local bool attr_set = false;
-  if (smem > 48 * 1024 && !attr_set) {
-    USF_CUDA(cudaFuncSetAttribute(usf_small_stack_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(227 * 1024)));
-    attr_set = true;
-  }
-  int per_sm = 1;
-  if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, usf_small_stack_kernel, SS_THREADS, smem) != cudaSuccess || per_sm < 1) {
-    cudaGetLastError();
-    per_sm = 1;
-  }
-  const int64_t tiles = ceil_div(B, SS_ROWS);
-  int64_t grid = (int64_t)num_sms() * per_sm;
-  if (grid > tiles) grid = tiles;
-  usf_small_stack_kernel<<<(unsigned)grid, SS_THREADS, smem, stream>>>(a);
-  USF_LAUNCH_CHECK("usf_small_stack_kernel");
-  return USF_OK;
+  a.out_terms = out_terms;
+  a.ldt = ldt;
+  if (out_terms != nullptr)
+    return small_launch(usf_small_stack_terms_kernel, static_cast<const SsTermsArgs&>(a), B,
+                        "launch of usf_small_stack_terms_kernel", stream);
+  return small_launch(usf_small_stack_kernel, static_cast<const SsArgs&>(a), B, "launch of usf_small_stack_kernel", stream);
 }
 
 int small_grad_run(const usf_stack_desc* st, const usf_stack_grad_desc* gd, const float* x, int64_t ldx, int64_t B,

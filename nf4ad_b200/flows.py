@@ -101,6 +101,18 @@ class _TierDecision(NamedTuple):
     err: Optional[float]        # max-row error of the bf16 calibration, None where it did not run
 
 
+class LogProbTerms(NamedTuple):
+    """`Flow.log_prob_terms`: log p(x) and the parts it is the sum of, log_prob = base + couplings.sum(-1) + affine (up to
+    the order of the fp32 adds).  For anomaly scores: which part of the model -- the latent density or the volume change
+    of a coupling -- makes a sample unlikely."""
+    log_prob: torch.Tensor      # (*lead,) what `flow.log_prob(x)` returns under torch.no_grad()
+    base: torch.Tensor          # (*lead,) log p_Z(z), the base distribution's normalising constant included
+    couplings: torch.Tensor     # (*lead, K) column k: the inverse log|det| of the k-th coupling of `flow.layers` (generative
+                                #   order), i.e. its contribution to log p; exactly 0.0 for an additive coupling
+    affine: torch.Tensor        # () the summed inverse log|det| of the affine layers (LU, Scale, Householder, ...)
+    z: torch.Tensor             # (*lead, *event) the latent point, as `flow.backward(x)`
+
+
 class _SmallDecision(NamedTuple):
     """`Flow._small_cache`: does the one-kernel path take the stack on the weights `key`, and its widest layer."""
     key: tuple
@@ -482,6 +494,42 @@ class Flow(torch.nn.Module):
         self.last_launches = n
         return lp.reshape(lead), g.reshape(x.shape)
 
+    @_on_device
+    def log_prob_terms(self, x, context=None):
+        """log p(x) split into its terms (`LogProbTerms`): the base log-density at the latent point, each coupling's
+        log-det term and the affine layers' constant -- the split likelihood-based out-of-distribution detection looks at
+        (latent density against volume change, and which coupling).  Same `x`, `context` and errors as `log_prob`; builds
+        no autograd graph.
+
+        A flat-event stack runs `log_prob`'s fused pass -- the same tier (`_tier`), one-kernel eligibility and packed
+        stack -- in its deterministic form, which keeps the per-block sums it adds for log p apart
+        (usf_stack_log_prob_terms): `log_prob` is `flow.log_prob(x)`'s bit for bit when `deterministic` is set (and always on
+        the one-kernel path), `z` is `flow.backward(x)`'s.  `effective_precision` and `last_launches` report the call as
+        for `log_prob`.  Other flows (image-shaped events, opaque conditioners, softplus scales, an unsupported base, a
+        context handed to an unconditional flow) collect the terms from the layer-wise pass."""
+        with torch.no_grad():
+            x2, lead, context, cs, xin = self._fused(x, context)
+            if cs is not None and cs.desc.base_kind >= 0:
+                lp, t, z, n = cs.run_terms(xin)
+                self.last_launches = n
+                nb = cs.desc.n_blocks
+                return LogProbTerms(lp.reshape(lead), (t[nb] + cs.base_const).reshape(lead),
+                                    t[:nb].flip(0).t().reshape(*lead, nb),         # execution -> generative order
+                                    torch.full((), -cs.logdet_const, dtype=torch.float32, device=x2.device),
+                                    z.reshape(*lead, *self._tail(x, z)))
+            parts = []
+            z, neg_ladj = self._inverse_layers(self._unflat(x2), context, collect=parts)
+            base = self._base_log_prob(z.reshape(z.shape[0], -1))
+            B = x2.shape[0]
+            cols = [c.expand(B) for item, c in reversed(parts) if stack._is_coupling(item)]
+            affine = torch.zeros((), dtype=torch.float32, device=x2.device)
+            for item, c in parts:
+                if not stack._is_coupling(item):
+                    affine = affine + c
+            couplings = torch.stack(cols, -1) if cols else base.new_zeros(B, 0)
+            return LogProbTerms((base + neg_ladj).reshape(lead), base.reshape(lead), couplings.reshape(*lead, len(cols)),
+                                affine.reshape(lead) if affine.dim() else affine, z.reshape(*lead, *self._tail(x, z)))
+
     def _prefetch_lu_inverses(self, y):
         """Mixed-precision training: the dense inverses of all LU layers this pass will apply are independent of the
         data and of each other, and one inversion (two 25-CTA triangular solves on the identity) cannot fill the GPU.
@@ -684,8 +732,10 @@ class Flow(torch.nn.Module):
                 cond.__dict__["_usf_pre"] = (pre, st)
         self.__dict__["_cond_pending"] = st
 
-    def _inverse_layers(self, y, context=None):
-        """Layer-wise data -> latent with the accumulated -sum(ladj) (autograd-capable)."""
+    def _inverse_layers(self, y, context=None, collect=None):
+        """Layer-wise data -> latent with the accumulated -sum(ladj) (autograd-capable).  `collect`: a list that receives
+        (layer, its -ladj as an fp32 tensor) per layer in the order of the pass (a composed affine run: (its layer list,
+        -log-det))."""
         # (fp32 training -- the reference's arithmetic -- stays layer-wise: composed, its C2 step takes 14.2 instead of
         # 23.2 ms, but the reflection vectors' gradients, differences of large terms of dM, end up 4.6e-3 from the fp64
         # oracle's instead of 7e-5; the tensor-core tiers are at that level in either form)
@@ -706,6 +756,8 @@ class Flow(torch.nn.Module):
                     torch.cuda.current_stream(y.device).wait_stream(st)
                 y = ops.linear_fn(y, Mt, c, False, w_transposed=True, operands=operands)
                 consts.append(const)
+                if collect is not None:
+                    collect.append((item, -const))
                 continue
             for layer in (item if isinstance(item, list) else (item,)):
                 if hasattr(layer, "inverse_and_ladj"):
@@ -717,6 +769,8 @@ class Flow(torch.nn.Module):
                     x = layer.backward(y) if context is None else layer.backward(y, context)
                     ladj = layer.log_abs_det_jacobian(x, y)
                 total = total - ladj
+                if collect is not None:
+                    collect.append((layer, -torch.as_tensor(ladj, dtype=torch.float32, device=y.device)))
                 y = x
         if consts:
             total = total - torch.stack(consts).sum()

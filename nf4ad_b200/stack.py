@@ -189,6 +189,7 @@ class CompiledStack:
                 for layer in run:
                     logdet = logdet + float(layer.log_abs_det_jacobian(probe, probe))
             self.logdet_const = logdet      # sum of log|det| of all affine layers (generative direction)
+            self.base_const = None          # the base log-density's normalising constant (None: no supported base)
 
             st = StackDesc()
             st.D, st.n_blocks, st.ctx_dim = D, n, cd
@@ -207,6 +208,7 @@ class CompiledStack:
                     base_const = -float(scale.log().sum()) - 0.5 * D * _LOG_2PI
                 else:
                     base_const = -float((2.0 * scale).log().sum())
+                self.base_const = base_const
                 st.const_term = base_const - logdet
             self.desc = st
 
@@ -369,11 +371,23 @@ class CompiledStack:
         return self._call("usf_stack_run_bf16in" if bf16_rows else "usf_stack_run", x, want_logprob, want_y, want_ladj,
                           deterministic)
 
+    def run_terms(self, x):
+        """log p(x) and its terms (usf_stack_log_prob_terms, always in the deterministic form) of rows x:(B, D + ctx_dim).
+        Returns (logprob (B,), terms (n_blocks + 1, B), z (B, D), n_launches): terms[j] is block j's coupling term in
+        execution order (block j inverts coupling n_blocks - 1 - j of the layer list), terms[n_blocks] the data-dependent
+        part of the base log-density; logprob = desc.const_term + their sum, with const_term = base_const - logdet_const."""
+        if self.desc.base_kind < 0:
+            raise _lib.USFError("this stack was compiled without a supported base distribution")
+        lp, z, terms, n = self._call("usf_stack_log_prob_terms", x, True, True, True, True)
+        return lp, terms, z, n
+
     def _call(self, entry, x, want_lp, want_rows, want_ladj, deterministic):
         """One library call of `entry` on the rows x:(B, D + ctx_dim), `deterministic` mode set for it: the fp32 outputs
         it writes are a (B,) log p, (B, D) rows (y, or the gradient of usf_stack_log_prob_grad, which has no ladj) and a
-        (B,) ladj.  -> (lp | None, rows | None, ladj | None, n_launches)."""
+        (B,) ladj -- or, for usf_stack_log_prob_terms, the (n_blocks + 1, B) terms in its place.
+        -> (lp | None, rows | None, ladj | terms | None, n_launches)."""
         grad = entry == "usf_stack_log_prob_grad"
+        terms = entry == "usf_stack_log_prob_terms"
         bf16_rows = entry == "usf_stack_run_bf16in"
         _lib.require_cuda(x)
         if x.dim() != 2 or x.shape[1] != self.D + self.ctx_dim:
@@ -387,12 +401,19 @@ class CompiledStack:
         B, dev = x.shape[0], x.device
         lp = torch.empty(B, device=dev, dtype=torch.float32) if want_lp else None
         rows = torch.empty(B, self.D, device=dev, dtype=torch.float32) if want_rows else None
-        ladj = torch.empty(B, device=dev, dtype=torch.float32) if want_ladj else None
+        ladj = torch.empty(*((self.desc.n_blocks + 1,) if terms else ()), B, device=dev, dtype=torch.float32) \
+            if want_ladj else None
         if B == 0:
             return lp, rows, ladj, 0
         descs = (C.byref(self.desc), C.byref(self.grad_desc)) if grad else (C.byref(self.desc),)
-        query = "usf_stack_grad_workspace_bytes" if grad else "usf_stack_workspace_bytes"
-        outs = (ptr(lp), ptr(rows), self.D) if grad else (ptr(lp), ptr(rows), self.D, ptr(ladj))
+        query = {"usf_stack_log_prob_grad": "usf_stack_grad_workspace_bytes",
+                 "usf_stack_log_prob_terms": "usf_stack_terms_workspace_bytes"}.get(entry, "usf_stack_workspace_bytes")
+        if grad:
+            outs = (ptr(lp), ptr(rows), self.D)
+        elif terms:
+            outs = (ptr(lp), ptr(ladj), B, ptr(rows), self.D)
+        else:
+            outs = (ptr(lp), ptr(rows), self.D, ptr(ladj))
         tier = () if bf16_rows else (self.precision,)          # (usf_stack_run_bf16in runs the bf16 tier)
         L = lib()
         prev = L.usf_set_deterministic(int(bool(deterministic)))
